@@ -3,7 +3,7 @@
 spectrum, at 1/2/4/8 B200 vs the reference CPU path; % of roofline).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--workload c3|c4|c5|c2|c1|c3dense]
+                    [--workload c3|c4|c5|c2|c1|c3dense] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one synthetic trajectory block that is already resident in
 HBM: ``calc_polarizabilities`` over every frame of the rank's block and ``MDRamanSpectrum.measure``
@@ -20,6 +20,10 @@ frames in total sharded over the ranks (strong); "c5" = configs[4], 1536-atom su
 After the timed region every run checks ITS OWN output against the CPU oracle (``parity`` in the
 JSON line): random frame blocks of the series per rank (<= 1e-10) and the whole spectrum on rank 0
 (<= 1e-8).
+
+``--dump-outputs DIR`` writes what the last timed step returned on rank 0 as float64 ``.npy`` files:
+``polarizability_ts`` (rank 0's frames), ``wavenumbers`` and ``intensities``.  The inputs are seeded, so
+two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -60,7 +64,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--cpu-sample", type=int, default=8192, help="frames in the CPU-baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (b200 only)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 def workload_frames(args, world):
@@ -149,6 +160,26 @@ def ncu_traffic(kernel: str, workload: str):
         with open(path, encoding="utf-8") as fh:
             return json.load(fh).get(f"{kernel}:{workload}")
     return None
+
+
+DUMP_ARRAY_BYTES = 16 << 20  # per array: three arrays stay well under 64 MB
+
+
+def dump_outputs(directory, outputs):
+    """Write each array of ``outputs`` as ``directory/<name>.npy`` in float64.  An array larger than
+    DUMP_ARRAY_BYTES keeps a fixed, seeded sample of its rows (ascending), the same for every run with
+    the same number of rows."""
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    for name, array in outputs.items():
+        array = torch.as_tensor(array)
+        rows = int(array.shape[0])
+        keep = max(1, DUMP_ARRAY_BYTES // (8 * int(np.prod(array.shape[1:]))))
+        if rows > keep:
+            index = np.sort(np.random.default_rng(0).choice(rows, size=keep, replace=False))
+            array = array[torch.from_numpy(index).to(array.device)]
+        np.save(os.path.join(directory, f"{name}.npy"), array.to(torch.float64).cpu().numpy())
 
 
 def build_state(structure, kind):
@@ -394,6 +425,10 @@ def run_b200(args):
         elapsed_ms, launches = float(tmax[0]), int(t[1])
     ms_per_step = elapsed_ms / args.steps
     value = total_frames / (ms_per_step * 1e-3)
+
+    if args.dump_outputs and rank == 0:
+        local = spectrum.local_polarizability_ts if world > 1 else spectrum._polarizability_ts  # pylint: disable=protected-access
+        dump_outputs(args.dump_outputs, {"polarizability_ts": local, "wavenumbers": wn, "intensities": inten})
 
     # ---- parity of the timed step's own output (outside the timed region) ----
     parity = None

@@ -2,11 +2,13 @@
 GPU box, where tests/test_gpu_install.py drives the same code through a stand-in package):
 ``ModelState.from_reference`` / ``accelerate`` on models the unmodified reference built, the fingerprint
 that re-packs a mutated model, and ``install()`` / ``uninstall()`` of the four patched entry points."""
+import os
+
 import numpy as np
 import pytest
 
 import ramannoodle_b200 as rb
-from oracle.ref_bootstrap import import_reference, reference_available
+from oracle.ref_bootstrap import REFERENCE_ROOT, import_reference, reference_available
 from ramannoodle_b200 import dropin as rb_install
 from ramannoodle_b200 import synthetic
 from ramannoodle_b200.exceptions import NativeLibraryError
@@ -30,7 +32,7 @@ def _tio2_reference_model(order, art=False):
     from ramannoodle.pmodel._art import ARTModel
     from ramannoodle.pmodel._interpolation import InterpolationModel
 
-    data_dir = "/root/reference/test/data/TiO2"
+    data_dir = os.path.join(REFERENCE_ROOT, "test", "data", "TiO2")
     structure = generic_io.read_ref_structure(f"{data_dir}/phonons_OUTCAR", file_format="outcar")
     _, ref_pol = generic_io.read_positions_and_polarizability(f"{data_dir}/ref_eps_OUTCAR", file_format="outcar")
     model = (ARTModel if art else InterpolationModel)(structure, ref_pol)
