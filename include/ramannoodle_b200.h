@@ -156,6 +156,25 @@ int rn_calc_polarizabilities_sweep(const rn_model* const* models, int num_models
 int rn_calc_polarizabilities_host_sweep(const rn_model* const* models, int num_models,
                                         const double* h_positions, int64_t num_frames,
                                         double* const* d_alpha_outputs, int64_t chunk_frames);
+/* Routed mask sweep for the shared multi-GPU spectrum: d_alpha_outputs[g] receives what
+ * rn_calc_polarizabilities_sweep writes (this rank's block of mask g's series; spline models always take the
+ * whole-tile schedule here, so short blocks may differ from the plain sweep's unit-balanced one in the last
+ * bits), and row n of mask g is
+ * also stored to peer_series[g*world + r] for r = owner(n) and r = owner(n-1) — the rule of
+ * rn_calc_polarizabilities_routed, one row of `world` base pointers per mask (NULL for this rank and
+ * for ranks that own nothing).  The host form sends each chunk across PCIe once for all masks; its
+ * private streams start after the work already enqueued on `stream` and it returns when done. */
+int rn_calc_polarizabilities_sweep_routed(const rn_model* const* models, int num_models,
+                                          const double* d_positions, int64_t num_frames,
+                                          double* const* d_alpha_outputs, double* const* peer_series,
+                                          int world, int64_t first_frame, int64_t period, int64_t width,
+                                          void* stream);
+int rn_calc_polarizabilities_host_sweep_routed(const rn_model* const* models, int num_models,
+                                               const double* h_positions, int64_t num_frames,
+                                               double* const* d_alpha_outputs,
+                                               double* const* peer_series, int world,
+                                               int64_t first_frame, int64_t period, int64_t width,
+                                               int64_t chunk_frames, void* stream);
 
 /* Trajectory.__init__ stores apply_pbc(positions_ts) (dynamics/_trajectory.py:45;
  * structure/utils.py:27: p - p // 1).  Elementwise, in place allowed (d_out == d_in). */

@@ -86,6 +86,14 @@ PROTOTYPES = {
                                                       ctypes.c_void_p, ctypes.c_void_p]),
     "rn_calc_polarizabilities_host_sweep": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
                                                            ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64]),
+    "rn_calc_polarizabilities_sweep_routed": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+                                                             ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                                                             ctypes.c_int, ctypes.c_int64, ctypes.c_int64,
+                                                             ctypes.c_int64, ctypes.c_void_p]),
+    "rn_calc_polarizabilities_host_sweep_routed": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+                                                                  ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                                                                  ctypes.c_int, ctypes.c_int64, ctypes.c_int64,
+                                                                  ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p]),
     "rn_xdatcar_scan": (ctypes.c_int, [ctypes.c_char_p, c_int64_p, c_int64_p, ctypes.c_void_p]),
     "rn_xdatcar_read": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64,
                                        ctypes.c_int, ctypes.c_int]),

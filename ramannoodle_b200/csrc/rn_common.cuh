@@ -245,10 +245,19 @@ int eval_with_peers(const rn_model* model, const double* d_positions, int64_t nu
                     cudaStream_t stream, const AlphaPeers& peers);
 int make_routed_peers(double* const* peer_series, int world, int64_t first_frame, int64_t period, int64_t width,
                       AlphaPeers* peers);
-// rn_dense_sweep.cu: spline part of 2..4 masked copies of one model with a shared projection
+// rn_dense_sweep.cu: spline part of 2..4 masked copies of one model with a shared projection; `routed`
+// (null, or one entry per model) names the ranks the finished rows of each model also go to
 bool dense_sweep_eligible(const rn_model* m);
 bool dense_sweep_compatible(const rn_model* a, const rn_model* b);
 int launch_dense_sweep(const rn_model* const* models, int count, const double* d_in, bool accumulate,
-                       int64_t num_frames, double* const* d_alpha, cudaStream_t stream);
+                       int64_t num_frames, double* const* d_alpha, cudaStream_t stream,
+                       const AlphaPeers* routed = nullptr);
+// rn_sweep.cu: mask sweep of device-resident frames; `routed` as above
+constexpr int kMaxSweepModels = 64;
+int sweep_eval(const rn_model* const* models, int num_models, const double* d_positions, int64_t num_frames,
+               double* const* d_alpha_outputs, cudaStream_t stream, const AlphaPeers* routed);
+// routed[g] = make_routed_peers(peer_series + g * world, ...) for every model
+int make_sweep_peers(int num_models, double* const* peer_series, int world, int64_t first_frame, int64_t period,
+                     int64_t width, AlphaPeers* routed);
 
 }  // namespace rn

@@ -288,13 +288,15 @@ static int launch_tp_cfg(const rn_model* m, const double* d_in, bool wrap, bool 
     mk.c9[0] = m->d_tp_c9;
     mk.alpha[0] = d_alpha;
     mk.a0[0] = a0;
+    TpPeers<1> tpeers;
+    tpeers.mask[0] = peers;
 #define RN_TP_LAUNCH(W, A)                                                                                   \
     {                                                                                                        \
         auto kern = dense_kernel_tp<DEG, NBK, FULL, W, A, 1>;                                                \
         RN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));         \
         kern<<<grid, 384, smem, stream>>>(d_in, m->d_ref_wrapped, V, m->d_tp_x0, m->d_tp_brk, num_frames, K, \
                                           (int)m->v_cols, (int)m->dense_pad, (int)m->num_dense, accumulate ? 1 : 0,             \
-                                          (split ? 1 : 0) | (g_dense_variant.load(std::memory_order_relaxed) << 1), stages, mk, peers);                                         \
+                                          (split ? 1 : 0) | (g_dense_variant.load(std::memory_order_relaxed) << 1), stages, mk, tpeers);                                        \
     }
     if (wrap) {
         if (align16) RN_TP_LAUNCH(true, true) else RN_TP_LAUNCH(true, false)

@@ -14,7 +14,8 @@ constexpr int kDenseSweepMax = 4;
 
 template <int DEG, int NBK, bool FULL, int NG>
 static int launch_tp_sweep_cfg(const rn_model* const* models, const double* d_in, bool accumulate,
-                               int64_t num_frames, double* const* d_alpha, cudaStream_t stream) {
+                               int64_t num_frames, double* const* d_alpha, cudaStream_t stream,
+                               const AlphaPeers* routed) {
     const rn_model* m = models[0];
     const int K = (int)m->dim;
     constexpr int FT = 128;
@@ -26,7 +27,8 @@ static int launch_tp_sweep_cfg(const rn_model* const* models, const double* d_in
     // unit-balanced schedule for short trajectories, as in rn_dense.cu: launch_tp_cfg
     const int64_t jtiles = m->dense_pad / kJT2;
     const int64_t rounds = (tiles + m->sm_count - 1) / m->sm_count;
-    const bool split = tiles * jtiles >= 2 && (double)(rounds * m->sm_count) > 1.04 * (double)tiles;
+    // (not with routed stores: the peers need finished rows)
+    const bool split = !routed && tiles * jtiles >= 2 && (double)(rounds * m->sm_count) > 1.04 * (double)tiles;
     if (split) {
         grid = (int)std::min<int64_t>(tiles * jtiles, m->sm_count);
         if (!accumulate) {
@@ -46,17 +48,24 @@ static int launch_tp_sweep_cfg(const rn_model* const* models, const double* d_in
         for (int q = 0; q < 9; q++)
             mk.a0[g].v[q] = accumulate ? (mg->alpha0_tp[q] - mg->alpha0[q]) : mg->alpha0_tp[q];
     }
-    AlphaPeers peers;
-    peers.count = 0;
-#define RN_TP_SWEEP_LAUNCH(A)                                                                                   \
+    // routed: one set of destinations per mask (kernels of their own, the plain sweep's code stays as it is)
+    TpPeers<1> none;
+    none.mask[0] = no_peers();
+    TpPeers<NG> peers;
+    for (int g = 0; g < NG; g++) peers.mask[g] = routed ? routed[g] : no_peers();
+#define RN_TP_SWEEP_LAUNCH(A, NP, P)                                                                            \
     {                                                                                                           \
-        auto kern = dense_kernel_tp<DEG, NBK, FULL, true, A, NG>;                                               \
+        auto kern = dense_kernel_tp<DEG, NBK, FULL, true, A, NG, NP>;                                           \
         RN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
         kern<<<grid, 384, smem, stream>>>(d_in, m->d_ref_wrapped, m->d_v_frac, m->d_tp_x0, m->d_tp_brk,         \
                                           num_frames, K, (int)m->v_cols, (int)m->dense_pad, (int)m->num_dense, accumulate ? 1 : 0, \
-                                          split ? 1 : 0, stages, mk, peers);                                            \
+                                          split ? 1 : 0, stages, mk, P);                                                \
     }
-    if (align16) RN_TP_SWEEP_LAUNCH(true) else RN_TP_SWEEP_LAUNCH(false)
+    if (routed) {
+        if (align16) RN_TP_SWEEP_LAUNCH(true, NG, peers) else RN_TP_SWEEP_LAUNCH(false, NG, peers)
+    } else {
+        if (align16) RN_TP_SWEEP_LAUNCH(true, 1, none) else RN_TP_SWEEP_LAUNCH(false, 1, none)
+    }
 #undef RN_TP_SWEEP_LAUNCH
     RN_LAUNCHED();
     RN_CUDA(cudaGetLastError());
@@ -65,31 +74,31 @@ static int launch_tp_sweep_cfg(const rn_model* const* models, const double* d_in
 
 template <int DEG, int NG>
 static int launch_tp_sweep_deg(const rn_model* const* models, const double* d_in, bool accumulate, int64_t num_frames,
-                               double* const* d_alpha, cudaStream_t stream) {
+                               double* const* d_alpha, cudaStream_t stream, const AlphaPeers* routed) {
     const rn_model* m = models[0];
     const bool full = m->tp_mode == 2;
     switch (m->tp_breaks) {
-        case 0: return launch_tp_sweep_cfg<DEG, 0, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream);
+        case 0: return launch_tp_sweep_cfg<DEG, 0, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
         case 1:
-            return full ? launch_tp_sweep_cfg<DEG, 1, true, NG>(models, d_in, accumulate, num_frames, d_alpha, stream)
-                        : launch_tp_sweep_cfg<DEG, 1, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream);
+            return full ? launch_tp_sweep_cfg<DEG, 1, true, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed)
+                        : launch_tp_sweep_cfg<DEG, 1, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
         case 2:
-            return full ? launch_tp_sweep_cfg<DEG, 2, true, NG>(models, d_in, accumulate, num_frames, d_alpha, stream)
-                        : launch_tp_sweep_cfg<DEG, 2, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream);
+            return full ? launch_tp_sweep_cfg<DEG, 2, true, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed)
+                        : launch_tp_sweep_cfg<DEG, 2, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
         case 3:
             return full ? 1
-                        : launch_tp_sweep_cfg<DEG, 3, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream);
+                        : launch_tp_sweep_cfg<DEG, 3, false, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
         default: return 1;
     }
 }
 
 template <int NG>
 static int launch_tp_sweep_ng(const rn_model* const* models, const double* d_in, bool accumulate, int64_t num_frames,
-                              double* const* d_alpha, cudaStream_t stream) {
+                              double* const* d_alpha, cudaStream_t stream, const AlphaPeers* routed) {
     switch (models[0]->dense_degree) {
-        case 1: return launch_tp_sweep_deg<1, NG>(models, d_in, accumulate, num_frames, d_alpha, stream);
-        case 2: return launch_tp_sweep_deg<2, NG>(models, d_in, accumulate, num_frames, d_alpha, stream);
-        case 3: return launch_tp_sweep_deg<3, NG>(models, d_in, accumulate, num_frames, d_alpha, stream);
+        case 1: return launch_tp_sweep_deg<1, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
+        case 2: return launch_tp_sweep_deg<2, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
+        case 3: return launch_tp_sweep_deg<3, NG>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
         default: return 1;
     }
 }
@@ -107,13 +116,14 @@ bool dense_sweep_eligible(const rn_model* m) {
 }
 
 // Dense (spline) part of `count` (2 or 4) compatible models on fractional positions: accumulates onto
-// d_alpha[g] when `accumulate` (their affine parts were written first), else writes alpha0 + sum.
+// d_alpha[g] when `accumulate` (their affine parts were written first), else writes alpha0 + sum; with
+// `routed`, the finished rows of model g also go to the ranks routed[g] names.
 // Returns 1 when no kernel configuration covers the models (caller evaluates them one by one).
 int launch_dense_sweep(const rn_model* const* models, int count, const double* d_in, bool accumulate,
-                       int64_t num_frames, double* const* d_alpha, cudaStream_t stream) {
+                       int64_t num_frames, double* const* d_alpha, cudaStream_t stream, const AlphaPeers* routed) {
     // instantiated for 2 and 4 masks (build time); the caller deals runs of 3 out as 2 + 1
-    if (count == 2) return launch_tp_sweep_ng<2>(models, d_in, accumulate, num_frames, d_alpha, stream);
-    if (count == 4) return launch_tp_sweep_ng<4>(models, d_in, accumulate, num_frames, d_alpha, stream);
+    if (count == 2) return launch_tp_sweep_ng<2>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
+    if (count == 4) return launch_tp_sweep_ng<4>(models, d_in, accumulate, num_frames, d_alpha, stream, routed);
     return 1;
 }
 

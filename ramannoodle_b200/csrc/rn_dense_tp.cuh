@@ -59,16 +59,24 @@ struct TpMasks {
     Alpha0 a0[NG];
 };
 
+// Extra destinations of the finished rows: NP = 1, one set for every mask (a single model: the fused
+// all-gather / routed stores of rn_calc_polarizabilities_multi / _routed; a sweep: none), or NP = NG, one
+// set per mask (rn_calc_polarizabilities_sweep_routed).
+template <int NP>
+struct TpPeers {
+    AlphaPeers mask[NP];
+};
+
 // Chained-DMMA epilogue: the amplitude accumulators of the projection are turned, in registers,
 // into truncated-power features that feed a second DMMA against the per-DOF coefficient table
 // (the C fragment layout of m8n8k4 is, up to the k-permutation, an A fragment layout: lane (g,t)
 // holds amplitudes of frame g for DOFs 2t and 2t+1).  No shared-memory round trip, no per-frame
 // table walks: one coefficient fragment is shared by 32 frames of the warp.
-template <int DEG, int NBK, bool FULL, bool WRAP, bool ALIGN16, int NG>
+template <int DEG, int NBK, bool FULL, bool WRAP, bool ALIGN16, int NG, int NP = 1>
 __global__ void __launch_bounds__(384, 1)
     dense_kernel_tp(const double* __restrict__ in, const double* __restrict__ ref, const double* __restrict__ V,
                     const double* __restrict__ tp_x0, const double* __restrict__ tp_brk, int64_t num_frames, int K,
-                    int Kv, int Jpad, int Jreal, int accumulate, int split, int stages, TpMasks<NG> mk, AlphaPeers peers) {
+                    int Kv, int Jpad, int Jreal, int accumulate, int split, int stages, TpMasks<NG> mk, TpPeers<NP> peers) {
     constexpr int FT = 128;    // frames per tile: 8 MMA warps x 16
     constexpr int MMAW = 8;    // MMA warps (two per scheduler: one covers the other's LDS / barrier bubbles)
     constexpr int MTW = 2;     // 8-frame groups per MMA warp
@@ -389,12 +397,13 @@ __global__ void __launch_bounds__(384, 1)
                     dst[2 * t + 1] = r1;
                     if (t == 0) dst[8] = r8;
                     // fused all-gather: the same row goes to every peer GPU's series over NVLink
-                    if (peers.count > 0) {
-                        const uint32_t mask = alpha_peer_mask(peers, frame, 1);
-                        const int64_t off = alpha_peer_offset(peers, frame);
-                        for (int p = 0; p < peers.count; p++) {
-                            if (!((mask >> p) & 1u) || !peers.ptr[p]) continue;
-                            double* pd = peers.ptr[p] + off;
+                    const AlphaPeers& P = peers.mask[NP == 1 ? 0 : m];
+                    if (P.count > 0) {
+                        const uint32_t mask = alpha_peer_mask(P, frame, 1);
+                        const int64_t off = alpha_peer_offset(P, frame);
+                        for (int p = 0; p < P.count; p++) {
+                            if (!((mask >> p) & 1u) || !P.ptr[p]) continue;
+                            double* pd = P.ptr[p] + off;
                             pd[2 * t] = r0;
                             pd[2 * t + 1] = r1;
                             if (t == 0) pd[8] = r8;

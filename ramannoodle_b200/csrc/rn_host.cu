@@ -164,14 +164,11 @@ extern "C" int rn_calc_polarizabilities_host_routed(const rn_model* model, const
     return host_pipeline(model, h_positions, num_frames, nullptr, d_alpha, peers, chunk_frames, stream);
 }
 
-extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int num_models, const double* d_positions,
-                                              int64_t num_frames, double* const* d_alpha_outputs, void* stream);
-
-// Mask sweep from a host trajectory: every chunk crosses PCIe once and is evaluated by all models.
-extern "C" int rn_calc_polarizabilities_host_sweep(const rn_model* const* models, int num_models,
-                                                   const double* h_positions, int64_t num_frames,
-                                                   double* const* d_alpha_outputs, int64_t chunk_frames) {
-    RN_CHECK_ARG(models != nullptr && num_models >= 1 && num_models <= 64, "1..64 models are required");
+// Mask sweep from a host trajectory: every chunk crosses PCIe once and is evaluated by all models.  `routed`
+// (null, or one entry per model) names the ranks the rows also go to; its first_frame is shifted per chunk.
+static int host_sweep(const rn_model* const* models, int num_models, const double* h_positions, int64_t num_frames,
+                      double* const* d_alpha_outputs, const AlphaPeers* routed, int64_t chunk_frames, void* stream) {
+    RN_CHECK_ARG(models != nullptr && num_models >= 1 && num_models <= kMaxSweepModels, "1..64 models are required");
     RN_CHECK_ARG(d_alpha_outputs != nullptr, "output pointers are required");
     for (int g = 0; g < num_models; g++) {
         RN_CHECK_ARG(models[g] != nullptr && d_alpha_outputs[g] != nullptr, "null model or output pointer");
@@ -192,19 +189,43 @@ extern "C" int rn_calc_polarizabilities_host_sweep(const rn_model* const* models
     HostPipe* pipe = nullptr;
     int rc = acquire_pipe(model->device, chunk_frames * K, 0, &pipe);
     if (rc != RN_OK) return rc;
-    rc = order_after_caller(*pipe, nullptr);
+    rc = order_after_caller(*pipe, static_cast<cudaStream_t>(stream));
     if (rc != RN_OK) return rc;
     int slot = 0;
+    AlphaPeers chunk_routed[kMaxSweepModels];
     for (int64_t f0 = 0; f0 < num_frames; f0 += chunk_frames, slot ^= 1) {
         const int64_t n = std::min(chunk_frames, num_frames - f0);
         cudaStream_t s = pipe->stream[slot];
         RN_CUDA(cudaMemcpyAsync(pipe->d_pos[slot], h_positions + f0 * K, sizeof(double) * n * K, cudaMemcpyHostToDevice, s));
-        double* outs[64];
-        for (int g = 0; g < num_models; g++) outs[g] = d_alpha_outputs[g] + f0 * 9;
-        rc = rn_calc_polarizabilities_sweep(models, num_models, pipe->d_pos[slot], n, outs, s);
+        double* outs[kMaxSweepModels];
+        for (int g = 0; g < num_models; g++) {
+            outs[g] = d_alpha_outputs[g] + f0 * 9;
+            if (routed) {
+                chunk_routed[g] = routed[g];
+                chunk_routed[g].first_frame = routed[g].first_frame + f0;
+            }
+        }
+        rc = sweep_eval(models, num_models, pipe->d_pos[slot], n, outs, s, routed ? chunk_routed : nullptr);
         if (rc != RN_OK) return rc;
     }
     RN_CUDA(cudaStreamSynchronize(pipe->stream[0]));
     RN_CUDA(cudaStreamSynchronize(pipe->stream[1]));
     return RN_OK;
+}
+
+extern "C" int rn_calc_polarizabilities_host_sweep(const rn_model* const* models, int num_models,
+                                                   const double* h_positions, int64_t num_frames,
+                                                   double* const* d_alpha_outputs, int64_t chunk_frames) {
+    return host_sweep(models, num_models, h_positions, num_frames, d_alpha_outputs, nullptr, chunk_frames, nullptr);
+}
+
+extern "C" int rn_calc_polarizabilities_host_sweep_routed(const rn_model* const* models, int num_models,
+                                                          const double* h_positions, int64_t num_frames,
+                                                          double* const* d_alpha_outputs, double* const* peer_series,
+                                                          int world, int64_t first_frame, int64_t period, int64_t width,
+                                                          int64_t chunk_frames, void* stream) {
+    AlphaPeers routed[kMaxSweepModels];
+    const int rc = make_sweep_peers(num_models, peer_series, world, first_frame, period, width, routed);
+    if (rc != RN_OK) return rc;
+    return host_sweep(models, num_models, h_positions, num_frames, d_alpha_outputs, routed, chunk_frames, stream);
 }

@@ -48,6 +48,11 @@ struct SweepOut {
     int columns;                    // 9 * masks
 };
 
+// routed destinations of the masks of one launch (rn_calc_polarizabilities_sweep_routed)
+struct SweepPeers {
+    AlphaPeers mask[kSweepMaxMasks];
+};
+
 // stacked[e][c] = G_{c/9}[e][c%9] for c < columns, 0 in the padding columns
 __global__ void sweep_stack_kernel(SweepTables tabs, int64_t rows, int columns, int padded, double* __restrict__ stacked) {
     const int64_t total = rows * padded;
@@ -81,11 +86,12 @@ __device__ __forceinline__ double wrap_disp_sel(double pos, double ref, bool& fa
 }
 
 // 8 warps, one CTA per SM (the B fragments of all column tiles fill the register file).
-template <int KP, int NT, bool WRAP, bool MASKED>
+// ROUTED: every finished element is also stored to the ranks that own its row (plain peer stores).
+template <int KP, int NT, bool WRAP, bool MASKED, bool ROUTED>
 __global__ void __launch_bounds__(kSweepWarps * 32, 1)
     affine_sweep_kernel(const double* __restrict__ in, const double* __restrict__ ref,
                         const double* __restrict__ stacked, int64_t num_frames, int K, int row_stride,
-                        int stage_doubles, int num_stages, SweepOut out) {
+                        int stage_doubles, int num_stages, SweepOut out, const __grid_constant__ SweepPeers peers) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int ROWS = 8;
     constexpr int RS = SweepSmem<NT>::kRed;
@@ -166,7 +172,16 @@ __global__ void __launch_bounds__(kSweepWarps * 32, 1)
                 double sum = 0;
 #pragma unroll
                 for (int w = 0; w < kSweepWarps; w++) sum += r[(size_t)w * ROWS * RS];
-                tab_out[idx][tile * (int64_t)(ROWS * 9)] = sum + tab_a0[idx];
+                const double value = sum + tab_a0[idx];
+                tab_out[idx][tile * (int64_t)(ROWS * 9)] = value;
+                if (ROUTED) {
+                    const AlphaPeers& P = peers.mask[c / 9];
+                    const int64_t frame = tile * ROWS + f;
+                    const uint32_t owners = alpha_peer_mask(P, frame, 1);
+                    const int64_t off = alpha_peer_offset(P, frame) + (c - 9 * (c / 9));
+                    for (int p = 0; p < P.count; p++)
+                        if (((owners >> p) & 1u) && P.ptr[p]) P.ptr[p][off] = value;
+                }
             }
         }
     };
@@ -253,17 +268,22 @@ static SweepLayout sweep_layout(int K, int kp, int nt) {
 
 template <int KP, int NT, bool WRAP>
 static int launch_sweep_cfg(const rn_model* m, const double* d_in, int64_t frames, const double* d_stacked,
-                            const SweepOut& out, cudaStream_t stream) {
+                            const SweepOut& out, const SweepPeers* peers, cudaStream_t stream) {
     const int K = (int)m->dim;
     const SweepLayout L = sweep_layout(K, KP, NT);
     if (L.bytes > 227 * 1024) return 1;
     const bool masked = (K != kSweepWarps * 8 * KP);
-    auto kern = masked ? affine_sweep_kernel<KP, NT, WRAP, true> : affine_sweep_kernel<KP, NT, WRAP, false>;
+    auto kern = peers ? (masked ? affine_sweep_kernel<KP, NT, WRAP, true, true> : affine_sweep_kernel<KP, NT, WRAP, false, true>)
+                      : (masked ? affine_sweep_kernel<KP, NT, WRAP, true, false> : affine_sweep_kernel<KP, NT, WRAP, false, false>);
     RN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.bytes));
     const int64_t tiles = (frames + 7) / 8;
     const int grid = (int)std::min<int64_t>(tiles, (int64_t)m->sm_count);
+    SweepPeers routed;
+    if (peers) routed = *peers;
+    else
+        for (int r = 0; r < kSweepMaxMasks; r++) routed.mask[r] = no_peers();
     kern<<<grid, kSweepWarps * 32, L.bytes, stream>>>(d_in, WRAP ? m->d_ref_wrapped : m->d_zero_ref, d_stacked, frames, K,
-                                                      L.row_stride, L.stage_doubles, L.stages, out);
+                                                      L.row_stride, L.stage_doubles, L.stages, out, routed);
     RN_LAUNCHED();
     RN_CUDA(cudaGetLastError());
     return RN_OK;
@@ -271,20 +291,20 @@ static int launch_sweep_cfg(const rn_model* m, const double* d_in, int64_t frame
 
 template <int KP, bool WRAP>
 static int launch_sweep_nt(int nt, const rn_model* m, const double* d_in, int64_t frames, const double* d_stacked,
-                           const SweepOut& out, cudaStream_t stream) {
+                           const SweepOut& out, const SweepPeers* peers, cudaStream_t stream) {
     switch (nt) {
-        case 3: return launch_sweep_cfg<KP, 3, WRAP>(m, d_in, frames, d_stacked, out, stream);
-        case 4: return launch_sweep_cfg<KP, 4, WRAP>(m, d_in, frames, d_stacked, out, stream);
-        case 5: return launch_sweep_cfg<KP, 5, WRAP>(m, d_in, frames, d_stacked, out, stream);
+        case 3: return launch_sweep_cfg<KP, 3, WRAP>(m, d_in, frames, d_stacked, out, peers, stream);
+        case 4: return launch_sweep_cfg<KP, 4, WRAP>(m, d_in, frames, d_stacked, out, peers, stream);
+        case 5: return launch_sweep_cfg<KP, 5, WRAP>(m, d_in, frames, d_stacked, out, peers, stream);
         default: return 1;
     }
 }
 
 static int launch_sweep(int nt, const rn_model* m, const double* d_in, int64_t frames, const double* d_stacked,
-                        const SweepOut& out, cudaStream_t stream) {
+                        const SweepOut& out, const SweepPeers* peers, cudaStream_t stream) {
     switch (m->affine_kp) {
 #define RN_SWEEP_CASE(KP) \
-    case KP: return launch_sweep_nt<KP, true>(nt, m, d_in, frames, d_stacked, out, stream);
+    case KP: return launch_sweep_nt<KP, true>(nt, m, d_in, frames, d_stacked, out, peers, stream);
         RN_SWEEP_CASE(1)
         RN_SWEEP_CASE(2)
         RN_SWEEP_CASE(3)
@@ -312,16 +332,14 @@ static bool sweep_eligible(const rn_model* m, const double* d_in) {
            reinterpret_cast<uintptr_t>(d_in) % 16 == 0;
 }
 
-}  // namespace rn
-
-using namespace rn;
-
 // Evaluates every model of `models` (masked copies of one model: same reference structure) on the
 // same positions: d_alpha_outputs[g] (num_frames*9) receives model g's series.  Replaces G calls of
 // InterpolationModel.calc_polarizabilities (pmodel/_interpolation.py:191-252) on get_masked_model
-// copies (:697-708).
-extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int num_models, const double* d_positions,
-                                              int64_t num_frames, double* const* d_alpha_outputs, void* stream) {
+// copies (:697-708).  `routed` (null, or one entry per model): the final rows of model g also go to the
+// ranks routed[g] names; the affine parts of mixed models are written locally first and only the
+// finished sums are stored to the peers.
+int sweep_eval(const rn_model* const* models, int num_models, const double* d_positions, int64_t num_frames,
+               double* const* d_alpha_outputs, cudaStream_t s, const AlphaPeers* routed) {
     RN_CHECK_ARG(models != nullptr && num_models >= 1, "at least one model is required");
     RN_CHECK_ARG(d_alpha_outputs != nullptr, "output pointers are required");
     for (int g = 0; g < num_models; g++)
@@ -329,7 +347,6 @@ extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int
     RN_CHECK_ARG(num_frames >= 0, "num_frames must be non-negative");
     if (num_frames == 0) return RN_OK;
     RN_CHECK_ARG(d_positions != nullptr, "null positions pointer");
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
     DeviceGuard guard(models[0]->device);
     if (!guard.ok) {
         set_error("cudaSetDevice(%d) failed", models[0]->device);
@@ -352,11 +369,13 @@ extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int
             const int nt = (columns + 7) / 8;
             SweepTables tabs;
             SweepOut out;
+            SweepPeers peers;
             for (int c = 0; c < 8 * kSweepMaxTiles; c++) out.a0[c] = 0.0;
             for (int r = 0; r < kSweepMaxMasks; r++) {
                 const rn_model* mr = models[g + std::min(r, run - 1)];
                 tabs.g[r] = mr->d_g_frac;
                 out.alpha[r] = d_alpha_outputs[g + std::min(r, run - 1)];
+                peers.mask[r] = (routed && r < run) ? routed[g + r] : no_peers();
                 if (r < run)
                     for (int q = 0; q < 9; q++) out.a0[9 * r + q] = mr->alpha0[q];
             }
@@ -382,7 +401,7 @@ extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int
             sweep_stack_kernel<<<(unsigned)std::min<int64_t>((rows * 8 * nt + 255) / 256, 1024), 256, 0, s>>>(
                 tabs, rows, columns, 8 * nt, d_stacked);
             RN_LAUNCHED();
-            int rc = launch_sweep(nt, m, d_positions, num_frames, d_stacked, out, s);
+            int rc = launch_sweep(nt, m, d_positions, num_frames, d_stacked, out, routed ? &peers : nullptr, s);
             cudaError_t free_rc = cudaFreeAsync(d_stacked, s);
             if (rc != RN_OK && rc != 1) return rc;
             RN_CUDA(free_rc);
@@ -404,7 +423,8 @@ extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int
                 for (int r = 0; r < drun && rc == RN_OK && has_affine; r++)
                     rc = launch_affine(models[g + r], d_positions, true, num_frames, d_alpha_outputs[g + r], s);
                 if (rc != RN_OK) return rc;
-                rc = launch_dense_sweep(models + g, drun, d_positions, has_affine, num_frames, d_alpha_outputs + g, s);
+                rc = launch_dense_sweep(models + g, drun, d_positions, has_affine, num_frames, d_alpha_outputs + g, s,
+                                        routed ? routed + g : nullptr);
                 if (rc != RN_OK && rc != 1) return rc;
                 if (rc == RN_OK) {
                     g += drun;
@@ -412,11 +432,45 @@ extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int
                 }
             }
         }
-        int rc = rn_calc_polarizabilities(models[g], d_positions, num_frames, d_alpha_outputs[g], stream);
+        int rc = routed ? eval_with_peers(models[g], d_positions, num_frames, d_alpha_outputs[g], s, routed[g])
+                        : rn_calc_polarizabilities(models[g], d_positions, num_frames, d_alpha_outputs[g], s);
         if (rc != RN_OK) return rc;
         g++;
     }
     return RN_OK;
+}
+
+int make_sweep_peers(int num_models, double* const* peer_series, int world, int64_t first_frame, int64_t period,
+                     int64_t width, AlphaPeers* routed) {
+    RN_CHECK_ARG(num_models >= 1 && num_models <= kMaxSweepModels, "1..64 models are required");
+    RN_CHECK_ARG(peer_series != nullptr, "peer series pointers are required");
+    for (int g = 0; g < num_models; g++) {
+        const int rc = make_routed_peers(peer_series + (int64_t)g * world, world, first_frame, period, width, routed + g);
+        if (rc != RN_OK) return rc;
+    }
+    return RN_OK;
+}
+
+}  // namespace rn
+
+using namespace rn;
+
+extern "C" int rn_calc_polarizabilities_sweep(const rn_model* const* models, int num_models, const double* d_positions,
+                                              int64_t num_frames, double* const* d_alpha_outputs, void* stream) {
+    return sweep_eval(models, num_models, d_positions, num_frames, d_alpha_outputs, static_cast<cudaStream_t>(stream),
+                      nullptr);
+}
+
+extern "C" int rn_calc_polarizabilities_sweep_routed(const rn_model* const* models, int num_models,
+                                                     const double* d_positions, int64_t num_frames,
+                                                     double* const* d_alpha_outputs, double* const* peer_series,
+                                                     int world, int64_t first_frame, int64_t period, int64_t width,
+                                                     void* stream) {
+    AlphaPeers routed[kMaxSweepModels];
+    const int rc = make_sweep_peers(num_models, peer_series, world, first_frame, period, width, routed);
+    if (rc != RN_OK) return rc;
+    return sweep_eval(models, num_models, d_positions, num_frames, d_alpha_outputs, static_cast<cudaStream_t>(stream),
+                      routed);
 }
 
 // test hook: 0 = always evaluate the models one after the other

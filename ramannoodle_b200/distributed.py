@@ -108,14 +108,20 @@ def _all_ranks_agree(ok: bool, device, group) -> bool:
 
 class _SharedContext:
     """Everything the shared spectrum of one (S, device, group) needs: the dist plan and ONE symmetric
-    allocation holding this rank's full-layout series buffer, work buffer, receive buffer and power
-    buffer (cached: allocation and rendezvous are collectives)."""
+    allocation holding this rank's full-layout series buffers, work buffer, receive buffer and power
+    buffer (cached: allocation and rendezvous are collectives).
 
-    def __init__(self, num_frames: int, device, group) -> None:
+    ``slots`` series buffers of ``align(S*72)`` bytes each lie at the start of the allocation, one per
+    model of a mask sweep (``ShardedTrajectory.get_raman_spectra``); the work, receive and power buffers
+    are shared by all slots: the spectra of the slots are measured one after the other on one stream,
+    with barriers between the steps, like two ``measure()`` calls on one spectrum."""
+
+    def __init__(self, num_frames: int, device, group, slots: int = 1) -> None:
         import torch  # pylint: disable=import-outside-toplevel
         import torch.distributed as dist  # pylint: disable=import-outside-toplevel
 
         self.num_frames = int(num_frames)
+        self.slots = int(slots)
         self.device = device
         self.group = group
         self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
@@ -142,7 +148,8 @@ class _SharedContext:
         def align(nbytes: int) -> int:
             return (nbytes + 255) // 256 * 256
 
-        series_bytes = align(self.num_frames * 72)
+        self.series_bytes = align(self.num_frames * 72)
+        series_bytes = self.slots * self.series_bytes
         self.offsets = {"series": 0, "work": series_bytes, "recv": series_bytes + align(sizes[0].value),
                         "spectrum": series_bytes + align(sizes[0].value) + align(sizes[1].value)}
         total = self.offsets["spectrum"] + align(sizes[2].value)
@@ -177,15 +184,16 @@ class _SharedContext:
         self.local_base = int(self.buffer.data_ptr())
         self.peer_bases = [int(self.handle.buffer_ptrs[r]) for r in range(self.world)]
 
-    def ptr(self, rank: int, name: str) -> int:
-        return self.peer_bases[rank] + self.offsets[name]
+    def ptr(self, rank: int, name: str, slot: int = 0) -> int:
+        return self.peer_bases[rank] + self.offsets[name] + (slot * self.series_bytes if name == "series" else 0)
 
     def table(self, name: str, count: int):
         return (ctypes.c_void_p * count)(*[ctypes.c_void_p(self.ptr(r, name)) for r in range(count)])
 
-    def series_view(self, start: int, stop: int):
-        """This rank's rows [start, stop) of its own series buffer as a (n,3,3) tensor."""
-        return self.buffer[start * 9: stop * 9].view(stop - start, 3, 3)
+    def series_view(self, start: int, stop: int, slot: int = 0):
+        """This rank's rows [start, stop) of its own series buffer ``slot`` as a (n,3,3) tensor."""
+        base = slot * self.series_bytes // 8
+        return self.buffer[base + start * 9: base + stop * 9].view(stop - start, 3, 3)
 
     def barrier(self, channel: int = 0) -> None:
         self.handle.barrier(channel=channel)
@@ -221,17 +229,18 @@ class _SharedContext:
 _SHARED: dict = {}
 
 
-def _shared_context(num_frames: int, device, group):
-    """The cached ``_SharedContext``, or None if symmetric memory is unavailable (every rank agrees)."""
+def _shared_context(num_frames: int, device, group, slots: int = 1):
+    """The cached ``_SharedContext`` with at least ``slots`` series buffers, or None if symmetric memory is
+    unavailable (every rank agrees)."""
     import torch.distributed as dist  # pylint: disable=import-outside-toplevel
 
     global _UNAVAILABLE_WARNED  # pylint: disable=global-statement
     pg = group if group is not None else dist.group.WORLD
     key = (int(num_frames), str(device), pg.group_name)
-    if key in _SHARED:
+    if key in _SHARED and (_SHARED[key] is None or _SHARED[key].slots >= slots):
         return _SHARED[key]
     try:
-        ctx = _SharedContext(num_frames, device, group)
+        ctx = _SharedContext(num_frames, device, group, slots)
     except SymmetricMemoryUnavailable as exc:
         if not _UNAVAILABLE_WARNED:
             warnings.warn(f"symmetric memory unavailable ({exc}); using the all-gather path", RuntimeWarning)
@@ -259,7 +268,7 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
     """
 
     def __init__(self, polarizability_ts, timestep: float, group=None, context=None, generation: int = 0,
-                 bounds=None):
+                 bounds=None, slot: int = 0):
         if context is None:
             super().__init__(polarizability_ts, timestep)
         else:  # the local block only; the full series is assembled on demand
@@ -269,6 +278,7 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
         self._context = context
         self._generation = generation
         self._bounds = bounds
+        self._slot = slot
 
     def _check_live(self) -> None:
         if self._context.generation != self._generation:
@@ -282,7 +292,7 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
             start, stop = self._bounds if self._bounds else (0, len(self._polarizability_ts))
             return self._polarizability_ts[start:stop]
         self._check_live()
-        return self._context.series_view(*self._bounds)
+        return self._context.series_view(*self._bounds, self._slot)
 
     def _gathered(self):
         if self._polarizability_ts is None:
@@ -335,7 +345,7 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
                 return wavenumbers, intensities
             stream = _stream(device)
             group = ctx.transform_ranks
-            series_ptr = ctypes.c_void_p(ctx.ptr(ctx.rank, "series"))
+            series_ptr = ctypes.c_void_p(ctx.ptr(ctx.rank, "series", self._slot))
             work_ptr = ctypes.c_void_p(ctx.ptr(ctx.rank, "work"))
             if ctx.pipeline:
                 # The three packed sequences are independent transforms: sequence s runs pack -> barrier ->
@@ -453,6 +463,69 @@ class ShardedTrajectory(Dynamics):
         full = allgather_series(series, self._num_frames, self._group)
         bounds = shard_bounds(self._num_frames, dist.get_world_size(self._group), dist.get_rank(self._group))
         return ShardedMDRamanSpectrum(full, self._local.timestep, self._group, bounds=bounds)
+
+    def get_raman_spectra(self, polarizability_models, shared: bool = True) -> list:
+        """Mask sweep (``Trajectory.get_raman_spectra``) of the sharded trajectory: one
+        ``ShardedMDRamanSpectrum`` per model, all evaluated in one pass over the local block; equal to
+        ``[self.get_raman_spectrum(m) for m in polarizability_models]`` with each spectrum measured before the
+        next is evaluated.
+
+        ``shared=True``: the rows of model g are routed into series slot g of the shared context, and every
+        spectrum's ``measure`` runs the chirp-z transform shared by the ranks on its slot.  The G spectra stay
+        valid together — measured in any order, any number of times — until the next ``get_raman_spectrum`` /
+        ``get_raman_spectra`` call of the same size.  Otherwise, or if symmetric memory is unavailable: the
+        local block is swept and one ``all_gather_into_tensor`` per model assembles the series on every rank."""
+        models = list(polarizability_models)
+        if shared:
+            spectra = self._get_raman_spectra_shared(models)
+            if spectra is not None:
+                return spectra
+        import torch  # pylint: disable=import-outside-toplevel
+        import torch.distributed as dist  # pylint: disable=import-outside-toplevel
+
+        bounds = shard_bounds(self._num_frames, dist.get_world_size(self._group), dist.get_rank(self._group))
+        spectra = []
+        for local in self._local.get_raman_spectra(models):
+            series = local._polarizability_ts  # pylint: disable=protected-access
+            if not hasattr(series, "data_ptr"):
+                series = torch.from_numpy(series)
+            full = allgather_series(series, self._num_frames, self._group)
+            spectra.append(ShardedMDRamanSpectrum(full, self._local.timestep, self._group, bounds=bounds))
+        return spectra
+
+    def _get_raman_spectra_shared(self, models):
+        import torch  # pylint: disable=import-outside-toplevel
+        import torch.distributed as dist  # pylint: disable=import-outside-toplevel
+
+        from .pmodel import InterpolationModel, calc_polarizabilities_sweep_routed  # pylint: disable=import-outside-toplevel
+
+        # anything the sweep rejects (no models, more than 64, foreign models) raises on the all-gather path
+        if not 1 <= len(models) <= 64 or not all(isinstance(m, InterpolationModel) for m in models):
+            return None
+        if not torch.cuda.is_available() or dist.get_backend(self._group) != "nccl":
+            return None
+        world, rank = dist.get_world_size(self._group), dist.get_rank(self._group)
+        if world == 1 or world > 8 or self._num_frames < 2:
+            return None
+        positions = self._local._positions_ts  # pylint: disable=protected-access
+        device = positions.device if hasattr(positions, "data_ptr") else torch.device("cuda", torch.cuda.current_device())
+        ctx = _shared_context(self._num_frames, device, self._group, slots=len(models))
+        if ctx is None:
+            return None
+        start, stop = shard_bounds(self._num_frames, world, rank)
+        local_ptrs = [ctx.ptr(rank, "series", g) + start * 72 for g in range(len(models))]
+        peers = [[0 if r == rank else ctx.ptr(r, "series", g) for r in range(world)] for g in range(len(models))]
+        if ctx.pack_event is not None:  # a first pack half that no measure() waited for still reads the buffers
+            torch.cuda.current_stream(device).wait_event(ctx.pack_event)
+            ctx.pack_event = None
+        try:
+            calc_polarizabilities_sweep_routed(models, positions, local_ptrs, peers, start, ctx.period, ctx.width)
+        except ValueError as exc:
+            raise ValueError("polarizability_model and trajectory are incompatible") from exc
+        ctx.generation += 1
+        ctx.barrier()  # every rank's rows of every mask have landed where they are consumed
+        return [ShardedMDRamanSpectrum(None, self._local.timestep, self._group, context=ctx, generation=ctx.generation,
+                                       bounds=(start, stop), slot=g) for g in range(len(models))]
 
     def _phased(self, ctx, model, positions, start: int) -> bool:
         """True if EVERY rank can evaluate its block in the two phases of the overlapped schedule (decided

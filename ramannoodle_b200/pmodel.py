@@ -379,14 +379,8 @@ class InterpolationModel(PolarizabilityModel):
         return alpha
 
 
-def calc_polarizabilities_sweep(models, positions_batch, to_device: bool = False):
-    """Evaluate several models of ONE structure (typically ``get_masked_model`` copies,
-    ``_interpolation.py:697-708``) on the same positions in one pass: returns ``(G,S,3,3)``.
-
-    A host trajectory crosses PCIe once; purely linear models (every ``ARTModel``) are contracted
-    together by one kernel (``rn_calc_polarizabilities_sweep``), other models run one after the other
-    on the resident positions.  Each slice equals ``models[g].calc_polarizabilities(positions_batch)``.
-    numpy in -> numpy out (a CUDA tensor if ``to_device``); CUDA tensor in -> CUDA tensor out."""
+def _sweep_inputs(models, positions_batch):
+    """Validated models and positions of a sweep: (models, contiguous float64 positions, device, is_tensor)."""
     import torch  # pylint: disable=import-outside-toplevel
 
     models = list(models)
@@ -410,14 +404,28 @@ def calc_polarizabilities_sweep(models, positions_batch, to_device: bool = False
         raise get_shape_error("positions", positions_batch, f"(_,{num_atoms},3)")
     for model in models:
         model._check_dummy()  # pylint: disable=protected-access
-    count = len(models)
-    num_frames = int(positions_batch.shape[0])
     if is_tensor:
         data = positions_batch.to(torch.float64).contiguous()
         device = models[0]._resolve_device(data)  # pylint: disable=protected-access
     else:
         data = np.ascontiguousarray(positions_batch, dtype=np.float64)
         device = models[0]._resolve_device()  # pylint: disable=protected-access
+    return models, data, device, is_tensor
+
+
+def calc_polarizabilities_sweep(models, positions_batch, to_device: bool = False):
+    """Evaluate several models of ONE structure (typically ``get_masked_model`` copies,
+    ``_interpolation.py:697-708``) on the same positions in one pass: returns ``(G,S,3,3)``.
+
+    A host trajectory crosses PCIe once; purely linear models (every ``ARTModel``) are contracted
+    together by one kernel (``rn_calc_polarizabilities_sweep``), other models run one after the other
+    on the resident positions.  Each slice equals ``models[g].calc_polarizabilities(positions_batch)``.
+    numpy in -> numpy out (a CUDA tensor if ``to_device``); CUDA tensor in -> CUDA tensor out."""
+    import torch  # pylint: disable=import-outside-toplevel
+
+    models, data, device, is_tensor = _sweep_inputs(models, positions_batch)
+    count = len(models)
+    num_frames = int(data.shape[0])
     natives = [model._native_model(device) for model in models]  # pylint: disable=protected-access
     handles = (ctypes.c_void_p * count)(*[native.handle for native in natives])
     with torch.cuda.device(device):
@@ -435,6 +443,43 @@ def calc_polarizabilities_sweep(models, positions_batch, to_device: bool = False
         status = _lib.lib().rn_calc_polarizabilities_host_sweep(handles, count, _ptr(data), num_frames, outputs, 0)
         _lib.check(status, "rn_calc_polarizabilities_host_sweep")
     return alpha if to_device else alpha.cpu().numpy()
+
+
+# pylint: disable=too-many-arguments,too-many-positional-arguments,too-many-locals
+def calc_polarizabilities_sweep_routed(models, positions_batch, local_ptrs, peer_series, first_frame: int,
+                                       period: int, width: int, chunk_frames: int = 0) -> None:
+    """Mask sweep of this rank's block for the shared multi-GPU spectrum
+    (``rn_calc_polarizabilities_sweep_routed``): model g's rows go to ``local_ptrs[g]`` (this rank's block
+    inside its own series buffer of mask g) and, written by the kernels over NVLink, to
+    ``peer_series[g][r]`` (base pointers of mask g's series buffer on rank r, 0 for this rank) for the
+    ranks that consume them, as in ``InterpolationModel.calc_polarizabilities_routed``.  A host block
+    crosses PCIe once for all models (in chunks of ``chunk_frames``, 0 = automatic)."""
+    import torch  # pylint: disable=import-outside-toplevel
+
+    models, data, device, is_tensor = _sweep_inputs(models, positions_batch)
+    count = len(models)
+    if len(local_ptrs) != count or len(peer_series) != count:
+        raise ValueError("one local pointer and one row of peer pointers per model are required")
+    world = len(peer_series[0])
+    if not 1 <= world <= 8 or any(len(row) != world for row in peer_series):
+        raise ValueError("between 1 and 8 ranks, the same number for every model")
+    natives = [model._native_model(device) for model in models]  # pylint: disable=protected-access
+    handles = (ctypes.c_void_p * count)(*[native.handle for native in natives])
+    outputs = (ctypes.c_void_p * count)(*[ctypes.c_void_p(int(ptr)) for ptr in local_ptrs])
+    peers = (ctypes.c_void_p * (count * world))(*[ctypes.c_void_p(int(ptr)) if ptr else None
+                                                  for row in peer_series for ptr in row])
+    num_frames = int(data.shape[0])
+    with torch.cuda.device(device):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+        if is_tensor:
+            status = _lib.lib().rn_calc_polarizabilities_sweep_routed(
+                handles, count, ctypes.c_void_p(data.data_ptr()), num_frames, outputs, peers, world, int(first_frame),
+                int(period), int(width), stream)
+        else:
+            status = _lib.lib().rn_calc_polarizabilities_host_sweep_routed(
+                handles, count, _ptr(data), num_frames, outputs, peers, world, int(first_frame), int(period),
+                int(width), int(chunk_frames), stream)
+    _lib.check(status, "rn_calc_polarizabilities_sweep_routed")
 
 
 class ARTModel(InterpolationModel):
