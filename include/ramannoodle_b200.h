@@ -198,6 +198,19 @@ int64_t rn_spectrum_num_points(int64_t num_frames);
 int rn_md_spectrum(rn_spectrum_plan* plan, const double* d_alpha, double timestep_fs,
                    int laser_correction, double laser_wavelength_nm, int bose_einstein_correction,
                    double temperature_K, double* d_wavenumbers, double* d_intensities, void* stream);
+/* Windowed spectra (no reference counterpart; each row is rn_md_spectrum of one slice).
+ * rn_spectrum_plan_create_batched: a single-GPU plan for windows of window_frames frames whose work,
+ * power, energy-partial and ticket buffers hold `batch` windows (1 .. 65535; batch = 1 is
+ * rn_spectrum_plan_create).  rn_md_spectrum also accepts such a plan.
+ * rn_md_spectrum_windows: d_alpha (num_frames,3,3) -> d_wavenumbers (P,), d_intensities (W,P) with
+ * P = rn_spectrum_num_points(window_frames), W = 1 + (num_frames - window_frames) / hop_frames;
+ * row w is rn_md_spectrum of frames [w hop_frames, w hop_frames + window_frames).  Trailing frames
+ * that fill no window are not read.  The windows run in chunks of `batch` on `stream`. */
+int rn_spectrum_plan_create_batched(int64_t window_frames, int64_t batch, int device, rn_spectrum_plan** out);
+int rn_md_spectrum_windows(rn_spectrum_plan* plan, const double* d_alpha, int64_t num_frames, int64_t hop_frames,
+                           double timestep_fs, int laser_correction, double laser_wavelength_nm,
+                           int bose_einstein_correction, double temperature_K, double* d_wavenumbers,
+                           double* d_intensities, void* stream);
 /* One transform shared by the ranks of a multi-GPU run (one process per GPU; no reference
  * counterpart — same result as rn_md_spectrum on the whole series).  The chirp-z transform of
  * length L is decimated in frequency over the G = 2, 4 or 8 ranks of the group (the largest power

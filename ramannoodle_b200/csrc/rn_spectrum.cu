@@ -51,6 +51,7 @@ struct rn_spectrum_plan {
     double* d_epart = nullptr;  // energy partial of every pack block, then their sum
     unsigned int* d_ticket = nullptr;
     int pack_blocks = 0;
+    int64_t batch = 1;      // windows the work, power, partial and ticket buffers hold (single-GPU plans)
 };
 
 namespace rn {
@@ -102,6 +103,7 @@ struct PackParams {
     int log2_stripe;       // >= 0: this launch packs one half of every block of 2^(log2_stripe+1) n' ...
     int phase;             // ... the first (0) or the second (1)
     Twiddles tw;
+    int64_t win_stride;    // windowed pack: doubles between the series of windows blockIdx.y and blockIdx.y + 1
 };
 
 // block reduction of one double (fixed tree: bit-reproducible), result valid in thread 0
@@ -148,11 +150,27 @@ __device__ __forceinline__ void publish_energy(double block_total, double* epart
 
 // MD series: np.diff (_raman.py:282), the six weighted signals, chirp pre-multiply; with G > 1 the
 // G-point DFT over the blocks q (inputs q >= G/2 are zero: M <= L/2) and the twiddle W_L^{r n'}.
-template <int G>
+// WIN (G == 1): blockIdx.y numbers a window of a batch; window w reads the series at src + w win_stride,
+// packs into its own 3 Lh of dst[0] and sums its energy with its own partials and ticket, exactly as a
+// single-window launch does.
+template <int G, bool WIN = false>
 __global__ void __launch_bounds__(kPackThreads) pack_alpha_kernel(const __grid_constant__ PackParams P) {
+    static_assert(!WIN || G == 1, "windows are packed for single-GPU transforms only");
     constexpr int GH = G > 1 ? G / 2 : 1;
     __shared__ __align__(16) double rows[(kPackThreads + 1) * 9 + 1];
     __shared__ double red[kPackThreads / 32];
+    const double* src = P.src;
+    double2* dst0 = P.dst[0];
+    double* epart = P.epart;
+    unsigned int* ticket = P.ticket;
+    bool aligned16 = P.aligned16;
+    if constexpr (WIN) {
+        src += (int64_t)blockIdx.y * P.win_stride;
+        dst0 += (int64_t)blockIdx.y * 3 * P.Lh;
+        epart += (int64_t)blockIdx.y * (gridDim.x + 1);
+        ticket += blockIdx.y;
+        aligned16 = reinterpret_cast<uintptr_t>(src) % 16 == 0;  // 72 hop bytes: odd hops alternate
+    }
     int64_t n0 = P.begin + (int64_t)blockIdx.x * kPackThreads;
     if (P.log2_stripe >= 0) {  // stripes are multiples of the block size: a block stays inside one stripe
         const int64_t idx = (int64_t)blockIdx.x * kPackThreads, stripe = (int64_t)1 << P.log2_stripe;
@@ -167,19 +185,19 @@ __global__ void __launch_bounds__(kPackThreads) pack_alpha_kernel(const __grid_c
         const int64_t avail = min((int64_t)kPackThreads + 1, P.M + 1 - first);  // series rows first .. first+avail-1
         __syncthreads();
         const int64_t valid = avail > 0 ? avail * 9 : 0;  // doubles of the series this block may read
-        if (P.aligned16) {
+        if (aligned16) {
             // independent 16-byte loads, all in flight before the first store (first * 72 bytes is a multiple of 16:
             // block starts are even)
             constexpr int kVec = ((kPackThreads + 1) * 9 + 1) / 2;
             constexpr int kPer = (kVec + kPackThreads - 1) / kPackThreads;
-            const double2* src2 = reinterpret_cast<const double2*>(P.src + first * 9);
+            const double2* src2 = reinterpret_cast<const double2*>(src + first * 9);
             double2 staged[kPer];
 #pragma unroll
             for (int i = 0; i < kPer; i++) {
                 const int e = threadIdx.x + i * kPackThreads;
                 staged[i] = make_double2(0.0, 0.0);
                 if (2 * e + 1 < valid) staged[i] = __ldg(src2 + e);
-                else if (2 * e < valid) staged[i].x = __ldg(P.src + first * 9 + 2 * e);
+                else if (2 * e < valid) staged[i].x = __ldg(src + first * 9 + 2 * e);
             }
 #pragma unroll
             for (int i = 0; i < kPer; i++) {
@@ -191,7 +209,7 @@ __global__ void __launch_bounds__(kPackThreads) pack_alpha_kernel(const __grid_c
             }
         } else {
             for (int e = threadIdx.x; e < (kPackThreads + 1) * 9; e += kPackThreads)
-                rows[e] = (e < valid) ? __ldg(P.src + first * 9 + e) : 0.0;
+                rows[e] = (e < valid) ? __ldg(src + first * 9 + e) : 0.0;
         }
         __syncthreads();
         const int64_t n = first + threadIdx.x;
@@ -215,7 +233,7 @@ __global__ void __launch_bounds__(kPackThreads) pack_alpha_kernel(const __grid_c
         if constexpr (G == 1) {
             if (n1 < P.M) {
 #pragma unroll
-                for (int s = 0; s < 3; s++) P.dst[0][(int64_t)s * P.Lh + n1] = a[0][s];
+                for (int s = 0; s < 3; s++) dst0[(int64_t)s * P.Lh + n1] = a[0][s];
             }
         } else {
             const double2 w1 = fft::tw_global(P.tw, (uint32_t)n1);  // W_L^{n'}
@@ -234,7 +252,7 @@ __global__ void __launch_bounds__(kPackThreads) pack_alpha_kernel(const __grid_c
     }
     if (P.seq_sel <= 0) {  // uniform over the grid
         const double total = block_sum(energy, red);
-        publish_energy(total, P.epart, P.ticket, red, G > 1 ? &P : nullptr);
+        publish_energy(total, epart, ticket, red, G > 1 ? &P : nullptr);
     }
 }
 
@@ -404,12 +422,23 @@ __global__ void __launch_bounds__(256) finish_dist_kernel(const double* __restri
 // I[k] = (P[k] + P[M-k]) / (4 L^2) + E/2 for k = 1 .. ceil(M/2)-1 (bin 0 dropped, _raman.py:299-301),
 // wavenumbers, laser / Bose-Einstein corrections (_raman.py:13-69,303-307).  power: (nseq, M);
 // epart: nparts energy partials summed in a fixed order by every block.
+// WIN: blockIdx.y numbers a window of a batch; window w reads sequences nseq w .. nseq w + nseq - 1 of power,
+// the partials at epart + w epart_stride, writes row w of int_out (points per row) and, for w = 0 only and
+// if wn_out is given, the wavenumbers.
+template <bool WIN = false>
 __global__ void __launch_bounds__(256) combine_md_kernel(const double* __restrict__ power, int nseq,
                                                          const double* __restrict__ epart, int nparts, int64_t M,
                                                          double scale, int64_t points, SpectrumParams prm,
-                                                         double* __restrict__ wn_out, double* __restrict__ int_out) {
+                                                         double* __restrict__ wn_out, double* __restrict__ int_out,
+                                                         int64_t epart_stride = 0) {
     __shared__ double red[8];
     __shared__ double s_energy;
+    if constexpr (WIN) {
+        power += (int64_t)blockIdx.y * nseq * M;
+        epart += (int64_t)blockIdx.y * epart_stride;
+        int_out += (int64_t)blockIdx.y * points;
+        if (blockIdx.y != 0) wn_out = nullptr;
+    }
     double v = 0.0;
     for (int b = threadIdx.x; b < nparts; b += blockDim.x) v += epart[b];
     const double total = block_sum(v, red);
@@ -421,7 +450,7 @@ __global__ void __launch_bounds__(256) combine_md_kernel(const double* __restric
         double sum = 0.0;
         for (int s = 0; s < nseq; s++) sum += power[(int64_t)s * M + k] + power[(int64_t)s * M + (M - k)];
         const double wn = wavenumber_of(k, M, prm.timestep);
-        wn_out[o] = wn;
+        if (!WIN || wn_out) wn_out[o] = wn;
         int_out[o] = corrected(sum * scale + econst, wn, prm);
     }
 }
@@ -570,11 +599,18 @@ static double2 unit_root(int64_t num, int64_t den) {
     return make_double2((double)cosl(ang), (double)-sinl(ang));
 }
 
-static int create_plan(int64_t num_frames, int device, int world, int rank, rn_spectrum_plan** out) {
+// largest batch of windows: gridDim.y of the windowed pack and combine
+constexpr int64_t kMaxBatch = 65535;
+
+static int create_plan(int64_t num_frames, int device, int world, int rank, rn_spectrum_plan** out,
+                       int64_t batch = 1) {
     RN_CHECK_ARG(out != nullptr, "out is null");
     *out = nullptr;
     RN_CHECK_ARG(num_frames >= 2, "a spectrum needs at least 2 frames (got %lld)", (long long)num_frames);
     RN_CHECK_ARG(world >= 1 && world <= 8 && rank >= 0 && rank < world, "invalid rank %d of %d", rank, world);
+    RN_CHECK_ARG(batch >= 1 && batch <= kMaxBatch && (batch == 1 || world == 1),
+                 "invalid batch %lld (1 .. %lld windows, single-GPU plans only)", (long long)batch,
+                 (long long)kMaxBatch);
     int count = 0;
     RN_CUDA(cudaGetDeviceCount(&count));
     RN_CHECK_ARG(device >= 0 && device < count, "device %d out of range (%d devices)", device, count);
@@ -592,7 +628,11 @@ static int create_plan(int64_t num_frames, int device, int world, int rank, rn_s
     int log2l = kLog2E;
     while (((int64_t)1 << log2l) < std::max<int64_t>(2 * M - 1, (int64_t)kE * group)) log2l++;
     RN_CHECK_ARG(log2l <= 30, "series too long for one spectrum plan (%lld frames)", (long long)num_frames);
+    // the level and tile passes launch 3 batch L / 4096 blocks along gridDim.x
+    RN_CHECK_ARG(3 * batch * (((int64_t)1 << log2l) >> kLog2E) <= (int64_t)INT32_MAX,
+                 "batch %lld too large for windows of %lld frames", (long long)batch, (long long)num_frames);
     rn_spectrum_plan* p = new rn_spectrum_plan();
+    p->batch = batch;
     p->device = device;
     p->sm_count = prop.multiProcessorCount;
     p->S = num_frames;
@@ -631,10 +671,12 @@ static int create_plan(int64_t num_frames, int device, int world, int rank, rn_s
     alloc((void**)&p->d_wlo, sizeof(double2) * n_lo);
     alloc((void**)&p->d_wsub, sizeof(double2) * kE);
     alloc((void**)&p->d_H, sizeof(double2) * p->Lh);
-    alloc((void**)&p->d_work, sizeof(double2) * (group > 1 ? 1 : 3) * p->Lh);
-    if (group == 1) alloc((void**)&p->d_power, sizeof(double) * 3 * M);
-    alloc((void**)&p->d_epart, sizeof(double) * 2 * (p->pack_blocks + 1));  // two pack phases
-    alloc((void**)&p->d_ticket, 2 * sizeof(unsigned int));
+    // partials and tickets: two pack phases (shared transforms) or one set per window
+    const int64_t psets = std::max<int64_t>(2, batch);
+    alloc((void**)&p->d_work, sizeof(double2) * (group > 1 ? 1 : 3 * batch) * p->Lh);
+    if (group == 1) alloc((void**)&p->d_power, sizeof(double) * 3 * batch * M);
+    alloc((void**)&p->d_epart, sizeof(double) * psets * (p->pack_blocks + 1));
+    alloc((void**)&p->d_ticket, psets * sizeof(unsigned int));
     if (err != cudaSuccess) {
         set_error("cudaMalloc failed while creating a spectrum plan for %lld frames: %s", (long long)num_frames,
                   cudaGetErrorString(err));
@@ -642,7 +684,7 @@ static int create_plan(int64_t num_frames, int device, int world, int rank, rn_s
         cudaGetLastError();
         return RN_ERR_OUT_OF_MEMORY;
     }
-    cudaMemset(p->d_ticket, 0, 2 * sizeof(unsigned int));
+    cudaMemset(p->d_ticket, 0, psets * sizeof(unsigned int));
     std::vector<double2> whi((size_t)n_hi), wlo((size_t)n_lo), wsub((size_t)kE);
     for (int64_t a = 0; a < n_hi; a++) whi[(size_t)a] = unit_root(a << p->split, p->L);
     for (int64_t b = 0; b < n_lo; b++) wlo[(size_t)b] = unit_root(b, p->L);
@@ -689,6 +731,31 @@ static SpectrumParams spectrum_params(double timestep_fs, int laser, double lase
     return prm;
 }
 
+// pack of one whole (S,3,3) series on a single-GPU plan into its first work buffer
+static PackParams md_pack_params(const rn_spectrum_plan* plan, const double* d_alpha) {
+    PackParams pp;
+    pp.src = d_alpha;
+    pp.M = plan->M;
+    pp.Lh = plan->Lh;
+    pp.begin = 0;
+    pp.end = plan->M;
+    for (int i = 0; i < 8; i++) pp.dst[i] = nullptr;
+    pp.dst[0] = plan->d_work;
+    pp.aligned16 = (reinterpret_cast<uintptr_t>(pp.src) % 16 == 0) ? 1 : 0;
+    pp.seq_sel = -1;
+    pp.num_share = 0;
+    pp.share_slot = 0;
+    pp.zero_slot = -1;
+    pp.log2_stripe = -1;
+    pp.phase = 0;
+    for (int i = 0; i < 8; i++) pp.share[i] = nullptr;
+    pp.epart = plan->d_epart;
+    pp.ticket = plan->d_ticket;
+    pp.tw = plan_twiddles(plan);
+    pp.win_stride = 0;
+    return pp;
+}
+
 }  // namespace rn
 
 using namespace rn;
@@ -701,6 +768,11 @@ extern "C" int64_t rn_spectrum_num_points(int64_t num_frames) {
 
 extern "C" int rn_spectrum_plan_create(int64_t num_frames, int device, rn_spectrum_plan** out) {
     return create_plan(num_frames, device, 1, 0, out);
+}
+
+extern "C" int rn_spectrum_plan_create_batched(int64_t window_frames, int64_t batch, int device,
+                                               rn_spectrum_plan** out) {
+    return create_plan(window_frames, device, 1, 0, out, batch);
 }
 
 extern "C" int rn_spectrum_plan_create_dist(int64_t num_frames, int device, int world, int rank,
@@ -744,25 +816,7 @@ extern "C" int rn_md_spectrum(rn_spectrum_plan* plan, const double* d_alpha, dou
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const int64_t M = plan->M;
 
-    PackParams pp;
-    pp.src = d_alpha;
-    pp.M = M;
-    pp.Lh = plan->Lh;
-    pp.begin = 0;
-    pp.end = M;
-    for (int i = 0; i < 8; i++) pp.dst[i] = nullptr;
-    pp.dst[0] = plan->d_work;
-    pp.aligned16 = (reinterpret_cast<uintptr_t>(pp.src) % 16 == 0) ? 1 : 0;
-    pp.seq_sel = -1;
-    pp.num_share = 0;
-    pp.share_slot = 0;
-    pp.zero_slot = -1;
-    pp.log2_stripe = -1;
-    pp.phase = 0;
-    for (int i = 0; i < 8; i++) pp.share[i] = nullptr;
-    pp.epart = plan->d_epart;
-    pp.ticket = plan->d_ticket;
-    pp.tw = plan_twiddles(plan);
+    const PackParams pp = md_pack_params(plan, d_alpha);
     pack_alpha_kernel<1><<<plan->pack_blocks, kPackThreads, 0, s>>>(pp);
     RN_LAUNCHED();
     fft::OutSpec out = plain_out();
@@ -778,6 +832,53 @@ extern "C" int rn_md_spectrum(rn_spectrum_plan* plan, const double* d_alpha, dou
                                                                       M, scale, points, prm, d_wavenumbers, d_intensities);
     RN_LAUNCHED();
     RN_CUDA(cudaGetLastError());
+    return RN_OK;
+}
+
+// Every window of a batch runs the arithmetic of rn_md_spectrum on its slice in the same order: the pack
+// reads it at its own offset and sums its energy with its own partials, the convolution treats the 3 nb
+// sequences independently, the combine reads its own three rows of power and its own energy.
+extern "C" int rn_md_spectrum_windows(rn_spectrum_plan* plan, const double* d_alpha, int64_t num_frames,
+                                      int64_t hop_frames, double timestep_fs, int laser_correction,
+                                      double laser_wavelength_nm, int bose_einstein_correction, double temperature_K,
+                                      double* d_wavenumbers, double* d_intensities, void* stream) {
+    RN_CHECK_ARG(plan != nullptr, "plan is null");
+    RN_CHECK_ARG(plan->world == 1, "rn_md_spectrum_windows needs a single-GPU plan (rn_spectrum_plan_create_batched)");
+    RN_CHECK_ARG(d_alpha != nullptr, "d_alpha is null");
+    RN_CHECK_ARG(num_frames >= plan->S, "a window of %lld frames does not fit a series of %lld frames",
+                 (long long)plan->S, (long long)num_frames);
+    RN_CHECK_ARG(hop_frames >= 1, "hop_frames must be at least 1 (got %lld)", (long long)hop_frames);
+    RN_CHECK_ARG(timestep_fs > 0, "timestep must be positive");
+    if (laser_correction) RN_CHECK_ARG(laser_wavelength_nm > 0, "invalid laser_wavelength");
+    if (bose_einstein_correction) RN_CHECK_ARG(temperature_K > 0, "invalid temperature: %g <= 0", temperature_K);
+    const int64_t points = rn_spectrum_num_points(plan->S);
+    if (points == 0) return RN_OK;
+    RN_CHECK_ARG(d_wavenumbers && d_intensities, "null output pointer");
+    DeviceGuard guard(plan->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int64_t M = plan->M;
+    const int64_t windows = 1 + (num_frames - plan->S) / hop_frames;
+    const SpectrumParams prm = spectrum_params(timestep_fs, laser_correction, laser_wavelength_nm,
+                                               bose_einstein_correction, temperature_K);
+    const double scale = 0.25 / ((double)plan->L * (double)plan->L);
+    for (int64_t first = 0; first < windows; first += plan->batch) {
+        const int64_t nb = std::min(plan->batch, windows - first);
+        PackParams pp = md_pack_params(plan, d_alpha + first * hop_frames * 9);
+        pp.win_stride = hop_frames * 9;
+        pack_alpha_kernel<1, true><<<dim3(plan->pack_blocks, (unsigned)nb), kPackThreads, 0, s>>>(pp);
+        RN_LAUNCHED();
+        fft::OutSpec out = plain_out();
+        out.mode = fft::OUT_POWER;
+        out.power = plan->d_power;
+        out.M = M;
+        int rc = run_convolution(plan, plan->d_work, (int)(3 * nb), M, out, nullptr, s);
+        if (rc != RN_OK) return rc;
+        combine_md_kernel<true><<<dim3(grid_for(points, plan->sm_count), (unsigned)nb), 256, 0, s>>>(
+            plan->d_power, 3, plan->d_epart + plan->pack_blocks, 1, M, scale, points, prm,
+            first == 0 ? d_wavenumbers : nullptr, d_intensities + first * points, plan->pack_blocks + 1);
+        RN_LAUNCHED();
+        RN_CUDA(cudaGetLastError());
+    }
     return RN_OK;
 }
 

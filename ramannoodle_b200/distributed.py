@@ -31,7 +31,7 @@ from . import _lib
 from .abstract import Dynamics
 from .dynamics import Trajectory
 from .exceptions import get_type_error
-from .spectrum import MDRamanSpectrum, _stream
+from .spectrum import MDRamanSpectrum, _check_measure_args, _check_window_args, _measure_windows, _stream
 
 
 def shard_bounds(num_frames: int, world_size: int, rank: int) -> tuple[int, int]:
@@ -307,6 +307,23 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
         if self._context is not None:
             return self._gathered().cpu().numpy()
         return MDRamanSpectrum.polarizability_ts.fget(self)
+
+    # pylint: disable=too-many-arguments,too-many-positional-arguments
+    def measure_windows_device(self, window_frames, hop_frames=None, orientation="polycrystalline",
+                               laser_correction=False, laser_wavelength=522, bose_einstein_correction=False,
+                               temperature=300):
+        """``MDRamanSpectrum.measure_windows_device`` of the whole series; every rank returns all W rows.
+
+        With a shared context the series is first assembled on every rank (an all-gather on first use, as
+        for ``polarizability_ts``): every rank of the group must call it.  The windows then run on the
+        local GPU."""
+        if self._context is None:
+            return super().measure_windows_device(window_frames, hop_frames, orientation, laser_correction,
+                                                  laser_wavelength, bose_einstein_correction, temperature)
+        hop = _check_window_args(window_frames, hop_frames, int(self._context.num_frames))
+        _check_measure_args(orientation, laser_correction, laser_wavelength, bose_einstein_correction, temperature)
+        return _measure_windows(self._gathered(), self._timestep, int(window_frames), hop, laser_correction,
+                                laser_wavelength, bose_einstein_correction, temperature)
 
     # pylint: disable=too-many-arguments,too-many-positional-arguments,too-many-locals
     def measure_device(self, orientation="polycrystalline", laser_correction=False, laser_wavelength=522,

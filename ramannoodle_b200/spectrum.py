@@ -42,12 +42,16 @@ def _stream(device: int) -> ctypes.c_void_p:
 
 
 class _Plan:
-    """``rn_spectrum_plan`` for one series length on one device."""
+    """``rn_spectrum_plan`` for one series length on one device (``batch`` windows of that length)."""
 
-    def __init__(self, num_frames: int, device: int) -> None:
+    def __init__(self, num_frames: int, device: int, batch: int = 1) -> None:
         handle = ctypes.c_void_p()
-        _lib.check(_lib.lib().rn_spectrum_plan_create(num_frames, device, ctypes.byref(handle)),
-                   "rn_spectrum_plan_create")
+        if batch == 1:
+            _lib.check(_lib.lib().rn_spectrum_plan_create(num_frames, device, ctypes.byref(handle)),
+                       "rn_spectrum_plan_create")
+        else:
+            _lib.check(_lib.lib().rn_spectrum_plan_create_batched(num_frames, batch, device, ctypes.byref(handle)),
+                       "rn_spectrum_plan_create_batched")
         self.handle = handle
 
     def close(self) -> None:
@@ -67,7 +71,7 @@ _PLAN_CACHE_SIZE = 4
 _PLAN_CACHE_LOCK = threading.Lock()
 
 
-def _get_plan(num_frames: int, device: int) -> _Plan:
+def _get_plan(num_frames: int, device: int, batch: int = 1) -> _Plan:
     """A plan owns its work buffers, so it is shared only by calls that are ordered anyway: the same
     Python thread AND the same CUDA stream (two streams or two threads measuring series of the same length
     would otherwise race on the buffers)."""
@@ -79,19 +83,20 @@ def _get_plan(num_frames: int, device: int) -> _Plan:
             stream_id = int(torch.cuda.current_stream(device).cuda_stream)
     except (ImportError, RuntimeError):
         stream_id = 0
-    key = (int(num_frames), int(device), stream_id, threading.get_ident())
+    key = (int(num_frames), int(device), stream_id, threading.get_ident(), int(batch))
     with _PLAN_CACHE_LOCK:
-        return _get_plan_locked(key, num_frames, device)
+        return _get_plan_locked(key, num_frames, device, batch)
 
 
-def _get_plan_locked(key, num_frames: int, device: int) -> _Plan:
+def _get_plan_locked(key, num_frames: int, device: int, batch: int = 1) -> _Plan:
     plan = _PLAN_CACHE.get(key)
     if plan is None:
         _lib.require_device(device)
         while len(_PLAN_CACHE) >= _PLAN_CACHE_SIZE:
             _, old = _PLAN_CACHE.popitem(last=False)
             old.close()
-        plan = _Plan(num_frames, device)
+        # a plan of one window is built with the two-argument form the single-series callers have always used
+        plan = _Plan(num_frames, device) if batch == 1 else _Plan(num_frames, device, batch)
         _PLAN_CACHE[key] = plan
     else:
         _PLAN_CACHE.move_to_end(key)
@@ -170,22 +175,7 @@ class MDRamanSpectrum(RamanSpectrum):
     def measure_device(self, orientation="polycrystalline", laser_correction=False, laser_wavelength=522,
                        bose_einstein_correction=False, temperature=300):
         """``measure`` with the result left on the GPU (two CUDA tensors)."""
-        if orientation != "polycrystalline":
-            raise NotImplementedError("only polycrystalline spectra are supported for now")
-        laser_wavenumber = None
-        if laser_correction:
-            laser_wavenumber = 10000000 / laser_wavelength
-            try:
-                if laser_wavenumber <= 0:
-                    raise ValueError(f"invalid laser_wavenumber: {laser_wavenumber} <= 0")
-            except TypeError as exc:
-                raise get_type_error("laser_wavenumber", laser_wavenumber, "float") from exc
-        if bose_einstein_correction:
-            try:
-                if temperature <= 0:
-                    raise ValueError(f"invalid temperature: {temperature} <= 0")
-            except TypeError as exc:
-                raise get_type_error("temperature", temperature, "float") from exc
+        _check_measure_args(orientation, laser_correction, laser_wavelength, bose_einstein_correction, temperature)
         torch = _torch()
         series = self._device_series()
         num_frames = int(series.shape[0])
@@ -213,6 +203,122 @@ class MDRamanSpectrum(RamanSpectrum):
         wavenumbers, intensities = self.measure_device(orientation, laser_correction, laser_wavelength,
                                                        bose_einstein_correction, temperature)
         return wavenumbers.cpu().numpy(), intensities.cpu().numpy()
+
+    # pylint: disable=too-many-arguments,too-many-positional-arguments,too-many-locals
+    def measure_windows_device(self, window_frames, hop_frames=None, orientation="polycrystalline",
+                               laser_correction=False, laser_wavelength=522, bose_einstein_correction=False,
+                               temperature=300):
+        """``measure_windows`` with the result left on the GPU (two CUDA tensors)."""
+        hop = _check_window_args(window_frames, hop_frames, int(self._polarizability_ts.shape[0]))
+        _check_measure_args(orientation, laser_correction, laser_wavelength, bose_einstein_correction, temperature)
+        return _measure_windows(self._device_series(), self._timestep, int(window_frames), hop, laser_correction,
+                                laser_wavelength, bose_einstein_correction, temperature)
+
+    def measure_windows(self, window_frames, hop_frames=None, orientation="polycrystalline", laser_correction=False,
+                        laser_wavelength=522, bose_einstein_correction=False, temperature=300):
+        """Spectra of windows of the series -> (wavenumbers, intensities), numpy arrays of shape (P,) and
+        (W, P), P = ceil((window_frames-1)/2) - 1.
+
+        Window w covers frames [w*hop, w*hop + window_frames) with hop = ``hop_frames`` (default
+        ``window_frames``: contiguous blocks, for block averages); a smaller hop gives overlapping windows
+        (a spectrogram), a larger one leaves gaps.  W = 1 + (S - window_frames) // hop: trailing frames that
+        do not fill a window are not used.  Row w is by definition
+        ``MDRamanSpectrum(polarizability_ts[w*hop : w*hop + window_frames], timestep).measure(...)[1]``
+        with the same keyword arguments, and the wavenumbers are those of that call.  All windows run as
+        one batched transform on the GPU.
+        """
+        wavenumbers, intensities = self.measure_windows_device(window_frames, hop_frames, orientation,
+                                                               laser_correction, laser_wavelength,
+                                                               bose_einstein_correction, temperature)
+        return wavenumbers.cpu().numpy(), intensities.cpu().numpy()
+
+
+def _check_measure_args(orientation, laser_correction, laser_wavelength, bose_einstein_correction,
+                        temperature) -> None:
+    """The argument errors of ``measure`` (``_raman.py:241-309``)."""
+    if orientation != "polycrystalline":
+        raise NotImplementedError("only polycrystalline spectra are supported for now")
+    if laser_correction:
+        laser_wavenumber = 10000000 / laser_wavelength
+        try:
+            if laser_wavenumber <= 0:
+                raise ValueError(f"invalid laser_wavenumber: {laser_wavenumber} <= 0")
+        except TypeError as exc:
+            raise get_type_error("laser_wavenumber", laser_wavenumber, "float") from exc
+    if bose_einstein_correction:
+        try:
+            if temperature <= 0:
+                raise ValueError(f"invalid temperature: {temperature} <= 0")
+        except TypeError as exc:
+            raise get_type_error("temperature", temperature, "float") from exc
+
+
+def _is_integer(value) -> bool:
+    return isinstance(value, (int, np.integer)) and not isinstance(value, (bool, np.bool_))
+
+
+def _check_window_args(window_frames, hop_frames, num_frames: int) -> int:
+    """Validate the window of ``measure_windows`` on a series of ``num_frames`` frames; returns the hop."""
+    if not _is_integer(window_frames):
+        raise get_type_error("window_frames", window_frames, "int")
+    if hop_frames is not None and not _is_integer(hop_frames):
+        raise get_type_error("hop_frames", hop_frames, "int")
+    if not 2 <= window_frames <= num_frames:
+        raise ValueError(f"invalid window_frames: {window_frames} (a window needs 2 to {num_frames} frames)")
+    hop = int(window_frames) if hop_frames is None else int(hop_frames)
+    if hop < 1:
+        raise ValueError(f"invalid hop_frames: {hop_frames} < 1")
+    return hop
+
+
+def num_windows(num_frames: int, window_frames: int, hop_frames: int) -> int:
+    """W = 1 + (S - window_frames) // hop: the windows ``measure_windows`` returns."""
+    return 1 + (int(num_frames) - int(window_frames)) // int(hop_frames)
+
+
+# Device memory the batch buffers of one windowed plan may take: the windows run in chunks of as many
+# as fit.  Larger chunks need fewer launches; the work of a window does not change.  A cached plan keeps its
+# buffers after the call returns, so up to _PLAN_CACHE_SIZE windowed plans (4 GiB) can stay allocated; the
+# batch is rounded up to a power of two so that calls with similar window counts share one plan.
+_WINDOW_BATCH_BYTES = 1 << 30
+_MAX_WINDOW_BATCH = 65535  # gridDim.y of the windowed pack and combine
+
+
+def _window_batch(window_frames: int, windows: int) -> int:
+    """Windows per chunk: the smallest power of two >= ``windows``, capped by the budget.  Per window the plan
+    holds 3 work sequences of L complex values, 3 rows of M powers, the pack's energy partials and a ticket
+    (``create_plan`` in ``csrc/rn_spectrum.cu``)."""
+    m = window_frames - 1
+    log2l = 12  # the plan pads L up to at least 4096
+    while (1 << log2l) < max(2 * m - 1, 4096):
+        log2l += 1
+    pack_blocks = (m + 255) // 256
+    per_window = 16 * 3 * (1 << log2l) + 8 * 3 * m + 8 * (pack_blocks + 1) + 4
+    rounded = 1 << max(0, int(windows) - 1).bit_length()
+    return max(1, min(rounded, _WINDOW_BATCH_BYTES // per_window, _MAX_WINDOW_BATCH))
+
+
+# pylint: disable=too-many-arguments,too-many-positional-arguments
+def _measure_windows(series, timestep, window_frames: int, hop: int, laser_correction, laser_wavelength,
+                     bose_einstein_correction, temperature):
+    """``rn_md_spectrum_windows`` on a contiguous float64 CUDA series (arguments already checked)."""
+    torch = _torch()
+    num_frames = int(series.shape[0])
+    windows = num_windows(num_frames, window_frames, hop)
+    device = int(series.device.index or 0)
+    points = int(_lib.lib().rn_spectrum_num_points(window_frames))
+    with torch.cuda.device(device):
+        wavenumbers = torch.empty(points, dtype=torch.float64, device=series.device)
+        intensities = torch.empty((windows, points), dtype=torch.float64, device=series.device)
+        if points > 0:
+            plan = _get_plan(window_frames, device, _window_batch(window_frames, windows))
+            status = _lib.lib().rn_md_spectrum_windows(
+                plan.handle, ctypes.c_void_p(series.data_ptr()), num_frames, hop, float(timestep),
+                1 if laser_correction else 0, float(laser_wavelength) if laser_correction else 0.0,
+                1 if bose_einstein_correction else 0, float(temperature) if bose_einstein_correction else 0.0,
+                ctypes.c_void_p(wavenumbers.data_ptr()), ctypes.c_void_p(intensities.data_ptr()), _stream(device))
+            _lib.check(status, "rn_md_spectrum_windows")
+    return wavenumbers, intensities
 
 
 class PhononRamanSpectrum(RamanSpectrum):
