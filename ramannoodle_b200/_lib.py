@@ -192,3 +192,15 @@ def require_device(device: int = 0) -> dict:
 
 def launch_count() -> int:
     return int(lib().rn_launch_count())
+
+
+def is_torch_tensor(obj) -> bool:
+    """Whether ``obj`` is a torch tensor (checked without importing torch)."""
+    return type(obj).__module__.startswith("torch") and hasattr(obj, "data_ptr")
+
+
+def current_stream(device: int) -> ctypes.c_void_p:
+    """torch's current CUDA stream on ``device``, as the ``void* stream`` argument of the C-ABI."""
+    import torch  # pylint: disable=import-outside-toplevel
+
+    return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)

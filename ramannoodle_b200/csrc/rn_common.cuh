@@ -230,6 +230,16 @@ inline AlphaPeers no_peers() {
 __host__ __device__ inline int64_t alpha_peer_offset(const AlphaPeers& P, int64_t local_row) {
     return (P.log2_period < 0 ? local_row : P.first_frame + local_row) * 9;
 }
+// the destinations of local rows f0, f0 + 1, ... as a launch that starts at local row f0 sees them
+inline AlphaPeers peers_at(const AlphaPeers& P, int64_t f0) {
+    AlphaPeers Q = P;
+    if (P.log2_period < 0) {
+        for (int p = 0; p < P.count; p++) Q.ptr[p] = P.ptr[p] + f0 * 9;
+    } else {
+        Q.first_frame = P.first_frame + f0;
+    }
+    return Q;
+}
 
 // kernels / launchers implemented in rn_polarizability.cu / rn_dense.cu.  `peers` may be null;
 // *peers_done is set when the launched kernel stored to the peers itself.

@@ -92,8 +92,44 @@ extern "C" int rn_host_unregister(void* h_ptr) {
     return RN_OK;
 }
 
-// Shared implementation: d_alpha is the local series (or null when only h_alpha is wanted);
-// `peers` describes further destinations of the rows (broadcast or routed, rn_common.cuh).
+// The chunk loop of every host entry: chunk [f0, f0 + n) is copied into staging slot `slot` on that slot's
+// stream and evaluated there by step(d_pos, out, f0, n, stream) -> rn_status, so that the copy of one chunk
+// overlaps the evaluation of the other.  `out` is where the chunk's rows go: d_alpha + 9 f0, a staging buffer
+// when only h_alpha is given, null when neither is (a sweep stores to its own outputs); h_alpha receives the
+// rows of every chunk.
+template <class Step>
+static int host_chunks(int device, int64_t K, const double* h_positions, int64_t num_frames, int64_t chunk_frames,
+                       double* h_alpha, double* d_alpha, void* stream, Step step) {
+    DeviceGuard guard(device);
+    if (!guard.ok) {
+        set_error("cudaSetDevice(%d) failed", device);
+        return RN_ERR_CUDA;
+    }
+    chunk_frames = pick_chunk(chunk_frames, num_frames, K);
+    const bool stage_alpha = h_alpha && !d_alpha;
+    HostPipe* pipe = nullptr;
+    int rc = acquire_pipe(device, chunk_frames * K, stage_alpha ? chunk_frames * 9 : 0, &pipe);
+    if (rc != RN_OK) return rc;
+    rc = order_after_caller(*pipe, static_cast<cudaStream_t>(stream));
+    if (rc != RN_OK) return rc;
+    int slot = 0;
+    for (int64_t f0 = 0; f0 < num_frames; f0 += chunk_frames, slot ^= 1) {
+        const int64_t n = std::min(chunk_frames, num_frames - f0);
+        cudaStream_t s = pipe->stream[slot];
+        // stream order serialises reuse of this slot's buffers; the other slot overlaps
+        RN_CUDA(cudaMemcpyAsync(pipe->d_pos[slot], h_positions + f0 * K, sizeof(double) * n * K, cudaMemcpyHostToDevice, s));
+        double* out = d_alpha ? d_alpha + f0 * 9 : stage_alpha ? pipe->d_alpha[slot] : nullptr;
+        rc = step(pipe->d_pos[slot], out, f0, n, s);
+        if (rc != RN_OK) return rc;
+        if (h_alpha) RN_CUDA(cudaMemcpyAsync(h_alpha + f0 * 9, out, sizeof(double) * n * 9, cudaMemcpyDeviceToHost, s));
+    }
+    RN_CUDA(cudaStreamSynchronize(pipe->stream[0]));
+    RN_CUDA(cudaStreamSynchronize(pipe->stream[1]));
+    return RN_OK;
+}
+
+// One model: d_alpha is the local series (or null when only h_alpha is wanted); `peers` describes further
+// destinations of the rows (broadcast or routed, rn_common.cuh).
 static int host_pipeline(const rn_model* model, const double* h_positions, int64_t num_frames, double* h_alpha,
                          double* d_alpha, const AlphaPeers& peers, int64_t chunk_frames, void* stream) {
     RN_CHECK_ARG(model != nullptr, "model is null");
@@ -101,39 +137,10 @@ static int host_pipeline(const rn_model* model, const double* h_positions, int64
     if (num_frames == 0) return RN_OK;
     RN_CHECK_ARG(h_positions != nullptr, "null host pointer");
     RN_CHECK_ARG(h_alpha || d_alpha, "no output buffer given");
-    DeviceGuard guard(model->device);
-    if (!guard.ok) {
-        set_error("cudaSetDevice(%d) failed", model->device);
-        return RN_ERR_CUDA;
-    }
-    const int64_t K = model->dim;
-    chunk_frames = pick_chunk(chunk_frames, num_frames, K);
-    HostPipe* pipe_ptr = nullptr;
-    int prc = acquire_pipe(model->device, chunk_frames * K, d_alpha ? 0 : chunk_frames * 9, &pipe_ptr);
-    if (prc != RN_OK) return prc;
-    HostPipe& pipe = *pipe_ptr;
-    prc = order_after_caller(pipe, static_cast<cudaStream_t>(stream));
-    if (prc != RN_OK) return prc;
-    int slot = 0;
-    for (int64_t f0 = 0; f0 < num_frames; f0 += chunk_frames, slot ^= 1) {
-        const int64_t n = std::min(chunk_frames, num_frames - f0);
-        cudaStream_t s = pipe.stream[slot];
-        // stream order serialises reuse of this slot's buffers; the other slot overlaps
-        RN_CUDA(cudaMemcpyAsync(pipe.d_pos[slot], h_positions + f0 * K, sizeof(double) * n * K, cudaMemcpyHostToDevice, s));
-        double* out = d_alpha ? d_alpha + f0 * 9 : pipe.d_alpha[slot];
-        AlphaPeers chunk_peers = peers;
-        if (peers.log2_period < 0) {
-            for (int p = 0; p < peers.count; p++) chunk_peers.ptr[p] = peers.ptr[p] + f0 * 9;
-        } else {
-            chunk_peers.first_frame = peers.first_frame + f0;
-        }
-        int rc = eval_with_peers(model, pipe.d_pos[slot], n, out, s, chunk_peers);
-        if (rc != RN_OK) return rc;
-        if (h_alpha) RN_CUDA(cudaMemcpyAsync(h_alpha + f0 * 9, out, sizeof(double) * n * 9, cudaMemcpyDeviceToHost, s));
-    }
-    RN_CUDA(cudaStreamSynchronize(pipe.stream[0]));
-    RN_CUDA(cudaStreamSynchronize(pipe.stream[1]));
-    return RN_OK;
+    return host_chunks(model->device, model->dim, h_positions, num_frames, chunk_frames, h_alpha, d_alpha, stream,
+                       [&](const double* d_pos, double* out, int64_t f0, int64_t n, cudaStream_t s) {
+                           return eval_with_peers(model, d_pos, n, out, s, peers_at(peers, f0));
+                       });
 }
 
 extern "C" int rn_calc_polarizabilities_host(const rn_model* model, const double* h_positions, int64_t num_frames,
@@ -165,7 +172,7 @@ extern "C" int rn_calc_polarizabilities_host_routed(const rn_model* model, const
 }
 
 // Mask sweep from a host trajectory: every chunk crosses PCIe once and is evaluated by all models.  `routed`
-// (null, or one entry per model) names the ranks the rows also go to; its first_frame is shifted per chunk.
+// (null, or one entry per model) names the ranks the rows also go to.
 static int host_sweep(const rn_model* const* models, int num_models, const double* h_positions, int64_t num_frames,
                       double* const* d_alpha_outputs, const AlphaPeers* routed, int64_t chunk_frames, void* stream) {
     RN_CHECK_ARG(models != nullptr && num_models >= 1 && num_models <= kMaxSweepModels, "1..64 models are required");
@@ -178,39 +185,16 @@ static int host_sweep(const rn_model* const* models, int num_models, const doubl
     RN_CHECK_ARG(num_frames >= 0, "num_frames must be non-negative");
     if (num_frames == 0) return RN_OK;
     RN_CHECK_ARG(h_positions != nullptr, "null host pointer");
-    const rn_model* model = models[0];
-    DeviceGuard guard(model->device);
-    if (!guard.ok) {
-        set_error("cudaSetDevice(%d) failed", model->device);
-        return RN_ERR_CUDA;
-    }
-    const int64_t K = model->dim;
-    chunk_frames = pick_chunk(chunk_frames, num_frames, K);
-    HostPipe* pipe = nullptr;
-    int rc = acquire_pipe(model->device, chunk_frames * K, 0, &pipe);
-    if (rc != RN_OK) return rc;
-    rc = order_after_caller(*pipe, static_cast<cudaStream_t>(stream));
-    if (rc != RN_OK) return rc;
-    int slot = 0;
-    AlphaPeers chunk_routed[kMaxSweepModels];
-    for (int64_t f0 = 0; f0 < num_frames; f0 += chunk_frames, slot ^= 1) {
-        const int64_t n = std::min(chunk_frames, num_frames - f0);
-        cudaStream_t s = pipe->stream[slot];
-        RN_CUDA(cudaMemcpyAsync(pipe->d_pos[slot], h_positions + f0 * K, sizeof(double) * n * K, cudaMemcpyHostToDevice, s));
-        double* outs[kMaxSweepModels];
-        for (int g = 0; g < num_models; g++) {
-            outs[g] = d_alpha_outputs[g] + f0 * 9;
-            if (routed) {
-                chunk_routed[g] = routed[g];
-                chunk_routed[g].first_frame = routed[g].first_frame + f0;
-            }
-        }
-        rc = sweep_eval(models, num_models, pipe->d_pos[slot], n, outs, s, routed ? chunk_routed : nullptr);
-        if (rc != RN_OK) return rc;
-    }
-    RN_CUDA(cudaStreamSynchronize(pipe->stream[0]));
-    RN_CUDA(cudaStreamSynchronize(pipe->stream[1]));
-    return RN_OK;
+    return host_chunks(models[0]->device, models[0]->dim, h_positions, num_frames, chunk_frames, nullptr, nullptr,
+                       stream, [&](const double* d_pos, double*, int64_t f0, int64_t n, cudaStream_t s) {
+                           double* outs[kMaxSweepModels];
+                           AlphaPeers chunk_routed[kMaxSweepModels];
+                           for (int g = 0; g < num_models; g++) {
+                               outs[g] = d_alpha_outputs[g] + f0 * 9;
+                               if (routed) chunk_routed[g] = peers_at(routed[g], f0);
+                           }
+                           return sweep_eval(models, num_models, d_pos, n, outs, s, routed ? chunk_routed : nullptr);
+                       });
 }
 
 extern "C" int rn_calc_polarizabilities_host_sweep(const rn_model* const* models, int num_models,

@@ -30,8 +30,7 @@ import warnings
 from . import _lib
 from .abstract import Dynamics
 from .dynamics import Trajectory
-from .exceptions import get_type_error
-from .spectrum import MDRamanSpectrum, _check_measure_args, _check_window_args, _measure_windows, _stream
+from .spectrum import MDRamanSpectrum, _check_measure_args, _check_window_args, _measure_windows
 
 
 def shard_bounds(num_frames: int, world_size: int, rank: int) -> tuple[int, int]:
@@ -333,21 +332,7 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
         if self._context is None:
             return super().measure_device(orientation, laser_correction, laser_wavelength,
                                           bose_einstein_correction, temperature)
-        if orientation != "polycrystalline":
-            raise NotImplementedError("only polycrystalline spectra are supported for now")
-        if laser_correction:
-            laser_wavenumber = 10000000 / laser_wavelength
-            try:
-                if laser_wavenumber <= 0:
-                    raise ValueError(f"invalid laser_wavenumber: {laser_wavenumber} <= 0")
-            except TypeError as exc:
-                raise get_type_error("laser_wavenumber", laser_wavenumber, "float") from exc
-        if bose_einstein_correction:
-            try:
-                if temperature <= 0:
-                    raise ValueError(f"invalid temperature: {temperature} <= 0")
-            except TypeError as exc:
-                raise get_type_error("temperature", temperature, "float") from exc
+        _check_measure_args(orientation, laser_correction, laser_wavelength, bose_einstein_correction, temperature)
         ctx = self._context
         self._check_live()
         if ctx.num_frames < 2:
@@ -360,7 +345,7 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
             intensities = torch.empty(points, dtype=torch.float64, device=ctx.device)
             if points == 0:
                 return wavenumbers, intensities
-            stream = _stream(device)
+            stream = _lib.current_stream(device)
             group = ctx.transform_ranks
             series_ptr = ctypes.c_void_p(ctx.ptr(ctx.rank, "series", self._slot))
             work_ptr = ctypes.c_void_p(ctx.ptr(ctx.rank, "work"))
@@ -469,17 +454,7 @@ class ShardedTrajectory(Dynamics):
             spectrum = self._get_raman_spectrum_shared(polarizability_model)
             if spectrum is not None:
                 return spectrum
-        local = self._local.get_raman_spectrum(polarizability_model)
-        series = local._polarizability_ts  # pylint: disable=protected-access
-        if not hasattr(series, "data_ptr"):
-            import torch  # pylint: disable=import-outside-toplevel
-
-            series = torch.from_numpy(series)
-        import torch.distributed as dist  # pylint: disable=import-outside-toplevel
-
-        full = allgather_series(series, self._num_frames, self._group)
-        bounds = shard_bounds(self._num_frames, dist.get_world_size(self._group), dist.get_rank(self._group))
-        return ShardedMDRamanSpectrum(full, self._local.timestep, self._group, bounds=bounds)
+        return self._allgather_spectrum(self._local.get_raman_spectrum(polarizability_model))
 
     def get_raman_spectra(self, polarizability_models, shared: bool = True) -> list:
         """Mask sweep (``Trajectory.get_raman_spectra``) of the sharded trajectory: one
@@ -497,18 +472,19 @@ class ShardedTrajectory(Dynamics):
             spectra = self._get_raman_spectra_shared(models)
             if spectra is not None:
                 return spectra
+        return [self._allgather_spectrum(local) for local in self._local.get_raman_spectra(models)]
+
+    def _allgather_spectrum(self, local: MDRamanSpectrum) -> ShardedMDRamanSpectrum:
+        """All-gather path: the spectrum of the whole series assembled from this rank's ``local`` spectrum."""
         import torch  # pylint: disable=import-outside-toplevel
         import torch.distributed as dist  # pylint: disable=import-outside-toplevel
 
+        series = local._polarizability_ts  # pylint: disable=protected-access
+        if not _lib.is_torch_tensor(series):
+            series = torch.from_numpy(series)
+        full = allgather_series(series, self._num_frames, self._group)
         bounds = shard_bounds(self._num_frames, dist.get_world_size(self._group), dist.get_rank(self._group))
-        spectra = []
-        for local in self._local.get_raman_spectra(models):
-            series = local._polarizability_ts  # pylint: disable=protected-access
-            if not hasattr(series, "data_ptr"):
-                series = torch.from_numpy(series)
-            full = allgather_series(series, self._num_frames, self._group)
-            spectra.append(ShardedMDRamanSpectrum(full, self._local.timestep, self._group, bounds=bounds))
-        return spectra
+        return ShardedMDRamanSpectrum(full, self._local.timestep, self._group, bounds=bounds)
 
     def _get_raman_spectra_shared(self, models):
         import torch  # pylint: disable=import-outside-toplevel

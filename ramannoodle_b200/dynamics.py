@@ -21,10 +21,6 @@ from .spectrum import MDRamanSpectrum, PhononRamanSpectrum
 RAMAN_TENSOR_CENTRAL_DIFFERENCE = 0.001  # ramannoodle/constants.py:248
 
 
-def _is_torch_tensor(obj) -> bool:
-    return type(obj).__module__.startswith("torch") and hasattr(obj, "data_ptr")
-
-
 def apply_pbc(positions):
     """``ramannoodle/structure/utils.py:13-29``: ``positions - positions // 1`` (host)."""
     try:
@@ -46,7 +42,7 @@ class Trajectory(Dynamics, Sequence):
             raise ValueError("timestep must be positive")
         self._timestep = timestep
         self._pinned_owner = None
-        if _is_torch_tensor(positions_ts):
+        if _lib.is_torch_tensor(positions_ts):
             self._positions_ts = self._wrap_device(positions_ts, pin_memory)
         else:
             self._positions_ts = self._wrap_host(np.asarray(positions_ts), pin_memory)
@@ -75,9 +71,8 @@ class Trajectory(Dynamics, Sequence):
         device = int(data.device.index or 0)
         _lib.require_device(device)
         with torch.cuda.device(device):
-            stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
             status = _lib.lib().rn_apply_pbc(ctypes.c_void_p(data.data_ptr()), ctypes.c_void_p(out.data_ptr()),
-                                             data.numel(), stream)
+                                             data.numel(), _lib.current_stream(device))
         _lib.check(status, "rn_apply_pbc")
         return out
 
@@ -115,7 +110,7 @@ class Trajectory(Dynamics, Sequence):
     @property
     def positions_ts(self) -> np.ndarray:
         """(A copy of) the wrapped positions time series, shape (S,N,3)."""
-        if _is_torch_tensor(self._positions_ts):
+        if _lib.is_torch_tensor(self._positions_ts):
             return self._positions_ts.cpu().numpy()
         return self._positions_ts.copy()
 
@@ -125,7 +120,7 @@ class Trajectory(Dynamics, Sequence):
 
     @property
     def is_device_resident(self) -> bool:
-        return _is_torch_tensor(self._positions_ts)
+        return _lib.is_torch_tensor(self._positions_ts)
 
     def get_raman_spectrum(self, polarizability_model: PolarizabilityModel) -> MDRamanSpectrum:
         """One ``calc_polarizabilities`` call over the whole trajectory, wrapped into an
@@ -164,7 +159,7 @@ class Trajectory(Dynamics, Sequence):
             if "out of bounds" in str(exc) or "out of range" in str(exc):
                 raise IndexError("trajectory index out of bounds") from exc
             raise exc
-        return item.cpu().numpy() if _is_torch_tensor(item) else item
+        return item.cpu().numpy() if _lib.is_torch_tensor(item) else item
 
 
 class Phonons(Dynamics):

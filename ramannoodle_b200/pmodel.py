@@ -24,10 +24,6 @@ from .exceptions import UserError, get_shape_error, get_type_error, verify_ndarr
 from .state import ModelState
 
 
-def _is_torch_tensor(obj) -> bool:
-    return type(obj).__module__.startswith("torch") and hasattr(obj, "data_ptr")
-
-
 def _ptr(array: np.ndarray) -> ctypes.c_void_p:
     return ctypes.c_void_p(array.ctypes.data)
 
@@ -194,19 +190,13 @@ class InterpolationModel(PolarizabilityModel):
 
     def calc_polarizabilities(self, positions_batch):
         """Return polarizabilities (S,3,3) for fractional positions (S,N,3)."""
-        if _is_torch_tensor(positions_batch):
-            return self._eval_tensor(positions_batch, wrap=True, name="positions", columns=None)
-        if not isinstance(positions_batch, np.ndarray):
-            raise get_type_error("positions", positions_batch, "ndarray")
-        if positions_batch.ndim != 3 or positions_batch.shape[1:] != (self.num_atoms, 3):
-            raise get_shape_error("positions", positions_batch, f"(_,{self.num_atoms},3)")
-        self._check_dummy()
-        positions = np.ascontiguousarray(positions_batch, dtype=np.float64)
-        num_frames = positions.shape[0]
-        alpha = np.empty((num_frames, 3, 3), dtype=np.float64)
-        native = self._native_model()
-        status = _lib.lib().rn_calc_polarizabilities_host(native.handle, _ptr(positions), num_frames, _ptr(alpha),
-                                                          None, 0)
+        if _lib.is_torch_tensor(positions_batch):
+            return self._eval_tensor(positions_batch, wrap=True, name="positions")
+        _, positions, device, _ = _eval_inputs([self], positions_batch)
+        alpha = np.empty((positions.shape[0], 3, 3), dtype=np.float64)
+        native = self._native_model(device)
+        status = _lib.lib().rn_calc_polarizabilities_host(native.handle, _ptr(positions), positions.shape[0],
+                                                          _ptr(alpha), None, 0)
         _lib.check(status, "rn_calc_polarizabilities_host")
         return alpha
 
@@ -217,11 +207,7 @@ class InterpolationModel(PolarizabilityModel):
 
         if not isinstance(positions_batch, np.ndarray):
             raise get_type_error("positions", positions_batch, "ndarray")
-        if positions_batch.ndim != 3 or positions_batch.shape[1:] != (self.num_atoms, 3):
-            raise get_shape_error("positions", positions_batch, f"(_,{self.num_atoms},3)")
-        self._check_dummy()
-        positions = np.ascontiguousarray(positions_batch, dtype=np.float64)
-        device = self._resolve_device()
+        _, positions, device, _ = _eval_inputs([self], positions_batch)
         native = self._native_model(device)
         alpha = torch.empty((positions.shape[0], 3, 3), dtype=torch.float64, device=f"cuda:{device}")
         torch.cuda.synchronize(device)
@@ -240,37 +226,21 @@ class InterpolationModel(PolarizabilityModel):
         if not 1 <= count <= 8:
             raise ValueError("between 1 and 8 output pointers are required")
         outputs = (ctypes.c_void_p * count)(*[ctypes.c_void_p(int(ptr)) for ptr in output_ptrs])
-        if _is_torch_tensor(positions_batch):
+        _, positions, device, is_tensor = _eval_inputs([self], positions_batch)
+        native = self._native_model(device)
+        if is_tensor:
             import torch  # pylint: disable=import-outside-toplevel
 
-            if not positions_batch.is_cuda:
-                raise get_type_error("positions", positions_batch, "ndarray or CUDA tensor")
-            if positions_batch.ndim != 3 or tuple(positions_batch.shape[1:]) != (self.num_atoms, 3):
-                raise get_shape_error("positions", positions_batch, f"(_,{self.num_atoms},3)")
-            self._check_dummy()
-            data = positions_batch.to(torch.float64).contiguous()
-            device = self._resolve_device(data)
-            native = self._native_model(device)
             with torch.cuda.device(device):
-                stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
                 status = _lib.lib().rn_calc_polarizabilities_multi(
-                    native.handle, ctypes.c_void_p(data.data_ptr()), int(data.shape[0]), outputs, count, stream)
+                    native.handle, ctypes.c_void_p(positions.data_ptr()), int(positions.shape[0]), outputs, count,
+                    _lib.current_stream(device))
             _lib.check(status, "rn_calc_polarizabilities_multi")
             return
-        if not isinstance(positions_batch, np.ndarray):
-            raise get_type_error("positions", positions_batch, "ndarray")
-        if positions_batch.ndim != 3 or positions_batch.shape[1:] != (self.num_atoms, 3):
-            raise get_shape_error("positions", positions_batch, f"(_,{self.num_atoms},3)")
-        self._check_dummy()
-        positions = np.ascontiguousarray(positions_batch, dtype=np.float64)
-        native = self._native_model()
-        import torch  # pylint: disable=import-outside-toplevel
-
         # the pipeline's private streams start after the work already enqueued on the current stream
         # (e.g. the cross-rank barrier in front of this call)
-        stream = ctypes.c_void_p(torch.cuda.current_stream(native.device).cuda_stream)
         status = _lib.lib().rn_calc_polarizabilities_host_multi(native.handle, _ptr(positions), positions.shape[0],
-                                                                outputs, count, 0, stream)
+                                                                outputs, count, 0, _lib.current_stream(device))
         _lib.check(status, "rn_calc_polarizabilities_host_multi")
 
     # pylint: disable=too-many-arguments,too-many-positional-arguments
@@ -278,7 +248,7 @@ class InterpolationModel(PolarizabilityModel):
         """Whether ``calc_polarizabilities_routed(..., stripe=stripe, phase=0|1)`` can evaluate this block
         (``rn_routed_phases_supported``: a purely linear model on the TMA path, HBM-resident 16-byte aligned
         rows, block bounds on multiples of 16 frames)."""
-        if stripe <= 0 or not _is_torch_tensor(positions_batch) or not positions_batch.is_cuda:
+        if stripe <= 0 or not _lib.is_torch_tensor(positions_batch) or not positions_batch.is_cuda:
             return False
         import torch  # pylint: disable=import-outside-toplevel
 
@@ -297,54 +267,37 @@ class InterpolationModel(PolarizabilityModel):
         row ``n`` to ranks ``(n % period) // width`` and ``((n - 1) % period) // width``.
         ``phase`` 0 / 1 (with ``stripe``; CUDA tensors only, ``routed_phases_supported``): one half of the
         pipelined schedule, ``rn_calc_polarizabilities_routed_phase``."""
-        import torch  # pylint: disable=import-outside-toplevel
-
         world = len(peer_series)
         if not 1 <= world <= 8:
             raise ValueError("between 1 and 8 ranks")
         peers = (ctypes.c_void_p * world)(*[ctypes.c_void_p(int(ptr)) if ptr else None for ptr in peer_series])
-        if _is_torch_tensor(positions_batch):
-            if not positions_batch.is_cuda:
-                raise get_type_error("positions", positions_batch, "ndarray or CUDA tensor")
-            if positions_batch.ndim != 3 or tuple(positions_batch.shape[1:]) != (self.num_atoms, 3):
-                raise get_shape_error("positions", positions_batch, f"(_,{self.num_atoms},3)")
-            self._check_dummy()
-            data = positions_batch.to(torch.float64).contiguous()
-            device = self._resolve_device(data)
-            native = self._native_model(device)
-            with torch.cuda.device(device):
-                stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-                if phase >= 0:
-                    status = _lib.lib().rn_calc_polarizabilities_routed_phase(
-                        native.handle, ctypes.c_void_p(data.data_ptr()), int(data.shape[0]),
-                        ctypes.c_void_p(int(local_ptr)), peers, world, int(first_frame), int(period), int(width),
-                        int(stripe), int(phase), stream)
-                else:
-                    status = _lib.lib().rn_calc_polarizabilities_routed(
-                        native.handle, ctypes.c_void_p(data.data_ptr()), int(data.shape[0]),
-                        ctypes.c_void_p(int(local_ptr)), peers, world, int(first_frame), int(period), int(width), stream)
-            _lib.check(status, "rn_calc_polarizabilities_routed")
-            return
-        if phase >= 0:
+        if phase >= 0 and not _lib.is_torch_tensor(positions_batch):
             raise ValueError("phased evaluation needs an HBM-resident trajectory block")
-        if not isinstance(positions_batch, np.ndarray):
-            raise get_type_error("positions", positions_batch, "ndarray")
-        if positions_batch.ndim != 3 or positions_batch.shape[1:] != (self.num_atoms, 3):
-            raise get_shape_error("positions", positions_batch, f"(_,{self.num_atoms},3)")
-        self._check_dummy()
-        positions = np.ascontiguousarray(positions_batch, dtype=np.float64)
-        native = self._native_model()
-        stream = ctypes.c_void_p(torch.cuda.current_stream(native.device).cuda_stream)
-        status = _lib.lib().rn_calc_polarizabilities_host_routed(
-            native.handle, _ptr(positions), positions.shape[0], ctypes.c_void_p(int(local_ptr)), peers, world,
-            int(first_frame), int(period), int(width), 0, stream)
-        _lib.check(status, "rn_calc_polarizabilities_host_routed")
+        _, positions, device, is_tensor = _eval_inputs([self], positions_batch)
+        native = self._native_model(device)
+        routing = (ctypes.c_void_p(int(local_ptr)), peers, world, int(first_frame), int(period), int(width))
+        if not is_tensor:
+            status = _lib.lib().rn_calc_polarizabilities_host_routed(
+                native.handle, _ptr(positions), positions.shape[0], *routing, 0, _lib.current_stream(device))
+            _lib.check(status, "rn_calc_polarizabilities_host_routed")
+            return
+        import torch  # pylint: disable=import-outside-toplevel
+
+        data, num_frames = ctypes.c_void_p(positions.data_ptr()), int(positions.shape[0])
+        with torch.cuda.device(device):
+            if phase >= 0:
+                status = _lib.lib().rn_calc_polarizabilities_routed_phase(
+                    native.handle, data, num_frames, *routing, int(stripe), int(phase), _lib.current_stream(device))
+            else:
+                status = _lib.lib().rn_calc_polarizabilities_routed(native.handle, data, num_frames, *routing,
+                                                                    _lib.current_stream(device))
+        _lib.check(status, "rn_calc_polarizabilities_routed")
 
     def get_polarizability(self, cart_displacements):
         """Polarizabilities from precomputed Cartesian displacements (S,N,3) or (S,3N) in Å
         (what ``_interpolation.py:217-223`` produces)."""
-        if _is_torch_tensor(cart_displacements):
-            return self._eval_tensor(cart_displacements, wrap=False, name="cart_displacements", columns=None)
+        if _lib.is_torch_tensor(cart_displacements):
+            return self._eval_tensor(cart_displacements, wrap=False, name="cart_displacements")
         if not isinstance(cart_displacements, np.ndarray):
             raise get_type_error("cart_displacements", cart_displacements, "ndarray")
         import torch  # pylint: disable=import-outside-toplevel
@@ -352,37 +305,30 @@ class InterpolationModel(PolarizabilityModel):
         device = self._resolve_device()
         _lib.require_device(device)
         tensor = torch.from_numpy(np.ascontiguousarray(cart_displacements, dtype=np.float64)).to(f"cuda:{device}")
-        return self._eval_tensor(tensor, wrap=False, name="cart_displacements", columns=None).cpu().numpy()
+        return self._eval_tensor(tensor, wrap=False, name="cart_displacements").cpu().numpy()
 
-    def _eval_tensor(self, tensor, wrap: bool, name: str, columns):
+    def _eval_tensor(self, tensor, wrap: bool, name: str):
         import torch  # pylint: disable=import-outside-toplevel
 
-        if not tensor.is_cuda:
-            raise get_type_error(name, tensor, "ndarray or CUDA tensor")
-        dim = 3 * self.num_atoms
-        ok = (tensor.ndim == 3 and tuple(tensor.shape[1:]) == (self.num_atoms, 3)) or (
-            not wrap and tensor.ndim == 2 and tensor.shape[1] == dim)
-        if not ok:
-            raise get_shape_error(name, tensor, f"(_,{self.num_atoms},3)")
-        self._check_dummy()
-        data = tensor.to(torch.float64).contiguous()
-        device = self._resolve_device(data)
+        _, data, device, _ = _eval_inputs([self], tensor, name=name, flat=not wrap)
         native = self._native_model(device)
         num_frames = int(data.shape[0])
         with torch.cuda.device(device):
             alpha = torch.empty((num_frames, 3, 3), dtype=torch.float64, device=data.device)
-            stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
             entry = _lib.lib().rn_calc_polarizabilities if wrap else _lib.lib().rn_get_polarizability
             status = entry(native.handle, ctypes.c_void_p(data.data_ptr()), num_frames,
-                           ctypes.c_void_p(alpha.data_ptr()), stream)
+                           ctypes.c_void_p(alpha.data_ptr()), _lib.current_stream(device))
         _lib.check(status, "rn_calc_polarizabilities" if wrap else "rn_get_polarizability")
         return alpha
 
 
-def _sweep_inputs(models, positions_batch):
-    """Validated models and positions of a sweep: (models, contiguous float64 positions, device, is_tensor)."""
-    import torch  # pylint: disable=import-outside-toplevel
+def _eval_inputs(models, positions_batch, name: str = "positions", flat: bool = False):
+    """Validated inputs of an evaluation of ``models`` (one structure; one model, or the models of a sweep) on
+    ``positions_batch``: (models, contiguous float64 positions, device, is_tensor).
 
+    Checks, before any device work and in this order: the models, the type (ndarray or CUDA tensor), the
+    shape (S,N,3) (``flat``: (S,3N) as well), dummy models.  The device is the tensor's, or for numpy input
+    the one ``models[0]`` resolves."""
     models = list(models)
     if len(models) == 0:
         raise ValueError("at least one model is required")
@@ -394,17 +340,21 @@ def _sweep_inputs(models, positions_batch):
     num_atoms = models[0].num_atoms
     if any(model.num_atoms != num_atoms for model in models):
         raise ValueError("models of a sweep must describe the same structure")
-    is_tensor = _is_torch_tensor(positions_batch)
+    is_tensor = _lib.is_torch_tensor(positions_batch)
     if is_tensor:
         if not positions_batch.is_cuda:
-            raise get_type_error("positions", positions_batch, "ndarray or CUDA tensor")
+            raise get_type_error(name, positions_batch, "ndarray or CUDA tensor")
     elif not isinstance(positions_batch, np.ndarray):
-        raise get_type_error("positions", positions_batch, "ndarray")
-    if positions_batch.ndim != 3 or tuple(positions_batch.shape[1:]) != (num_atoms, 3):
-        raise get_shape_error("positions", positions_batch, f"(_,{num_atoms},3)")
+        raise get_type_error(name, positions_batch, "ndarray")
+    shape = tuple(positions_batch.shape)
+    if not (len(shape) == 3 and shape[1:] == (num_atoms, 3)) and not (
+            flat and len(shape) == 2 and shape[1] == 3 * num_atoms):
+        raise get_shape_error(name, positions_batch, f"(_,{num_atoms},3)")
     for model in models:
         model._check_dummy()  # pylint: disable=protected-access
     if is_tensor:
+        import torch  # pylint: disable=import-outside-toplevel
+
         data = positions_batch.to(torch.float64).contiguous()
         device = models[0]._resolve_device(data)  # pylint: disable=protected-access
     else:
@@ -423,7 +373,7 @@ def calc_polarizabilities_sweep(models, positions_batch, to_device: bool = False
     numpy in -> numpy out (a CUDA tensor if ``to_device``); CUDA tensor in -> CUDA tensor out."""
     import torch  # pylint: disable=import-outside-toplevel
 
-    models, data, device, is_tensor = _sweep_inputs(models, positions_batch)
+    models, data, device, is_tensor = _eval_inputs(models, positions_batch)
     count = len(models)
     num_frames = int(data.shape[0])
     natives = [model._native_model(device) for model in models]  # pylint: disable=protected-access
@@ -434,9 +384,8 @@ def calc_polarizabilities_sweep(models, positions_batch, to_device: bool = False
             return alpha if (is_tensor or to_device) else alpha.cpu().numpy()
         outputs = (ctypes.c_void_p * count)(*[ctypes.c_void_p(alpha[g].data_ptr()) for g in range(count)])
         if is_tensor:
-            stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
             status = _lib.lib().rn_calc_polarizabilities_sweep(handles, count, ctypes.c_void_p(data.data_ptr()),
-                                                               num_frames, outputs, stream)
+                                                               num_frames, outputs, _lib.current_stream(device))
             _lib.check(status, "rn_calc_polarizabilities_sweep")
             return alpha
         torch.cuda.synchronize(device)
@@ -456,7 +405,7 @@ def calc_polarizabilities_sweep_routed(models, positions_batch, local_ptrs, peer
     crosses PCIe once for all models (in chunks of ``chunk_frames``, 0 = automatic)."""
     import torch  # pylint: disable=import-outside-toplevel
 
-    models, data, device, is_tensor = _sweep_inputs(models, positions_batch)
+    models, data, device, is_tensor = _eval_inputs(models, positions_batch)
     count = len(models)
     if len(local_ptrs) != count or len(peer_series) != count:
         raise ValueError("one local pointer and one row of peer pointers per model are required")
@@ -470,7 +419,7 @@ def calc_polarizabilities_sweep_routed(models, positions_batch, local_ptrs, peer
                                                   for row in peer_series for ptr in row])
     num_frames = int(data.shape[0])
     with torch.cuda.device(device):
-        stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+        stream = _lib.current_stream(device)
         if is_tensor:
             status = _lib.lib().rn_calc_polarizabilities_sweep_routed(
                 handles, count, ctypes.c_void_p(data.data_ptr()), num_frames, outputs, peers, world, int(first_frame),

@@ -26,19 +26,11 @@ def _torch():
     return torch
 
 
-def _is_torch_tensor(obj) -> bool:
-    return type(obj).__module__.startswith("torch") and hasattr(obj, "data_ptr")
-
-
 def _current_device() -> int:
     torch = _torch()
     if not torch.cuda.is_available():
         _lib.require_device(0)  # raises NativeLibraryError with the reason
     return int(torch.cuda.current_device())
-
-
-def _stream(device: int) -> ctypes.c_void_p:
-    return ctypes.c_void_p(_torch().cuda.current_stream(device).cuda_stream)
 
 
 class _Plan:
@@ -153,7 +145,7 @@ class MDRamanSpectrum(RamanSpectrum):
     @property
     def polarizability_ts(self) -> np.ndarray:
         """The (S,3,3) series as numpy (copied from the GPU on first access if needed)."""
-        if _is_torch_tensor(self._polarizability_ts):
+        if _lib.is_torch_tensor(self._polarizability_ts):
             return self._polarizability_ts.detach().cpu().numpy()
         return self._polarizability_ts
 
@@ -164,7 +156,7 @@ class MDRamanSpectrum(RamanSpectrum):
     def _device_series(self):
         torch = _torch()
         series = self._polarizability_ts
-        if _is_torch_tensor(series):
+        if _lib.is_torch_tensor(series):
             if not series.is_cuda:
                 series = series.to(f"cuda:{_current_device()}")
             return series.to(torch.float64).contiguous()
@@ -192,7 +184,8 @@ class MDRamanSpectrum(RamanSpectrum):
                     plan.handle, ctypes.c_void_p(series.data_ptr()), float(self._timestep),
                     1 if laser_correction else 0, float(laser_wavelength) if laser_correction else 0.0,
                     1 if bose_einstein_correction else 0, float(temperature) if bose_einstein_correction else 0.0,
-                    ctypes.c_void_p(wavenumbers.data_ptr()), ctypes.c_void_p(intensities.data_ptr()), _stream(device))
+                    ctypes.c_void_p(wavenumbers.data_ptr()), ctypes.c_void_p(intensities.data_ptr()),
+                    _lib.current_stream(device))
                 _lib.check(status, "rn_md_spectrum")
         return wavenumbers, intensities
 
@@ -316,7 +309,8 @@ def _measure_windows(series, timestep, window_frames: int, hop: int, laser_corre
                 plan.handle, ctypes.c_void_p(series.data_ptr()), num_frames, hop, float(timestep),
                 1 if laser_correction else 0, float(laser_wavelength) if laser_correction else 0.0,
                 1 if bose_einstein_correction else 0, float(temperature) if bose_einstein_correction else 0.0,
-                ctypes.c_void_p(wavenumbers.data_ptr()), ctypes.c_void_p(intensities.data_ptr()), _stream(device))
+                ctypes.c_void_p(wavenumbers.data_ptr()), ctypes.c_void_p(intensities.data_ptr()),
+                _lib.current_stream(device))
             _lib.check(status, "rn_md_spectrum_windows")
     return wavenumbers, intensities
 
@@ -382,7 +376,7 @@ def calc_signal_spectrum(signal, sampling_rate: float):
         plan = _get_plan(length + 1, device)
         status = _lib.lib().rn_signal_spectrum(plan.handle, ctypes.c_void_p(data.data_ptr()), float(sampling_rate),
                                                ctypes.c_void_p(wavenumbers.data_ptr()),
-                                               ctypes.c_void_p(intensities.data_ptr()), _stream(device))
+                                               ctypes.c_void_p(intensities.data_ptr()), _lib.current_stream(device))
         _lib.check(status, "rn_signal_spectrum")
     return wavenumbers.cpu().numpy(), intensities.cpu().numpy()
 
@@ -393,11 +387,11 @@ def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", widt
     and error messages.  Accepts numpy arrays (or CUDA tensors) and returns numpy arrays."""
     torch = _torch()
     if out_wavenumbers is None:
-        if _is_torch_tensor(wavenumbers) and wavenumbers.is_cuda and wavenumbers.numel() > 0:
+        if _lib.is_torch_tensor(wavenumbers) and wavenumbers.is_cuda and wavenumbers.numel() > 0:
             # the default grid needs two numbers, not a copy of the spectrum
             low, high = (float(v) for v in torch.aminmax(wavenumbers))
         else:
-            wn_host = wavenumbers.detach().cpu().numpy() if _is_torch_tensor(wavenumbers) else wavenumbers
+            wn_host = wavenumbers.detach().cpu().numpy() if _lib.is_torch_tensor(wavenumbers) else wavenumbers
             low, high = np.min(wn_host), np.max(wn_host)
         min_wavenumber = low - 100
         max_wavenumber = high + 100
@@ -420,7 +414,7 @@ def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", widt
     _lib.require_device(device)
 
     def to_device(array):
-        if _is_torch_tensor(array):
+        if _lib.is_torch_tensor(array):
             return array.to(device=f"cuda:{device}", dtype=torch.float64).contiguous()
         return torch.from_numpy(np.ascontiguousarray(array, dtype=np.float64)).to(f"cuda:{device}")
 
@@ -433,7 +427,7 @@ def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", widt
         status = _lib.lib().rn_convolve_spectrum(
             ctypes.c_void_p(d_wn.data_ptr()), ctypes.c_void_p(d_in.data_ptr()), num_in, kind, float(width),
             ctypes.c_void_p(d_out_wn.data_ptr()), num_out, ctypes.c_void_p(d_out.data_ptr()),
-            ctypes.c_void_p(workspace.data_ptr()), _stream(device))
+            ctypes.c_void_p(workspace.data_ptr()), _lib.current_stream(device))
         _lib.check(status, "rn_convolve_spectrum")
-    out_host = out_wavenumbers.detach().cpu().numpy() if _is_torch_tensor(out_wavenumbers) else out_wavenumbers
+    out_host = out_wavenumbers.detach().cpu().numpy() if _lib.is_torch_tensor(out_wavenumbers) else out_wavenumbers
     return (out_host, d_out.cpu().numpy())

@@ -168,6 +168,33 @@ def test_argument_validation_matches_reference_messages():
     assert np.array_equal(traj.positions_ts, [[[0.25, 0.75, 0.5]]]) and traj.timestep == 1.0 and len(traj) == 1
 
 
+def test_multi_gpu_entry_argument_errors():
+    """The broadcast and routed evaluation forms and the shared-spectrum ``measure_device`` reject bad
+    arguments before any device work."""
+    import types
+
+    from ramannoodle_b200.distributed import ShardedMDRamanSpectrum
+
+    model = rb.ARTModel(synthetic.make_model("TiO2", "art", num_dofs=6))
+    positions = synthetic.make_trajectory("TiO2", 4)
+    for count in (0, 9):
+        with pytest.raises(ValueError, match="between 1 and 8 output pointers are required"):
+            model.calc_polarizabilities_multi(positions, [0] * count)
+        with pytest.raises(ValueError, match="between 1 and 8 ranks"):
+            model.calc_polarizabilities_routed(positions, 0, [0] * count, 0, 64, 32)
+    with pytest.raises(ValueError, match="phased evaluation needs an HBM-resident trajectory block"):
+        model.calc_polarizabilities_routed(positions, 0, [0, 0], 0, 64, 32, stripe=64, phase=0)
+    spectrum = ShardedMDRamanSpectrum(None, 1.0, context=types.SimpleNamespace(generation=0), bounds=(0, 4))
+    with pytest.raises(NotImplementedError, match="only polycrystalline spectra are supported for now"):
+        spectrum.measure_device(orientation="xx")
+    with pytest.raises(ValueError, match="invalid laser_wavenumber: -10000000.0 <= 0"):
+        spectrum.measure_device(laser_correction=True, laser_wavelength=-1)
+    with pytest.raises(ValueError, match="invalid temperature: 0 <= 0"):
+        spectrum.measure_device(bose_einstein_correction=True, temperature=0)
+    with pytest.raises(TypeError, match="temperature should have type float, not list"):
+        spectrum.measure_device(bose_einstein_correction=True, temperature=[])
+
+
 def test_corrections_match_oracle():
     from oracle import numpy_port as ora
 

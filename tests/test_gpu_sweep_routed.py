@@ -36,9 +36,10 @@ def _dense_split(frames):
     return -(-tiles // sms) * sms > 1.04 * tiles
 
 
-def _emulate(models, positions, world, period, width, host=False, chunk_frames=0):
-    """Evaluates every rank's block of ``positions`` with the routed sweep; returns the series buffers
-    ``[rank][mask]`` as (S,9) arrays."""
+def _emulate(models, positions, world, period, width, host=False, chunk_frames=0,
+             route=calc_polarizabilities_sweep_routed):
+    """Evaluates every rank's block of ``positions`` with the routed sweep (or ``route``, called with its
+    arguments); returns the series buffers ``[rank][mask]`` as (S,9) arrays."""
     frames = positions.shape[0]
     count = len(models)
     buffers = [[torch.full((frames * 9,), float("nan"), dtype=torch.float64, device="cuda:0") for _ in range(count)]
@@ -49,7 +50,7 @@ def _emulate(models, positions, world, period, width, host=False, chunk_frames=0
         block = np.ascontiguousarray(block) if host else to_cuda(block)
         local = [buffers[rank][g].data_ptr() + start * 72 for g in range(count)]
         peers = [[0 if r == rank else buffers[r][g].data_ptr() for r in range(world)] for g in range(count)]
-        calc_polarizabilities_sweep_routed(models, block, local, peers, start, period, width, chunk_frames=chunk_frames)
+        route(models, block, local, peers, start, period, width, chunk_frames=chunk_frames)
     torch.cuda.synchronize()
     return [[b.cpu().numpy().reshape(frames, 9) for b in row] for row in buffers]
 

@@ -13,7 +13,6 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import ramannoodle_b200 as rb  # noqa: E402
 from ramannoodle_b200 import _lib, synthetic  # noqa: E402
 from ramannoodle_b200.distributed import ShardedTrajectory, shard_bounds  # noqa: E402
-from ramannoodle_b200.spectrum import _stream  # noqa: E402
 
 rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
 local = int(os.environ["LOCAL_RANK"])
@@ -31,7 +30,7 @@ spectrum = sharded.get_raman_spectrum(model)
 spectrum.measure_device()
 ctx = spectrum._context  # pylint: disable=protected-access
 lib = _lib.lib()
-stream = _stream(local)
+stream = _lib.current_stream(local)
 points = int(lib.rn_spectrum_num_points(total))
 wn = torch.empty(points, dtype=torch.float64, device=device)
 inten = torch.empty(points, dtype=torch.float64, device=device)
