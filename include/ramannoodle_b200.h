@@ -211,6 +211,18 @@ int rn_md_spectrum_windows(rn_spectrum_plan* plan, const double* d_alpha, int64_
                            double timestep_fs, int laser_correction, double laser_wavelength_nm,
                            int bose_einstein_correction, double temperature_K, double* d_wavenumbers,
                            double* d_intensities, void* stream);
+/* Cross spectra of G series (extends _raman.py:241-309 and spectrum/utils.py:95-124; no reference
+ * counterpart).  d_alpha is a contiguous (G,S,3,3) array, plan a single-GPU plan of S frames whose batch
+ * is at least G (rn_spectrum_plan_create_batched(S, G, ...)).  -> d_wavenumbers (P,), d_intensities
+ * (G,G,P), P = rn_spectrum_num_points(S).  Row (g,h) is _raman.py:241-309 with every
+ * calc_signal_spectrum(sig) replaced by the spectrum of the symmetrised cross-correlation
+ * (correlate(sig_g, sig_h) + correlate(sig_h, sig_g)) / 2 of the same signals: symmetric in g and h,
+ * bilinear in the series, and row (g,g) is bit-identical to rn_md_spectrum of series g.  For series whose
+ * differences add up to those of a total series, the G x G rows add up to its spectrum.  The plan keeps
+ * G(G-1)/2 * (ceil((S-1)/256) + 1) doubles of energy partials between calls. */
+int rn_md_cross_spectra(rn_spectrum_plan* plan, const double* d_alpha, int64_t num_series, double timestep_fs,
+                        int laser_correction, double laser_wavelength_nm, int bose_einstein_correction,
+                        double temperature_K, double* d_wavenumbers, double* d_intensities, void* stream);
 /* One transform shared by the ranks of a multi-GPU run (one process per GPU; no reference
  * counterpart — same result as rn_md_spectrum on the whole series).  The chirp-z transform of
  * length L is decimated in frequency over the G = 2, 4 or 8 ranks of the group (the largest power

@@ -52,6 +52,8 @@ struct rn_spectrum_plan {
     unsigned int* d_ticket = nullptr;
     int pack_blocks = 0;
     int64_t batch = 1;      // windows the work, power, partial and ticket buffers hold (single-GPU plans)
+    double* d_cross = nullptr;  // cross spectra: energy partials of every series pair, then their sums
+    int64_t cross_doubles = 0;
 };
 
 namespace rn {
@@ -474,6 +476,134 @@ __global__ void __launch_bounds__(256) combine_signal_kernel(const double* __res
     }
 }
 
+// ---- cross spectra of G series (rn_md_cross_spectra) ----------------------------------------------
+// The orientational average is a sum of squares, so it polarizes into a symmetric bilinear form: with the
+// six weighted signals of the pack and X the length-M DFT,
+//   I_gh[k] = 1/2 sum_p (Re(X_gp[k] conj X_hp[k]) + E_gh),   E_gh = sum_p sum_n x_gp[n] x_hp[n],
+// and for packed Z = A + iB,  Re(Z_g Z_h*)[k] + Re(Z_g Z_h*)[M-k] = 2 Re(A_g A_h* + B_g B_h*)[k].  The chirp
+// post-factor has modulus 1 and is the same for every sequence at bin m, so the products of the transform
+// outputs y are those of the spectra: I_gh[k] = C[k] / (4 L^2) + E_gh / 2 with
+//   C[k] = sum_s Re(y_gs[k] conj y_hs[k]) + Re(y_gs[M-k] conj y_hs[M-k]).
+
+constexpr int kCrossTile = 4;  // series whose signals a thread of cross_energy_kernel holds at once
+
+// pair (g, h), g < h, in row-major order of the strict upper triangle
+__device__ __forceinline__ int64_t upper_pair(int64_t g, int64_t h, int64_t G) {
+    return g * (2 * G - g - 1) / 2 + (h - g - 1);
+}
+
+// the six weighted difference signals of frame n (rows r0 = n, r1 = n + 1), the formulas of pack_alpha_kernel
+__device__ __forceinline__ void md_signals(const double* __restrict__ r0, double z[6]) {
+    const double* r1 = r0 + 9;
+    const double xx = __ldg(r1 + 0) - __ldg(r0 + 0), yy = __ldg(r1 + 4) - __ldg(r0 + 4);
+    const double zz = __ldg(r1 + 8) - __ldg(r0 + 8), xy = __ldg(r1 + 1) - __ldg(r0 + 1);
+    const double yz = __ldg(r1 + 5) - __ldg(r0 + 5), xz = __ldg(r1 + 2) - __ldg(r0 + 2);
+    z[0] = kSqrt5 * (xx + yy + zz);
+    z[1] = kSqrt5_25 * (xx - zz);
+    z[2] = kSqrt1_75 * (xx - 2.0 * yy + zz);
+    z[3] = kSqrt21 * xy;
+    z[4] = kSqrt21 * yz;
+    z[5] = kSqrt21 * xz;
+}
+
+// E_gh for every pair g < h of the G series at src + g stride (one frame per thread).  Block b leaves the
+// partial of pair p in part[p gridDim.x + b]; the block that finishes last sums every pair's partials in
+// block order (bit-reproducible whichever block that is) into energy[p] and re-arms the ticket.  The diagonal
+// energies are the pack's.
+__global__ void __launch_bounds__(256) cross_energy_kernel(const double* __restrict__ src, int64_t stride, int G,
+                                                           int64_t M, double* __restrict__ part,
+                                                           double* __restrict__ energy, unsigned int* ticket) {
+    __shared__ double red[kCrossTile][8];
+    __shared__ bool last;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    for (int g0 = 0; g0 < G - 1; g0 += kCrossTile) {
+        double zg[kCrossTile][6];
+#pragma unroll
+        for (int r = 0; r < kCrossTile; r++) {
+#pragma unroll
+            for (int i = 0; i < 6; i++) zg[r][i] = 0.0;
+            if (n < M && g0 + r < G) md_signals(src + (int64_t)(g0 + r) * stride + n * 9, zg[r]);
+        }
+        for (int h = g0 + 1; h < G; h++) {
+            double zh[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+            if (n < M) md_signals(src + (int64_t)h * stride + n * 9, zh);
+#pragma unroll
+            for (int r = 0; r < kCrossTile; r++) {
+                double v = (zg[r][0] * zh[0] + zg[r][1] * zh[1]) + (zg[r][2] * zh[2] + zg[r][3] * zh[3]) +
+                           (zg[r][4] * zh[4] + zg[r][5] * zh[5]);
+#pragma unroll
+                for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+                if (lane == 0) red[r][warp] = v;
+            }
+            __syncthreads();
+            if (threadIdx.x < kCrossTile && g0 + (int)threadIdx.x < h) {
+                const int r = threadIdx.x;
+                double total = 0.0;
+                for (int w = 0; w < (int)(blockDim.x >> 5); w++) total += red[r][w];
+                part[upper_pair(g0 + r, h, G) * gridDim.x + blockIdx.x] = total;
+                __threadfence();
+            }
+            __syncthreads();  // `red` is reused
+        }
+    }
+    if (threadIdx.x == 0) last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    const int64_t pairs = (int64_t)G * (G - 1) / 2;
+    for (int64_t p = warp; p < pairs; p += blockDim.x >> 5) {
+        double v = 0.0;
+        for (unsigned int b = lane; b < gridDim.x; b += 32) v += __ldcg(part + p * gridDim.x + b);
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+        if (lane == 0) energy[p] = v;
+    }
+    if (threadIdx.x == 0) *ticket = 0;
+}
+
+// Re(a conj b) in the form store_out gives |v|^2 (v.x*v.x + v.y*v.y), so that a == b reproduces the power
+__device__ __forceinline__ double re_dot(double2 a, double2 b) { return a.x * b.x + a.y * b.y; }
+
+// I_gh[k], k = 1 .. points, for every pair g <= h, into rows (g, h) and (h, g) of int_out (G, G, points).
+// y: the 3 G transform outputs (natural order, sequence 3g + s of series g at y + (3g + s) Lh).  Row g of the
+// grid (strided by gridDim.y) holds its own y at bins k and M-k and pairs it with every h >= g.  The sums
+// over s and the final scale run in the order of combine_md_kernel and the diagonal energy is the pack's, so
+// row (g, g) is bit-identical to rn_md_spectrum of series g.
+__global__ void __launch_bounds__(256) cross_combine_kernel(const double2* __restrict__ y, int64_t Lh, int G,
+                                                            const double* __restrict__ epart, int64_t epart_stride,
+                                                            const double* __restrict__ energy, int64_t M,
+                                                            double scale, int64_t points, SpectrumParams prm,
+                                                            double* __restrict__ wn_out, double* __restrict__ int_out) {
+    for (int64_t g = blockIdx.y; g < G; g += gridDim.y) {
+        const double2* yg = y + 3 * g * Lh;
+        for (int64_t o = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; o < points;
+             o += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t k = o + 1;
+            double2 a[3][2];
+#pragma unroll
+            for (int s = 0; s < 3; s++) {
+                a[s][0] = yg[s * Lh + k];
+                a[s][1] = yg[s * Lh + (M - k)];
+            }
+            const double wn = wavenumber_of(k, M, prm.timestep);
+            if (g == 0) wn_out[o] = wn;
+            for (int64_t h = g; h < G; h++) {
+                const double2* yh = y + 3 * h * Lh;
+                double sum = 0.0;
+#pragma unroll
+                for (int s = 0; s < 3; s++)  // __dadd_rn: no product may fuse into these sums
+                    sum = __dadd_rn(sum, __dadd_rn(re_dot(a[s][0], yh[s * Lh + k]), re_dot(a[s][1], yh[s * Lh + (M - k)])));
+                const double e = h == g ? epart[g * epart_stride] : energy[upper_pair(g, h, G)];
+                const double econst = 0.5 * e;
+                const double inten = corrected(sum * scale + econst, wn, prm);
+                int_out[(g * G + h) * points + o] = inten;
+                if (h != g) int_out[(h * G + g) * points + o] = inten;
+            }
+        }
+    }
+}
+
 static int grid_for(int64_t n, int sms) {
     return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)sms * 16));
 }
@@ -589,6 +719,7 @@ static void destroy_plan(rn_spectrum_plan* p) {
     cudaFree(p->d_power);
     cudaFree(p->d_epart);
     cudaFree(p->d_ticket);
+    cudaFree(p->d_cross);
     delete p;
 }
 
@@ -879,6 +1010,67 @@ extern "C" int rn_md_spectrum_windows(rn_spectrum_plan* plan, const double* d_al
         RN_LAUNCHED();
         RN_CUDA(cudaGetLastError());
     }
+    return RN_OK;
+}
+
+// The G series are the windows of hop S over the (G,S,3,3) array: the windowed pack leaves the chirped signals
+// of series g in sequences 3g .. 3g+2 and its energy in its own partials, the convolution keeps every output
+// y (OUT_PLAIN), and the two cross kernels form every pair from them.
+extern "C" int rn_md_cross_spectra(rn_spectrum_plan* plan, const double* d_alpha, int64_t num_series,
+                                   double timestep_fs, int laser_correction, double laser_wavelength_nm,
+                                   int bose_einstein_correction, double temperature_K, double* d_wavenumbers,
+                                   double* d_intensities, void* stream) {
+    RN_CHECK_ARG(plan != nullptr, "plan is null");
+    RN_CHECK_ARG(plan->world == 1, "rn_md_cross_spectra needs a single-GPU plan (rn_spectrum_plan_create_batched)");
+    RN_CHECK_ARG(d_alpha != nullptr, "d_alpha is null");
+    RN_CHECK_ARG(num_series >= 1 && num_series <= plan->batch,
+                 "num_series must be 1 .. %lld (the plan's batch), got %lld", (long long)plan->batch,
+                 (long long)num_series);
+    RN_CHECK_ARG(timestep_fs > 0, "timestep must be positive");
+    if (laser_correction) RN_CHECK_ARG(laser_wavelength_nm > 0, "invalid laser_wavelength");
+    if (bose_einstein_correction) RN_CHECK_ARG(temperature_K > 0, "invalid temperature: %g <= 0", temperature_K);
+    const int64_t points = rn_spectrum_num_points(plan->S);
+    if (points == 0) return RN_OK;
+    RN_CHECK_ARG(d_wavenumbers && d_intensities, "null output pointer");
+    DeviceGuard guard(plan->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int64_t M = plan->M;
+    const int G = (int)num_series;
+    const int64_t energy_blocks = (M + 255) / 256;
+    const int64_t pairs = (int64_t)G * (G - 1) / 2;
+    const int64_t need = pairs * (energy_blocks + 1);
+    if (need > plan->cross_doubles) {  // kept with the plan; calls on one plan are ordered on one stream
+        RN_CUDA(cudaStreamSynchronize(s));
+        cudaFree(plan->d_cross);
+        plan->d_cross = nullptr;
+        plan->cross_doubles = 0;
+        if (cudaMalloc((void**)&plan->d_cross, sizeof(double) * need) != cudaSuccess) {
+            cudaGetLastError();
+            set_error("cudaMalloc of %lld bytes of cross-energy partials failed", (long long)(sizeof(double) * need));
+            return RN_ERR_OUT_OF_MEMORY;
+        }
+        plan->cross_doubles = need;
+    }
+    PackParams pp = md_pack_params(plan, d_alpha);
+    pp.win_stride = plan->S * 9;
+    pack_alpha_kernel<1, true><<<dim3(plan->pack_blocks, (unsigned)G), kPackThreads, 0, s>>>(pp);
+    RN_LAUNCHED();
+    int rc = run_convolution(plan, plan->d_work, 3 * G, M, plain_out(), nullptr, s);
+    if (rc != RN_OK) return rc;
+    double* energy = plan->d_cross + pairs * energy_blocks;
+    if (G > 1) {
+        cross_energy_kernel<<<(unsigned)energy_blocks, 256, 0, s>>>(d_alpha, plan->S * 9, G, M, plan->d_cross, energy,
+                                                                    plan->d_ticket);
+        RN_LAUNCHED();
+    }
+    const SpectrumParams prm = spectrum_params(timestep_fs, laser_correction, laser_wavelength_nm,
+                                               bose_einstein_correction, temperature_K);
+    const double scale = 0.25 / ((double)plan->L * (double)plan->L);
+    cross_combine_kernel<<<dim3(grid_for(points, plan->sm_count), (unsigned)std::min(G, 65535)), 256, 0, s>>>(
+        plan->d_work, plan->Lh, G, plan->d_epart + plan->pack_blocks, plan->pack_blocks + 1, energy, M, scale, points,
+        prm, d_wavenumbers, d_intensities);
+    RN_LAUNCHED();
+    RN_CUDA(cudaGetLastError());
     return RN_OK;
 }
 

@@ -300,6 +300,13 @@ class ShardedMDRamanSpectrum(MDRamanSpectrum):
                                                        self._group).clone()
         return self._polarizability_ts
 
+    def _num_frames(self) -> int:
+        return int(self._context.num_frames) if self._context is not None else super()._num_frames()
+
+    def _device_series(self):
+        """The whole series on this rank's GPU (with a shared context: gathered, a collective on first use)."""
+        return self._gathered() if self._context is not None else super()._device_series()
+
     @property
     def polarizability_ts(self):
         """The whole (S,3,3) series as numpy (a collective on first access: every rank must read it)."""

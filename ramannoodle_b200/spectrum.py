@@ -10,6 +10,7 @@ from __future__ import annotations
 import ctypes
 import threading
 from collections import OrderedDict
+from collections.abc import Sequence
 
 import numpy as np
 
@@ -152,6 +153,9 @@ class MDRamanSpectrum(RamanSpectrum):
     @property
     def timestep(self) -> float:
         return self._timestep
+
+    def _num_frames(self) -> int:
+        return int(self._polarizability_ts.shape[0])
 
     def _device_series(self):
         torch = _torch()
@@ -313,6 +317,92 @@ def _measure_windows(series, timestep, window_frames: int, hop: int, laser_corre
                 _lib.current_stream(device))
             _lib.check(status, "rn_md_spectrum_windows")
     return wavenumbers, intensities
+
+
+def _check_cross_spectra(spectra):
+    """Validate the spectra of ``measure_cross_spectra``; returns (list, frames, timestep)."""
+    if isinstance(spectra, (str, bytes)) or not isinstance(spectra, Sequence):
+        raise get_type_error("spectra", spectra, "list")
+    spectra = list(spectra)
+    if not spectra:
+        raise ValueError("spectra is empty")
+    for item in spectra:
+        if not isinstance(item, MDRamanSpectrum):
+            raise get_type_error("spectra", item, "MDRamanSpectrum")
+    frames = spectra[0]._num_frames()  # pylint: disable=protected-access
+    timestep = spectra[0].timestep
+    for g, item in enumerate(spectra):
+        if item._num_frames() != frames:  # pylint: disable=protected-access
+            raise ValueError(f"spectra[{g}] has {item._num_frames()} frames, spectra[0] has {frames}")  # pylint: disable=protected-access
+        if item.timestep != timestep:
+            raise ValueError(f"spectra[{g}] has timestep {item.timestep}, spectra[0] has {timestep}")
+    if frames < 2:
+        raise ValueError("polarizability_ts must contain at least 2 configurations")
+    return spectra, frames, timestep
+
+
+def _consecutive(series) -> bool:
+    """Whether the series are consecutive slices of one contiguous float64 CUDA array (one (G,S,3,3) block)."""
+    first = series[0]
+    step = first.numel() * first.element_size()
+    torch = _torch()
+    return all(t.is_cuda and t.dtype == torch.float64 and t.is_contiguous() and t.device == first.device
+               and t.data_ptr() == first.data_ptr() + g * step for g, t in enumerate(series))
+
+
+# pylint: disable=too-many-arguments,too-many-positional-arguments,too-many-locals
+def measure_cross_spectra_device(spectra, orientation="polycrystalline", laser_correction=False, laser_wavelength=522,
+                                 bose_einstein_correction=False, temperature=300):
+    """``measure_cross_spectra`` with the result left on the GPU (two CUDA tensors)."""
+    spectra, frames, timestep = _check_cross_spectra(spectra)
+    _check_measure_args(orientation, laser_correction, laser_wavelength, bose_einstein_correction, temperature)
+    torch = _torch()
+    series = [item._device_series() for item in spectra]  # pylint: disable=protected-access
+    if not _consecutive(series):  # e.g. separate arrays: one (G,S,3,3) copy on the current device
+        device = _current_device()
+        series = list(torch.stack([t.to(f"cuda:{device}") for t in series]))
+    num_series = len(series)
+    device = int(series[0].device.index or 0)
+    points = int(_lib.lib().rn_spectrum_num_points(frames))
+    with torch.cuda.device(device):
+        wavenumbers = torch.empty(points, dtype=torch.float64, device=series[0].device)
+        intensities = torch.empty((num_series, num_series, points), dtype=torch.float64, device=series[0].device)
+        if points > 0:
+            plan = _get_plan(frames, device, num_series)
+            status = _lib.lib().rn_md_cross_spectra(
+                plan.handle, ctypes.c_void_p(series[0].data_ptr()), num_series, float(timestep),
+                1 if laser_correction else 0, float(laser_wavelength) if laser_correction else 0.0,
+                1 if bose_einstein_correction else 0, float(temperature) if bose_einstein_correction else 0.0,
+                ctypes.c_void_p(wavenumbers.data_ptr()), ctypes.c_void_p(intensities.data_ptr()),
+                _lib.current_stream(device))
+            _lib.check(status, "rn_md_cross_spectra")
+    return wavenumbers, intensities
+
+
+def measure_cross_spectra(spectra, orientation="polycrystalline", laser_correction=False, laser_wavelength=522,
+                          bose_einstein_correction=False, temperature=300):
+    """Cross spectra of G MD Raman spectra -> (wavenumbers, intensities), numpy arrays of shape (P,) and (G,G,P).
+
+    ``spectra`` is a non-empty sequence of ``MDRamanSpectrum`` with the same frame count S >= 2 and the same
+    timestep, typically the list ``Trajectory.get_raman_spectra(models)`` returns for masked copies of one
+    model.  ``I[g,h]`` is ``spectra[g].measure(...)`` with the spectrum of every signal replaced by that of the
+    symmetrised cross-correlation ``(correlate(sig_g, sig_h) + correlate(sig_h, sig_g)) / 2`` of the same
+    signal of series g and series h: the same signals, weights, dropped 0 cm^-1 bin and corrections.  So
+    ``I[g,h] == I[h,g]``, ``I[g,g]`` is ``spectra[g].measure(...)[1]`` bit for bit, and ``I`` is bilinear in the
+    series.  Cross terms can be negative, and as large as ``sqrt(I[g,g] * I[h,h])``.
+
+    Sum rule: when the masks partition the DOFs (copy g keeps only group g), the differences of the G series
+    add up to those of the unmasked model, so ``I.sum(axis=(0, 1))`` is the total spectrum, and
+    ``I_g = I[g].sum(axis=0)`` attributes it additively to the groups (``sum_g I_g`` is the total).
+
+    All G spectra run as one batched transform on the GPU.  With ``ShardedMDRamanSpectrum`` inputs of a shared
+    transform context every series is first assembled on every rank (an all-gather, a collective): every rank
+    of the group must call this function with the same list in the same order; every rank returns the full
+    result.
+    """
+    wavenumbers, intensities = measure_cross_spectra_device(spectra, orientation, laser_correction, laser_wavelength,
+                                                            bose_einstein_correction, temperature)
+    return wavenumbers.cpu().numpy(), intensities.cpu().numpy()
 
 
 class PhononRamanSpectrum(RamanSpectrum):
