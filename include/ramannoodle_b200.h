@@ -285,6 +285,15 @@ size_t rn_convolve_workspace_size(int64_t num_in, int64_t num_out);
 int rn_convolve_spectrum(const double* d_wavenumbers, const double* d_intensities, int64_t num_in,
                          int kind, double width, const double* d_out_wavenumbers, int64_t num_out,
                          double* d_out_intensities, void* d_workspace, void* stream);
+/* convolve_spectrum (spectrum/utils.py:12-73) of num_rows rows that share one input and one output grid:
+ * d_intensities (B,K) row-major -> d_out_intensities (B,L).  Row b is bit-identical to rn_convolve_spectrum
+ * of row b.  Two launches whatever B is.  d_workspace must hold rn_convolve_spectra_workspace_size(B, K, L)
+ * bytes.  num_rows == 0 or num_out == 0: nothing is launched; num_in == 0: one memset of the output;
+ * num_rows == 1 runs the kernels of rn_convolve_spectrum. */
+size_t rn_convolve_spectra_workspace_size(int64_t num_rows, int64_t num_in, int64_t num_out);
+int rn_convolve_spectra(const double* d_wavenumbers, const double* d_intensities, int64_t num_rows, int64_t num_in,
+                        int kind, double width, const double* d_out_wavenumbers, int64_t num_out,
+                        double* d_out_intensities, void* d_workspace, void* stream);
 
 /* Trajectory ingest — replaces the Python text parsing of io.vasp.xdatcar.read_positions_ts
  * (ramannoodle/io/vasp/xdatcar.py:21-56; header/frames as io/vasp/poscar.py:_read_lattice,

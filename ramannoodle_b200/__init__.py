@@ -10,14 +10,14 @@ from .dynamics import Phonons, Trajectory
 from .exceptions import NativeLibraryError, UserError
 from .dropin import install, uninstall
 from .pmodel import ARTModel, InterpolationModel, accelerate, calc_polarizabilities_sweep
-from .spectrum import (MDRamanSpectrum, PhononRamanSpectrum, calc_signal_spectrum, convolve_spectrum,
-                       get_bose_einstein_correction, get_laser_correction, measure_cross_spectra,
-                       measure_cross_spectra_device)
+from .spectrum import (MDRamanSpectrum, PhononRamanSpectrum, calc_signal_spectrum, convolve_spectra,
+                       convolve_spectra_device, convolve_spectrum, get_bose_einstein_correction, get_laser_correction,
+                       measure_cross_spectra, measure_cross_spectra_device)
 from .state import ModelState
 
 __all__ = [
     "ARTModel", "Dynamics", "InterpolationModel", "MDRamanSpectrum", "ModelState", "NativeLibraryError",
     "Phonons", "PhononRamanSpectrum", "PolarizabilityModel", "RamanSpectrum", "Trajectory", "UserError", "accelerate", "calc_signal_spectrum", "install", "uninstall",
     "convolve_spectrum", "get_bose_einstein_correction", "get_laser_correction", "measure_cross_spectra",
-    "measure_cross_spectra_device",
+    "measure_cross_spectra_device", "convolve_spectra", "convolve_spectra_device",
 ]

@@ -90,7 +90,11 @@ PROTOTYPES = {
     "rn_convolve_spectrum": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int,
                                             ctypes.c_double, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
                                             ctypes.c_void_p, ctypes.c_void_p]),
-    "rn_calc_polarizabilities_sweep": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64,
+    "rn_convolve_spectra_workspace_size": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int64]),
+    "rn_convolve_spectra": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64,
+                                           ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_int64,
+                                           ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "rn_calc_polarizabilities_sweep":(ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64,
                                                       ctypes.c_void_p, ctypes.c_void_p]),
     "rn_calc_polarizabilities_host_sweep": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
                                                            ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64]),

@@ -16,7 +16,7 @@ import numpy as np
 
 from . import _lib
 from .abstract import RamanSpectrum
-from .exceptions import get_type_error, verify_ndarray, verify_ndarray_shape
+from .exceptions import get_type_error, shape_string, verify_ndarray, verify_ndarray_shape
 
 BOLTZMANN_CONSTANT = 8.617333262e-5  # eV/K (ramannoodle/constants.py:249)
 
@@ -471,15 +471,14 @@ def calc_signal_spectrum(signal, sampling_rate: float):
     return wavenumbers.cpu().numpy(), intensities.cpu().numpy()
 
 
-def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", width: float = 5,
-                      out_wavenumbers=None):
-    """Smear a spectrum (``ramannoodle/spectrum/utils.py:12-73``); same defaults, output grid
-    and error messages.  Accepts numpy arrays (or CUDA tensors) and returns numpy arrays."""
-    torch = _torch()
+def _smearing_args(wavenumbers, function, width, out_wavenumbers, check_inputs):
+    """The default output grid and the argument checks of ``convolve_spectrum`` (``utils.py:12-56``), in its
+    order; ``check_inputs()`` checks wavenumbers and intensities between the grid and the width.  Returns
+    (out_wavenumbers, kind).  The grid of CUDA wavenumbers is taken from their min/max on the device."""
     if out_wavenumbers is None:
         if _lib.is_torch_tensor(wavenumbers) and wavenumbers.is_cuda and wavenumbers.numel() > 0:
             # the default grid needs two numbers, not a copy of the spectrum
-            low, high = (float(v) for v in torch.aminmax(wavenumbers))
+            low, high = (float(v) for v in _torch().aminmax(wavenumbers))
         else:
             wn_host = wavenumbers.detach().cpu().numpy() if _lib.is_torch_tensor(wavenumbers) else wavenumbers
             low, high = np.min(wn_host), np.max(wn_host)
@@ -488,8 +487,7 @@ def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", widt
         num_samples = int(np.rint(max_wavenumber - min_wavenumber))
         out_wavenumbers = np.linspace(min_wavenumber, max_wavenumber, num_samples)
     verify_ndarray_shape("out_wavenumbers", out_wavenumbers, (None,))
-    verify_ndarray_shape("wavenumbers", wavenumbers, (None,))
-    verify_ndarray_shape("intensities", intensities, (len(wavenumbers),))
+    check_inputs()
     try:
         if width <= 0:
             raise ValueError(f"invalid width: {width} <= 0")
@@ -498,17 +496,36 @@ def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", widt
     verify_ndarray("out_wavenumbers", out_wavenumbers)
     if function not in ("gaussian", "lorentzian"):
         raise ValueError(f"unsupported convolution type: {function}")
-    kind = 0 if function == "gaussian" else 1
+    return out_wavenumbers, 0 if function == "gaussian" else 1
+
+
+def _to_device(array, device: int):
+    """A float64 contiguous copy of ``array`` on ``cuda:device``; such a tensor is returned as it is."""
+    torch = _torch()
+    if _lib.is_torch_tensor(array):
+        return array.to(device=f"cuda:{device}", dtype=torch.float64).contiguous()
+    return torch.from_numpy(np.ascontiguousarray(array, dtype=np.float64)).to(f"cuda:{device}")
+
+
+def _to_host(array):
+    return array.detach().cpu().numpy() if _lib.is_torch_tensor(array) else array
+
+
+def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", width: float = 5,
+                      out_wavenumbers=None):
+    """Smear a spectrum (``ramannoodle/spectrum/utils.py:12-73``); same defaults, output grid
+    and error messages.  Accepts numpy arrays (or CUDA tensors) and returns numpy arrays."""
+    torch = _torch()
+
+    def check_inputs():
+        verify_ndarray_shape("wavenumbers", wavenumbers, (None,))
+        verify_ndarray_shape("intensities", intensities, (len(wavenumbers),))
+
+    out_wavenumbers, kind = _smearing_args(wavenumbers, function, width, out_wavenumbers, check_inputs)
 
     device = _current_device()
     _lib.require_device(device)
-
-    def to_device(array):
-        if _lib.is_torch_tensor(array):
-            return array.to(device=f"cuda:{device}", dtype=torch.float64).contiguous()
-        return torch.from_numpy(np.ascontiguousarray(array, dtype=np.float64)).to(f"cuda:{device}")
-
-    d_wn, d_in, d_out_wn = to_device(wavenumbers), to_device(intensities), to_device(out_wavenumbers)
+    d_wn, d_in, d_out_wn = (_to_device(a, device) for a in (wavenumbers, intensities, out_wavenumbers))
     num_in, num_out = int(d_wn.shape[0]), int(d_out_wn.shape[0])
     with torch.cuda.device(device):
         d_out = torch.empty(num_out, dtype=torch.float64, device=d_wn.device)
@@ -519,5 +536,86 @@ def convolve_spectrum(wavenumbers, intensities, function: str = "gaussian", widt
             ctypes.c_void_p(d_out_wn.data_ptr()), num_out, ctypes.c_void_p(d_out.data_ptr()),
             ctypes.c_void_p(workspace.data_ptr()), _lib.current_stream(device))
         _lib.check(status, "rn_convolve_spectrum")
-    out_host = out_wavenumbers.detach().cpu().numpy() if _lib.is_torch_tensor(out_wavenumbers) else out_wavenumbers
-    return (out_host, d_out.cpu().numpy())
+    return (_to_host(out_wavenumbers), d_out.cpu().numpy())
+
+
+# Device memory the workspace of one convolve_spectra launch may take (chunks * rows * L partial sums): the rows
+# run in consecutive blocks of as many as fit.  Every row does the same work whatever the block.
+_SMEAR_BLOCK_BYTES = 1 << 30
+
+
+def _smear_rows_per_block(num_rows: int, row_bytes: int) -> int:
+    """Rows per launch of ``rn_convolve_spectra`` when each row takes ``row_bytes`` of workspace: all of them if
+    they fit ``_SMEAR_BLOCK_BYTES``, else as many as fit, and at least one."""
+    if row_bytes == 0:
+        return max(1, num_rows)
+    return max(1, min(num_rows, _SMEAR_BLOCK_BYTES // row_bytes))
+
+
+def _smeared_layout(shape, num_out: int):
+    """(rows, output shape) of ``convolve_spectra`` on intensities of ``shape`` (..., P)."""
+    return int(np.prod(shape[:-1], dtype=np.int64)), tuple(shape[:-1]) + (int(num_out),)
+
+
+def _convolve_rows(wavenumbers, intensities, function, width, out_wavenumbers):
+    """``convolve_spectra``: (out_wavenumbers as given or built, the same on the device, (..., Q) CUDA tensor)."""
+    torch = _torch()
+
+    def check_inputs():
+        verify_ndarray_shape("wavenumbers", wavenumbers, (None,))
+        verify_ndarray("intensities", intensities)
+        if len(intensities.shape) == 0 or intensities.shape[-1] != len(wavenumbers):
+            raise ValueError(f"intensities has shape {shape_string(intensities.shape)}, wavenumbers has shape "
+                             f"{shape_string(wavenumbers.shape)}: the last axis of intensities must be as long as "
+                             "wavenumbers")
+
+    out_wavenumbers, kind = _smearing_args(wavenumbers, function, width, out_wavenumbers, check_inputs)
+
+    device = _current_device()
+    _lib.require_device(device)
+    d_wn, d_in, d_out_wn = (_to_device(a, device) for a in (wavenumbers, intensities, out_wavenumbers))
+    num_in, num_out = int(d_wn.shape[0]), int(d_out_wn.shape[0])
+    num_rows, out_shape = _smeared_layout(tuple(d_in.shape), num_out)
+    rows_per_block = _smear_rows_per_block(num_rows, int(_lib.lib().rn_convolve_spectra_workspace_size(1, num_in,
+                                                                                                       num_out)))
+    with torch.cuda.device(device):
+        d_out = torch.empty(out_shape, dtype=torch.float64, device=d_wn.device)
+        ws_bytes = int(_lib.lib().rn_convolve_spectra_workspace_size(min(rows_per_block, num_rows), num_in, num_out))
+        workspace = torch.empty(max(ws_bytes // 8, 1), dtype=torch.float64, device=d_wn.device)
+        for first in range(0, num_rows, rows_per_block):
+            rows = min(rows_per_block, num_rows - first)
+            status = _lib.lib().rn_convolve_spectra(
+                ctypes.c_void_p(d_wn.data_ptr()), ctypes.c_void_p(d_in.data_ptr() + 8 * first * num_in), rows,
+                num_in, kind, float(width), ctypes.c_void_p(d_out_wn.data_ptr()), num_out,
+                ctypes.c_void_p(d_out.data_ptr() + 8 * first * num_out), ctypes.c_void_p(workspace.data_ptr()),
+                _lib.current_stream(device))
+            _lib.check(status, "rn_convolve_spectra")
+    return out_wavenumbers, d_out_wn, d_out
+
+
+def convolve_spectra_device(wavenumbers, intensities, function: str = "gaussian", width: float = 5,
+                            out_wavenumbers=None):
+    """``convolve_spectra`` with the result left on the GPU: (out_wavenumbers (Q,), intensities (..., Q)),
+    two CUDA tensors."""
+    _, d_out_wn, d_out = _convolve_rows(wavenumbers, intensities, function, width, out_wavenumbers)
+    return d_out_wn, d_out
+
+
+def convolve_spectra(wavenumbers, intensities, function: str = "gaussian", width: float = 5,
+                     out_wavenumbers=None):
+    """Smear every row of a stack of spectra that share ``wavenumbers`` -> (out_wavenumbers (Q,),
+    intensities (..., Q)), numpy arrays.
+
+    ``intensities`` has shape (..., P) with P = len(wavenumbers): the (W, P) rows of ``measure_windows``, the
+    (G, G, P) cross spectra of ``measure_cross_spectra``, or one (P,) spectrum; numpy, a CPU tensor or a CUDA
+    tensor (contiguous float64 CUDA input is read in place).  Row ``idx`` of the result is by definition
+    ``convolve_spectrum(wavenumbers, intensities[idx], function, width, out_wavenumbers)[1]``, bit for bit, and
+    the default output grid is the one that call builds.  All rows run in two launches on the GPU, which
+    evaluate each smearing factor once for a group of rows; the rows are split into consecutive blocks when
+    the partial sums of all of them would take more than 1 GiB.  Argument errors are those of
+    ``convolve_spectrum`` (a wrong last axis or a 0-d ``intensities`` names both shapes) and are raised before
+    any output is allocated or kernel launched; only the default grid of CUDA wavenumbers reads their min and
+    max on the device first, as ``convolve_spectrum`` does.
+    """
+    out_wavenumbers, _, d_out = _convolve_rows(wavenumbers, intensities, function, width, out_wavenumbers)
+    return _to_host(out_wavenumbers), d_out.cpu().numpy()
