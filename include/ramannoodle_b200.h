@@ -223,6 +223,20 @@ int rn_md_spectrum_windows(rn_spectrum_plan* plan, const double* d_alpha, int64_
 int rn_md_cross_spectra(rn_spectrum_plan* plan, const double* d_alpha, int64_t num_series, double timestep_fs,
                         int laser_correction, double laser_wavelength_nm, int bose_einstein_correction,
                         double temperature_K, double* d_wavenumbers, double* d_intensities, void* stream);
+/* Vibrational density of states of G atom groups (no reference counterpart).  d_positions is a contiguous
+ * (S,N,3) array of fractional positions, plan a single-GPU plan of S frames (rn_spectrum_plan_create or
+ * rn_spectrum_plan_create_batched); h_lattice the (3,3) lattice in Angstrom, rows are lattice vectors;
+ * h_weights (N,) finite and >= 0, NULL = all 1; group g is the atoms h_atoms[h_group_offsets[g] ..
+ * h_group_offsets[g+1]-1] (CSR, non-empty, indices in [0, N)).  -> d_wavenumbers (P,), d_intensities (G,P),
+ * P = rn_spectrum_num_points(S): row g is sum over its atoms i and c = x, y, z of
+ * w_i calc_signal_spectrum(v_ic, timestep)[1:] (spectrum/utils.py:95-124) with the minimum-image velocity
+ * v = (wrap(x[n+1] - x[n]) @ lattice) / timestep in Angstrom/fs; the wavenumbers are those of rn_md_spectrum.
+ * Two memberships of a group form a slot; slots run in chunks of the plan's batch (one pack, the transform
+ * and one combine per chunk) and the result is bit-identical for every batch.  The plan keeps the slot
+ * table (24 bytes per slot plus 8 (G+1)) between calls.  P = 0 launches nothing. */
+int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms, const double* h_lattice,
+            const double* h_weights, const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups,
+            double timestep_fs, double* d_wavenumbers, double* d_intensities, void* stream);
 /* One transform shared by the ranks of a multi-GPU run (one process per GPU; no reference
  * counterpart — same result as rn_md_spectrum on the whole series).  The chirp-z transform of
  * length L is decimated in frequency over the G = 2, 4 or 8 ranks of the group (the largest power

@@ -69,6 +69,9 @@ PROTOTYPES = {
     "rn_md_cross_spectra": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_double,
                                            ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_double,
                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "rn_vdos": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                               ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_double, ctypes.c_void_p,
+                               ctypes.c_void_p, ctypes.c_void_p]),
     "rn_spectrum_plan_create_dist": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                     ctypes.POINTER(ctypes.c_void_p)]),
     "rn_spectrum_plan_info": (ctypes.c_int, [ctypes.c_void_p, c_int64_p]),

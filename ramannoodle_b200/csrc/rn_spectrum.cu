@@ -28,6 +28,7 @@
 #include <cmath>
 #include <cstdlib>
 
+#include "rn_device.cuh"
 #include "rn_fft.cuh"
 
 struct rn_spectrum_plan {
@@ -54,6 +55,8 @@ struct rn_spectrum_plan {
     int64_t batch = 1;      // windows the work, power, partial and ticket buffers hold (single-GPU plans)
     double* d_cross = nullptr;  // cross spectra: energy partials of every series pair, then their sums
     int64_t cross_doubles = 0;
+    void* d_vdos = nullptr;     // VDOS: slot table, then the slot offsets of the groups
+    int64_t vdos_bytes = 0;
 };
 
 namespace rn {
@@ -604,6 +607,112 @@ __global__ void __launch_bounds__(256) cross_combine_kernel(const double2* __res
     }
 }
 
+// ---- vibrational density of states (rn_vdos) -------------------------------------------------------
+// The VDOS of a group is sum_{atoms i} w_i sum_c calc_signal_spectrum(v_ic) with v the minimum-image velocity
+// (d @ lattice) / dt.  A slot holds two memberships a, b of one group: its six real signals sqrt(w) v_c of a
+// and of b packed as z_c = (x_a + i x_b)_c are the three sequences of one window of a batched plan, so the
+// identity of combine_md_kernel gives the slot's term (P[k] + P[M-k]) / (4 L^2) + E/2 unchanged.
+
+struct VdosSlot {
+    int atom[2];      // -1: the zero signal that pads a group of odd size
+    double sqrtw[2];  // sqrt(weight) of each membership
+};
+
+struct VdosPackParams {
+    const double* pos;   // (S,N,3) fractional, wrapped
+    int64_t num_atoms;
+    int64_t M, Lh;
+    const VdosSlot* slots;  // the chunk's slots: blockIdx.y numbers them
+    double lattice[9];      // rows are lattice vectors
+    double inv_dt;
+    double2* dst;           // (3 nb, Lh) work buffer
+    double* epart;          // (nb, gridDim.x + 1) partials, then their sum
+    unsigned int* ticket;   // nb tickets
+};
+
+// frames n .. n+256 of the slot's two atoms staged in shared memory; per difference n: the minimum image
+// wrap_disp(x[n+1], x[n]) of each component, times the lattice and sqrt(w)/dt, chirp pre-multiply; the
+// slot's energy is summed with its own partials and ticket, as the windowed pack does.
+__global__ void __launch_bounds__(kPackThreads) pack_velocity_kernel(const __grid_constant__ VdosPackParams P) {
+    __shared__ double rows[(kPackThreads + 1) * 6];
+    __shared__ double red[kPackThreads / 32];
+    const VdosSlot slot = P.slots[blockIdx.y];
+    double2* dst = P.dst + (int64_t)blockIdx.y * 3 * P.Lh;
+    const int64_t first = (int64_t)blockIdx.x * kPackThreads;
+    const int64_t avail = min((int64_t)kPackThreads + 1, P.M + 1 - first);  // frames first .. first+avail-1
+    const int64_t frame_stride = 3 * P.num_atoms;
+    for (int e = threadIdx.x; e < (kPackThreads + 1) * 6; e += kPackThreads) {
+        const int f = e / 6, j = e - 6 * (e / 6);
+        const int atom = j < 3 ? slot.atom[0] : slot.atom[1];
+        rows[e] = (f < avail && atom >= 0) ? __ldg(P.pos + (first + f) * frame_stride + 3 * atom + (j < 3 ? j : j - 3))
+                                           : 0.0;
+    }
+    __syncthreads();
+    const int64_t n = first + threadIdx.x;
+    double energy = 0.0;
+    if (n < P.M) {
+        const double* r0 = rows + threadIdx.x * 6;
+        const double* r1 = r0 + 6;
+        double2 z[3];
+#pragma unroll
+        for (int m = 0; m < 2; m++) {
+            const double d0 = wrap_disp(r1[3 * m], r0[3 * m]);
+            const double d1 = wrap_disp(r1[3 * m + 1], r0[3 * m + 1]);
+            const double d2 = wrap_disp(r1[3 * m + 2], r0[3 * m + 2]);
+            const double s = slot.sqrtw[m] * P.inv_dt;
+#pragma unroll
+            for (int c = 0; c < 3; c++) {
+                const double v = (d0 * P.lattice[c] + d1 * P.lattice[3 + c] + d2 * P.lattice[6 + c]) * s;
+                if (m == 0) z[c].x = v;
+                else z[c].y = v;
+            }
+        }
+        energy = (z[0].x * z[0].x + z[0].y * z[0].y) + (z[1].x * z[1].x + z[1].y * z[1].y) +
+                 (z[2].x * z[2].x + z[2].y * z[2].y);
+        const double2 c = chirp(n, P.M);
+#pragma unroll
+        for (int s = 0; s < 3; s++) dst[(int64_t)s * P.Lh + n] = cmul(z[s], c);
+    }
+    const double total = block_sum(energy, red);
+    publish_energy(total, P.epart + (int64_t)blockIdx.y * (gridDim.x + 1), P.ticket + blockIdx.y, red);
+}
+
+// Rows g_lo .. g_lo + num_groups - 1 of int_out (G, points), for the slots first .. first + nb - 1 of this chunk:
+// row g is the sum, over its slots in slot order, of (P[k] + P[M-k]) scale + E/2.  A group's first slot writes
+// the row; slots of later chunks read it and keep adding one at a time, so the sequence of additions is the
+// same whatever the chunking.  power: (3 nb, M); group_slots: (G+1,) slot offsets of the groups.
+__global__ void __launch_bounds__(256) combine_groups_kernel(const double* __restrict__ power,
+                                                             const double* __restrict__ epart, int64_t epart_stride,
+                                                             const int64_t* __restrict__ group_slots, int64_t first,
+                                                             int64_t nb, int64_t g_lo, int64_t num_groups, int64_t M,
+                                                             double scale, int64_t points, double dt,
+                                                             double* __restrict__ wn_out, double* __restrict__ int_out) {
+    for (int64_t g = g_lo + blockIdx.y; g < g_lo + num_groups; g += gridDim.y) {
+        const int64_t begin = group_slots[g];
+        const int64_t s0 = max(begin, first), s1 = min(group_slots[g + 1], first + nb);
+        double* row = int_out + g * points;
+        for (int64_t o = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; o < points;
+             o += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t k = o + 1;
+            double acc = begin < first ? row[o] : 0.0;
+#pragma unroll 1
+            for (int64_t slot = s0; slot < s1; slot++) {
+                const double* pw = power + (slot - first) * 3 * M;
+                double sum = 0.0;
+#pragma unroll
+                for (int s = 0; s < 3; s++) sum += pw[(int64_t)s * M + k] + pw[(int64_t)s * M + (M - k)];
+                const double term = __fma_rn(sum, scale, 0.5 * epart[(slot - first) * epart_stride]);
+                acc = slot == begin ? term : __dadd_rn(acc, term);
+            }
+            row[o] = acc;
+        }
+    }
+    if (wn_out && blockIdx.y == 0)
+        for (int64_t o = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; o < points;
+             o += (int64_t)gridDim.x * blockDim.x)
+            wn_out[o] = wavenumber_of(o + 1, M, dt);
+}
+
 static int grid_for(int64_t n, int sms) {
     return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)sms * 16));
 }
@@ -720,6 +829,7 @@ static void destroy_plan(rn_spectrum_plan* p) {
     cudaFree(p->d_epart);
     cudaFree(p->d_ticket);
     cudaFree(p->d_cross);
+    cudaFree(p->d_vdos);
     delete p;
 }
 
@@ -1071,6 +1181,113 @@ extern "C" int rn_md_cross_spectra(rn_spectrum_plan* plan, const double* d_alpha
         prm, d_wavenumbers, d_intensities);
     RN_LAUNCHED();
     RN_CUDA(cudaGetLastError());
+    return RN_OK;
+}
+
+// The slots of all groups, in group order, run in chunks of the plan's batch: per chunk one velocity pack, the
+// convolution of its 3 nb sequences with OUT_POWER and one combine that adds the chunk's slots to the rows of
+// the groups they belong to.
+extern "C" int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms, const double* h_lattice,
+                       const double* h_weights, const int64_t* h_group_offsets, const int64_t* h_atoms,
+                       int64_t num_groups, double timestep_fs, double* d_wavenumbers, double* d_intensities,
+                       void* stream) {
+    RN_CHECK_ARG(plan != nullptr, "plan is null");
+    RN_CHECK_ARG(plan->world == 1, "rn_vdos needs a single-GPU plan (rn_spectrum_plan_create_batched)");
+    RN_CHECK_ARG(d_positions && h_lattice && h_group_offsets && h_atoms, "null pointer");
+    RN_CHECK_ARG(num_atoms >= 1 && num_atoms <= INT32_MAX, "invalid num_atoms %lld", (long long)num_atoms);
+    RN_CHECK_ARG(num_groups >= 1, "num_groups must be at least 1 (got %lld)", (long long)num_groups);
+    RN_CHECK_ARG(timestep_fs > 0 && std::isfinite(timestep_fs), "timestep must be positive");
+    for (int i = 0; i < 9; i++) RN_CHECK_ARG(std::isfinite(h_lattice[i]), "lattice entry %d is not finite", i);
+    if (h_weights)
+        for (int64_t i = 0; i < num_atoms; i++)
+            RN_CHECK_ARG(std::isfinite(h_weights[i]) && h_weights[i] >= 0, "invalid weight %g of atom %lld",
+                         h_weights[i], (long long)i);
+    RN_CHECK_ARG(h_group_offsets[0] == 0, "group offsets must start at 0");
+    std::vector<int64_t> group_slots((size_t)num_groups + 1, 0);
+    for (int64_t g = 0; g < num_groups; g++) {
+        const int64_t size = h_group_offsets[g + 1] - h_group_offsets[g];
+        RN_CHECK_ARG(size >= 1, "group %lld is empty", (long long)g);
+        group_slots[(size_t)g + 1] = group_slots[(size_t)g] + (size + 1) / 2;
+    }
+    const int64_t num_slots = group_slots[(size_t)num_groups];
+    std::vector<VdosSlot> slots((size_t)num_slots);
+    for (int64_t g = 0; g < num_groups; g++) {
+        for (int64_t m = h_group_offsets[g]; m < h_group_offsets[g + 1]; m++) {
+            const int64_t atom = h_atoms[m];
+            RN_CHECK_ARG(atom >= 0 && atom < num_atoms, "atom index %lld of group %lld out of range [0, %lld)",
+                         (long long)atom, (long long)g, (long long)num_atoms);
+            const int64_t half = m - h_group_offsets[g];
+            VdosSlot& slot = slots[(size_t)(group_slots[(size_t)g] + half / 2)];
+            slot.atom[half & 1] = (int)atom;
+            slot.sqrtw[half & 1] = h_weights ? std::sqrt(h_weights[atom]) : 1.0;
+            if ((half & 1) == 0) {  // the partner, unless the group has another atom
+                slot.atom[1] = -1;
+                slot.sqrtw[1] = 0.0;
+            }
+        }
+    }
+    const int64_t points = rn_spectrum_num_points(plan->S);
+    if (points == 0) return RN_OK;
+    RN_CHECK_ARG(d_wavenumbers && d_intensities, "null output pointer");
+    DeviceGuard guard(plan->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int64_t table_bytes = (int64_t)sizeof(VdosSlot) * num_slots;
+    const int64_t need = table_bytes + (int64_t)sizeof(int64_t) * (num_groups + 1);
+    if (need > plan->vdos_bytes) {  // kept with the plan; calls on one plan are ordered on one stream
+        RN_CUDA(cudaStreamSynchronize(s));
+        cudaFree(plan->d_vdos);
+        plan->d_vdos = nullptr;
+        plan->vdos_bytes = 0;
+        if (cudaMalloc(&plan->d_vdos, (size_t)need) != cudaSuccess) {
+            cudaGetLastError();
+            set_error("cudaMalloc of %lld bytes of VDOS slot tables failed", (long long)need);
+            return RN_ERR_OUT_OF_MEMORY;
+        }
+        plan->vdos_bytes = need;
+    }
+    char* table = static_cast<char*>(plan->d_vdos);
+    // pageable sources: the copies return once the data is staged, so the vectors may go out of scope
+    RN_CUDA(cudaMemcpyAsync(table, slots.data(), (size_t)table_bytes, cudaMemcpyHostToDevice, s));
+    RN_CUDA(cudaMemcpyAsync(table + table_bytes, group_slots.data(), sizeof(int64_t) * (num_groups + 1),
+                            cudaMemcpyHostToDevice, s));
+    const VdosSlot* d_slots = reinterpret_cast<const VdosSlot*>(table);
+    const int64_t* d_group_slots = reinterpret_cast<const int64_t*>(table + table_bytes);
+
+    const int64_t M = plan->M;
+    const double scale = 0.25 / ((double)plan->L * (double)plan->L);
+    VdosPackParams pp;
+    pp.pos = d_positions;
+    pp.num_atoms = num_atoms;
+    pp.M = M;
+    pp.Lh = plan->Lh;
+    for (int i = 0; i < 9; i++) pp.lattice[i] = h_lattice[i];
+    pp.inv_dt = 1.0 / timestep_fs;
+    pp.dst = plan->d_work;
+    pp.epart = plan->d_epart;
+    pp.ticket = plan->d_ticket;
+    int64_t g_lo = 0;  // first group with a slot in the chunk
+    for (int64_t first = 0; first < num_slots; first += plan->batch) {
+        const int64_t nb = std::min(plan->batch, num_slots - first);
+        while (group_slots[(size_t)g_lo + 1] <= first) g_lo++;
+        int64_t g_hi = g_lo;  // last group with a slot in the chunk
+        while (group_slots[(size_t)g_hi + 1] < first + nb) g_hi++;
+        pp.slots = d_slots + first;
+        pack_velocity_kernel<<<dim3(plan->pack_blocks, (unsigned)nb), kPackThreads, 0, s>>>(pp);
+        RN_LAUNCHED();
+        fft::OutSpec out = plain_out();
+        out.mode = fft::OUT_POWER;
+        out.power = plan->d_power;
+        out.M = M;
+        int rc = run_convolution(plan, plan->d_work, (int)(3 * nb), M, out, nullptr, s);
+        if (rc != RN_OK) return rc;
+        const int64_t groups = g_hi - g_lo + 1;
+        combine_groups_kernel<<<dim3(grid_for(points, plan->sm_count), (unsigned)std::min<int64_t>(groups, 65535)), 256,
+                                0, s>>>(plan->d_power, plan->d_epart + plan->pack_blocks, plan->pack_blocks + 1,
+                                        d_group_slots, first, nb, g_lo, groups, M, scale, points, timestep_fs,
+                                        first == 0 ? d_wavenumbers : nullptr, d_intensities);
+        RN_LAUNCHED();
+        RN_CUDA(cudaGetLastError());
+    }
     return RN_OK;
 }
 

@@ -16,7 +16,7 @@ import numpy as np
 from . import _lib
 from .abstract import Dynamics, PolarizabilityModel
 from .exceptions import get_type_error, verify_ndarray_shape
-from .spectrum import MDRamanSpectrum, PhononRamanSpectrum
+from .spectrum import MDRamanSpectrum, PhononRamanSpectrum, _current_device, _get_plan, _is_integer, _window_batch
 
 RAMAN_TENSOR_CENTRAL_DIFFERENCE = 0.001  # ramannoodle/constants.py:248
 
@@ -27,6 +27,49 @@ def apply_pbc(positions):
         return positions - positions // 1
     except TypeError as exc:
         raise get_type_error("positions", positions, "ndarray") from exc
+
+
+def _host_array(value):
+    return value.detach().cpu().numpy() if _lib.is_torch_tensor(value) else np.asarray(value)
+
+
+def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_frames: int):
+    """Validate the arguments of ``get_vdos``; returns the lattice (3,3), the group offsets (G+1,) and atoms of the
+    groups as int64, and the weights (N,) or None, all contiguous host arrays."""
+    verify_ndarray_shape("lattice", lattice, (3, 3))
+    lattice = np.ascontiguousarray(_host_array(lattice), dtype=np.float64)
+    if not np.all(np.isfinite(lattice)):
+        raise ValueError("lattice contains non-finite values")
+    if atom_groups is None:
+        atom_groups = [range(num_atoms)]
+    if isinstance(atom_groups, (str, bytes)) or not isinstance(atom_groups, (Sequence, np.ndarray)):
+        raise get_type_error("atom_groups", atom_groups, "list")
+    if len(atom_groups) == 0:
+        raise ValueError("atom_groups is empty")
+    offsets, atoms = [0], []
+    for g, group in enumerate(atom_groups):
+        if isinstance(group, (str, bytes)) or not isinstance(group, (Sequence, np.ndarray)):
+            raise get_type_error(f"atom_groups[{g}]", group, "list")
+        if len(group) == 0:
+            raise ValueError(f"atom_groups[{g}] is empty")
+        for atom in group:
+            if not _is_integer(atom):
+                raise get_type_error(f"atom_groups[{g}] entry", atom, "int")
+            if not 0 <= atom < num_atoms:
+                raise ValueError(f"atom_groups[{g}] has atom index {atom} out of range [0, {num_atoms})")
+        if len(set(int(atom) for atom in group)) != len(group):
+            raise ValueError(f"atom_groups[{g}] repeats an atom")
+        atoms.extend(int(atom) for atom in group)
+        offsets.append(len(atoms))
+    weights = None
+    if atom_weights is not None:
+        verify_ndarray_shape("atom_weights", atom_weights, (num_atoms,))
+        weights = np.ascontiguousarray(_host_array(atom_weights), dtype=np.float64)
+        if not np.all(np.isfinite(weights)) or np.any(weights < 0):
+            raise ValueError("atom_weights must be finite and >= 0")
+    if num_frames < 2:
+        raise ValueError("positions_ts must contain at least 2 frames")
+    return lattice, np.asarray(offsets, dtype=np.int64), np.asarray(atoms, dtype=np.int64), weights
 
 
 class Trajectory(Dynamics, Sequence):
@@ -148,6 +191,54 @@ class Trajectory(Dynamics, Sequence):
         except ValueError as exc:
             raise ValueError("polarizability_model and trajectory are incompatible") from exc
         return [MDRamanSpectrum(series[g], self._timestep) for g in range(series.shape[0])]
+
+    def get_vdos_device(self, lattice, atom_groups=None, atom_weights=None):
+        """``get_vdos`` with the result left on the GPU (two CUDA tensors)."""
+        num_frames, num_atoms = int(self._positions_ts.shape[0]), int(self._positions_ts.shape[1])
+        lattice, offsets, atoms, weights = _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms, num_frames)
+        import torch  # pylint: disable=import-outside-toplevel
+
+        points = int(_lib.lib().rn_spectrum_num_points(num_frames))
+        positions = self._positions_ts
+        if not _lib.is_torch_tensor(positions):  # host (pinned) trajectory: one copy to the device
+            positions = torch.from_numpy(np.ascontiguousarray(positions, dtype=np.float64)).to(
+                f"cuda:{_current_device()}")
+        device = int(positions.device.index or 0)
+        num_groups = len(offsets) - 1
+        with torch.cuda.device(device):
+            wavenumbers = torch.empty(points, dtype=torch.float64, device=positions.device)
+            intensities = torch.empty((num_groups, points), dtype=torch.float64, device=positions.device)
+            if points > 0:
+                slots = int(np.sum((np.diff(offsets) + 1) // 2))
+                plan = _get_plan(num_frames, device, _window_batch(num_frames, slots))
+                status = _lib.lib().rn_vdos(
+                    plan.handle, ctypes.c_void_p(positions.data_ptr()), num_atoms, ctypes.c_void_p(lattice.ctypes.data),
+                    None if weights is None else ctypes.c_void_p(weights.ctypes.data),
+                    ctypes.c_void_p(offsets.ctypes.data), ctypes.c_void_p(atoms.ctypes.data), num_groups,
+                    self._timestep, ctypes.c_void_p(wavenumbers.data_ptr()),
+                    ctypes.c_void_p(intensities.data_ptr()), _lib.current_stream(device))
+                _lib.check(status, "rn_vdos")
+        return wavenumbers, intensities
+
+    def get_vdos(self, lattice, atom_groups=None, atom_weights=None):
+        """Vibrational density of states -> (wavenumbers, vdos), numpy arrays of shape (P,) and (G, P),
+        P = ceil((S-1)/2) - 1.
+
+        ``lattice`` is the (3,3) cell in Å with lattice vectors as rows (the convention of ``io.read_lattice``
+        and the models).  ``atom_groups`` is a sequence of G non-empty sequences of atom indices in [0, N),
+        without repeats inside a group (groups may overlap); the default is one group of all atoms.
+        ``atom_weights`` (N,) are finite and >= 0 (masses give the mass-weighted VDOS); the default is ones.
+
+        Row g is by definition ``sum_{i in group g} sum_c atom_weights[i] * calc_signal_spectrum(v[:, i, c],
+        timestep)[1][1:]`` with the velocities ``v = (d @ lattice) / timestep`` (Å/fs) of the minimum-image
+        steps ``d`` between consecutive frames: the power spectrum of the velocities, 0 cm^-1 bin dropped, no
+        corrections.  The wavenumbers are those of ``MDRamanSpectrum(series of S frames, timestep).measure()``
+        bit for bit, so VDOS and Raman peaks share the bins.  All groups run as one batched transform on the
+        GPU.  A device-resident trajectory is read in place; a host trajectory is copied to the device once
+        (its S·N·24 bytes must fit there).  Argument errors are raised before any device work.
+        """
+        wavenumbers, vdos = self.get_vdos_device(lattice, atom_groups, atom_weights)
+        return wavenumbers.cpu().numpy(), vdos.cpu().numpy()
 
     def __len__(self) -> int:
         return int(self._positions_ts.shape[0])
