@@ -237,6 +237,20 @@ int rn_md_cross_spectra(rn_spectrum_plan* plan, const double* d_alpha, int64_t n
 int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms, const double* h_lattice,
             const double* h_weights, const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups,
             double timestep_fs, double* d_wavenumbers, double* d_intensities, void* stream);
+/* Projected VDOS: power spectra of the velocities projected on K vectors, e.g. normal-mode velocities (no
+ * reference counterpart).  d_positions is a contiguous (S,N,3) array of fractional positions, plan a single-GPU
+ * plan of S frames (rn_spectrum_plan_create or rn_spectrum_plan_create_batched); h_lattice the (3,3) lattice in
+ * Angstrom, rows are lattice vectors; h_vectors (K,N,3) finite.  -> d_wavenumbers (P,), d_intensities (K,P),
+ * P = rn_spectrum_num_points(S): row k is calc_signal_spectrum(q_k, timestep)[1:] (spectrum/utils.py:95-124) of
+ * q_k = sum_{i,c} vectors[k,i,c] v[:,i,c] with the minimum-image velocity v = (wrap(x[n+1] - x[n]) @ lattice) /
+ * timestep in Angstrom/fs; the wavenumbers are those of rn_md_spectrum.  Six modes fill the three sequences of a
+ * window; windows run in chunks of the plan's batch (one projection on the FP64 tensor pipe, the transform and
+ * one combine per chunk) and the result is bit-identical for every batch.  A zero vector gives a zero row.  The
+ * plan keeps the projection matrix (6 ceil(K/6) + 64 rows of 3N doubles rounded up to 16) and the energy
+ * partials of the frame tiles between calls.  P = 0 launches nothing. */
+int rn_projected_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms, const double* h_lattice,
+                      const double* h_vectors, int64_t num_vectors, double timestep_fs, double* d_wavenumbers,
+                      double* d_intensities, void* stream);
 /* One transform shared by the ranks of a multi-GPU run (one process per GPU; no reference
  * counterpart — same result as rn_md_spectrum on the whole series).  The chirp-z transform of
  * length L is decimated in frequency over the G = 2, 4 or 8 ranks of the group (the largest power

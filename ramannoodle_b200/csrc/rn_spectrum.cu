@@ -57,6 +57,8 @@ struct rn_spectrum_plan {
     int64_t cross_doubles = 0;
     void* d_vdos = nullptr;     // VDOS: slot table, then the slot offsets of the groups
     int64_t vdos_bytes = 0;
+    double* d_proj = nullptr;   // projected VDOS: projection matrix, energy partials of the frame tiles, their sums
+    int64_t proj_bytes = 0;
 };
 
 namespace rn {
@@ -713,6 +715,268 @@ __global__ void __launch_bounds__(256) combine_groups_kernel(const double* __res
             wn_out[o] = wavenumber_of(o + 1, M, dt);
 }
 
+// ---- projected VDOS (rn_projected_vdos) ---------------------------------------------------------------
+// Row k is calc_signal_spectrum(q_k) of the mode velocity q_k[n] = sum_{i,c} vectors[k,i,c] v[n,i,c].  With the
+// lattice and 1/dt folded into the projection matrix B[(i,a), k] = sum_c lattice[a,c] vectors[k,i,c] / dt,
+// q_k[n] = sum_{(i,a)} wrap(x[n+1] - x[n])_(i,a) B[(i,a), k]: a (frames x 3N) x (3N x modes) product on the FP64
+// tensor pipe whose left factor is formed from the positions as they stream in.  Modes 2j and 2j+1 of a chunk
+// travel as sequence j = q_2j + i q_2j+1 of the work buffer; the real signals are separated after the transform.
+
+constexpr int kPvFT = 128;     // differences per frame tile: 8 MMA warps x 16
+constexpr int kPvNT = 64;      // modes per mode tile (blockIdx.x)
+constexpr int kPvKC = 16;      // coordinates per pipeline chunk
+constexpr int kPvRS = 20;      // padded smem row stride (doubles): conflict-free fragment loads
+constexpr int kPvStages = 4;   // ring slots; the copies run two chunks ahead
+constexpr int kPvThreads = 384;  // 8 MMA warps, then 4 producer warps
+constexpr size_t kPvSmemBytes = (size_t)kPvStages * ((kPvFT + 1) + kPvNT) * kPvRS * sizeof(double) +
+                                2 * kPvStages * sizeof(uint64_t);
+
+struct ProjParams {
+    const double* pos;     // (S,N,3) fractional, wrapped
+    int64_t cols;          // 3N
+    int64_t M, Lh;
+    const double* bt;      // the chunk's rows of the transposed projection matrix: (modes, rpad), zero padded
+    int rpad;              // 3N rounded up to kPvKC
+    int nseq;              // 3 nb sequences of the chunk's work buffer
+    int64_t tiles;         // frame tiles: ceil(M / kPvFT)
+    double2* dst;          // (3 nb, Lh) work buffer
+    double* epart;         // (gridDim.x kPvNT, tiles) energy of every mode in every frame tile
+    double* energy;        // (gridDim.x kPvNT) their sums
+    unsigned int* ticket;  // zero between launches
+};
+
+__device__ __forceinline__ void mbar_arrive_cta(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+
+// CTA (x, y): mode tile x of the chunk, a contiguous range of frame tiles.  Producers copy frames
+// n0 .. n0 + kPvFT (one halo frame) and kPvKC coordinates per ring slot with cp.async, replace them in place by
+// the minimum-image steps wrap_disp(x[n+1], x[n]) (the function pack_velocity_kernel uses) and release the slot;
+// the MMA warps contract it with the slot's kPvNT x kPvKC block of B.  Epilogue per frame tile: chirp
+// pre-multiply, store of the packed pairs, and the tile's energy of every mode (a fixed tree, no value atomics);
+// the CTA that finishes last sums every mode's tiles in tile order, so the energies do not depend on the grid.
+template <bool ALIGN16>
+__global__ void __launch_bounds__(kPvThreads, 1) project_velocity_kernel(const __grid_constant__ ProjParams P) {
+    extern __shared__ __align__(16) unsigned char pv_smem[];  // 16: the module's other kernels keep their layout
+    double* As = reinterpret_cast<double*>(pv_smem);                 // [stages][kPvFT + 1][kPvRS]
+    double* Bs = As + (size_t)kPvStages * (kPvFT + 1) * kPvRS;      // [stages][kPvNT][kPvRS]
+    uint64_t* bars = reinterpret_cast<uint64_t*>(Bs + (size_t)kPvStages * kPvNT * kPvRS);
+    __shared__ double red[8][kPvNT];
+    __shared__ bool last;
+    const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + kPvStages);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int chunks = P.rpad / kPvKC;
+    const int64_t tile_begin = P.tiles * blockIdx.y / gridDim.y, tile_end = P.tiles * (blockIdx.y + 1) / gridDim.y;
+    const int64_t total = (tile_end - tile_begin) * chunks;
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < kPvStages; s++) {
+            mbar_init(full0 + 8 * s, 128);  // every producer thread arrives after its steps
+            mbar_init(empty0 + 8 * s, 8);   // one arrival per MMA warp
+        }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+
+    if (warp >= 8) {
+        // =========================== producers (128 threads) ===========================
+        const int ptid = threadIdx.x - 256;
+        constexpr int SEGS = ALIGN16 ? kPvKC / 2 : kPvKC, ELEMS = ALIGN16 ? 2 : 1;
+        constexpr int A_ITEMS = ((kPvFT + 1) * SEGS + 127) / 128;
+        const int w_col = ptid & 15, w_row0 = (ptid >> 4) * 16;  // the 16 steps this thread forms
+        const double* bt_src = P.bt + (int64_t)blockIdx.x * kPvNT * P.rpad;
+        uint32_t is_st = 0, is_round = 0, wr_st = 0;
+        int64_t is_tile = tile_begin;
+        int is_kc = 0;
+        auto issue = [&]() {
+            if (is_tile < tile_end) {
+                const uint32_t st = is_st;
+                if (is_round > 0) mbar_wait(empty0 + 8 * st, (is_round - 1) & 1);  // consumed one round earlier
+                const int64_t tile = is_tile;
+                const int kc = is_kc;
+                const uint32_t a_dst = smem_u32(As + (size_t)st * (kPvFT + 1) * kPvRS);
+#pragma unroll
+                for (int i = 0; i < A_ITEMS; i++) {
+                    const int e = ptid + 128 * i;
+                    const int row = e / SEGS, seg = e % SEGS;
+                    if (row <= kPvFT) {
+                        const int64_t frame = tile * kPvFT + row;
+                        const int64_t col = (int64_t)kc * kPvKC + seg * ELEMS;
+                        const bool ok = frame <= P.M && col < P.cols;  // zero fill past the last frame / coordinate
+                        const double* src = ok ? P.pos + frame * P.cols + col : P.pos;
+                        const uint32_t d = a_dst + (uint32_t)(row * kPvRS + seg * ELEMS) * 8u;
+                        if (ALIGN16) cp_async_16(d, src, ok ? 16 : 0);
+                        else cp_async_8(d, src, ok ? 8 : 0);
+                    }
+                }
+                const uint32_t b_dst = smem_u32(Bs + (size_t)st * kPvNT * kPvRS);
+#pragma unroll
+                for (int i = 0; i < (kPvNT * 8) / 128; i++) {
+                    const int e = ptid + 128 * i;
+                    const int row = e >> 3, seg = e & 7;
+                    cp_async_16(b_dst + (uint32_t)(row * kPvRS + seg * 2) * 8u,
+                                bt_src + (int64_t)row * P.rpad + kc * kPvKC + seg * 2, 16);
+                }
+                if (++is_kc == chunks) {
+                    is_kc = 0;
+                    ++is_tile;
+                }
+                if (++is_st == (uint32_t)kPvStages) {
+                    is_st = 0;
+                    ++is_round;
+                }
+            }
+            cp_async_commit();
+        };
+        issue();
+        issue();
+        for (int64_t c = 0; c < total; c++) {
+            issue();             // item c+2
+            cp_async_wait<2>();  // this thread's copies of item c have landed
+            asm volatile("bar.sync 1, 128;" ::: "memory");  // ... and every producer's
+            double* a = As + (size_t)wr_st * (kPvFT + 1) * kPvRS + w_col;
+            const double halo = a[(w_row0 + 16) * kPvRS];  // the next thread's first frame, before it is replaced
+            asm volatile("bar.sync 1, 128;" ::: "memory");
+            double prev = a[w_row0 * kPvRS];
+#pragma unroll
+            for (int r = 0; r < 16; r++) {
+                const double next = r < 15 ? a[(w_row0 + r + 1) * kPvRS] : halo;
+                a[(w_row0 + r) * kPvRS] = wrap_disp(next, prev);
+                prev = next;
+            }
+            mbar_arrive_cta(full0 + 8 * wr_st);  // release: this thread's steps are visible to the MMA warps
+            if (++wr_st == (uint32_t)kPvStages) wr_st = 0;
+        }
+        cp_async_wait<0>();
+        return;
+    }
+
+    // =============================== MMA warps (256 threads) ===============================
+    const int g = lane >> 2, t = lane & 3;
+    const int wm = warp;  // differences 16 wm .. 16 wm + 15 of a tile
+    const int seq0 = blockIdx.x * (kPvNT / 2);
+    uint32_t co_st = 0, co_round = 0;
+    for (int64_t tile = tile_begin; tile < tile_end; tile++) {
+        double acc[2][8][2];
+#pragma unroll
+        for (int mt = 0; mt < 2; mt++)
+#pragma unroll
+            for (int nt = 0; nt < 8; nt++) acc[mt][nt][0] = acc[mt][nt][1] = 0.0;
+        for (int kc = 0; kc < chunks; kc++) {
+            const uint32_t st = co_st;
+            mbar_wait(full0 + 8 * st, co_round & 1);
+            const double* a_src = As + (size_t)st * (kPvFT + 1) * kPvRS + (wm * 16 + g) * kPvRS + t;
+            const double* b_src = Bs + (size_t)st * kPvNT * kPvRS + g * kPvRS + t;
+#pragma unroll
+            for (int s = 0; s < kPvKC / 4; s++) {
+                double af[2], bf[8];
+#pragma unroll
+                for (int mt = 0; mt < 2; mt++) af[mt] = a_src[mt * 8 * kPvRS + 4 * s];
+#pragma unroll
+                for (int nt = 0; nt < 8; nt++) bf[nt] = b_src[nt * 8 * kPvRS + 4 * s];
+#pragma unroll
+                for (int nt = 0; nt < 8; nt++)
+#pragma unroll
+                    for (int mt = 0; mt < 2; mt++) dmma884(acc[mt][nt][0], acc[mt][nt][1], af[mt], bf[nt]);
+            }
+            __syncwarp();
+            if (lane == 0) mbar_arrive_cta(empty0 + 8 * st);  // slot may be refilled
+            if (++co_st == (uint32_t)kPvStages) {
+                co_st = 0;
+                ++co_round;
+            }
+        }
+        // lane (g, t) holds q of difference 8 mt + g for modes 8 nt + 2t and 8 nt + 2t + 1: one packed value
+        double e[8][2];
+#pragma unroll
+        for (int nt = 0; nt < 8; nt++) e[nt][0] = e[nt][1] = 0.0;
+#pragma unroll
+        for (int mt = 0; mt < 2; mt++) {
+            const int64_t n = tile * kPvFT + wm * 16 + mt * 8 + g;
+            if (n < P.M) {
+                const double2 c = chirp(n, P.M);
+                double2* out = P.dst + (int64_t)(seq0 + t) * P.Lh + n;  // sequence seq0 + 4 nt + t
+#pragma unroll
+                for (int nt = 0; nt < 8; nt++) {
+                    const double2 z = make_double2(acc[mt][nt][0], acc[mt][nt][1]);
+                    e[nt][0] += z.x * z.x;
+                    e[nt][1] += z.y * z.y;
+                    if (seq0 + nt * 4 + t < P.nseq) *out = cmul(z, c);
+                    out += 4 * P.Lh;
+                }
+            }
+        }
+#pragma unroll
+        for (int nt = 0; nt < 8; nt++)
+#pragma unroll
+            for (int c = 0; c < 2; c++)
+#pragma unroll
+                for (int off = 4; off < 32; off <<= 1) e[nt][c] += __shfl_xor_sync(0xffffffffu, e[nt][c], off);
+        if (g == 0)
+#pragma unroll
+            for (int nt = 0; nt < 8; nt++) {
+                red[wm][nt * 8 + 2 * t] = e[nt][0];
+                red[wm][nt * 8 + 2 * t + 1] = e[nt][1];
+            }
+        asm volatile("bar.sync 2, 256;" ::: "memory");
+        if (threadIdx.x < kPvNT) {
+            double sum = 0.0;
+#pragma unroll
+            for (int w = 0; w < 8; w++) sum += red[w][threadIdx.x];
+            P.epart[((int64_t)blockIdx.x * kPvNT + threadIdx.x) * P.tiles + tile] = sum;
+        }
+        asm volatile("bar.sync 2, 256;" ::: "memory");  // `red` is reused
+    }
+    __threadfence();
+    asm volatile("bar.sync 2, 256;" ::: "memory");
+    if (threadIdx.x == 0) last = atomicAdd(P.ticket, 1u) == gridDim.x * gridDim.y - 1;
+    asm volatile("bar.sync 2, 256;" ::: "memory");
+    if (!last) return;
+    __threadfence();
+    for (int64_t m = warp; m < (int64_t)gridDim.x * kPvNT; m += 8) {
+        double v = 0.0;
+        for (int64_t b = lane; b < P.tiles; b += 32) v += __ldcg(P.epart + m * P.tiles + b);
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+        if (lane == 0) P.energy[m] = v;
+    }
+    if (threadIdx.x == 0) *P.ticket = 0;
+}
+
+// Rows first_mode + 2j and first_mode + 2j + 1 (those < num_modes) of int_out (num_modes, points) from sequence j
+// of the transform outputs y (natural order; the spectrum is Z[m] = chirp(m) y[m] / L).  The two real signals of
+// z = a + i b separate as A = (Z[k] + conj Z[M-k]) / 2 and B = (Z[k] - conj Z[M-k]) / (2i), formed before they
+// are squared, and each row is (|X|^2 + E) / 2 as in combine_signal_kernel with scale = 1 / (8 L^2) for the
+// unhalved sums.  A mode of zero energy is the zero signal: its row is exactly zero, free of its partner's
+// rounding.
+__global__ void __launch_bounds__(256) combine_modes_kernel(const double2* __restrict__ y, int64_t Lh, int nseq,
+                                                            const double* __restrict__ energy, int64_t first_mode,
+                                                            int64_t num_modes, int64_t M, double scale,
+                                                            int64_t points, double dt, double* __restrict__ wn_out,
+                                                            double* __restrict__ int_out) {
+    for (int64_t j = blockIdx.y; j < nseq; j += gridDim.y) {
+        const int64_t a = first_mode + 2 * j;
+        if (a >= num_modes) break;  // sequences past the last mode carry padding only
+        const bool has_b = a + 1 < num_modes;
+        const double ea = energy[2 * j], eb = energy[2 * j + 1];
+        const double2* yj = y + j * Lh;
+        for (int64_t o = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; o < points;
+             o += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t k = o + 1;
+            const double2 z1 = cmul(yj[k], chirp(k, M)), z2 = cmul(yj[M - k], chirp(M - k, M));
+            const double ax = z1.x + z2.x, ay = z1.y - z2.y;
+            int_out[a * points + o] = ea == 0.0 ? 0.0 : __fma_rn(ax * ax + ay * ay, scale, 0.5 * ea);
+            if (has_b) {
+                const double bx = z1.y + z2.y, by = z1.x - z2.x;
+                int_out[(a + 1) * points + o] = eb == 0.0 ? 0.0 : __fma_rn(bx * bx + by * by, scale, 0.5 * eb);
+            }
+        }
+    }
+    if (wn_out && blockIdx.y == 0)
+        for (int64_t o = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; o < points;
+             o += (int64_t)gridDim.x * blockDim.x)
+            wn_out[o] = wavenumber_of(o + 1, M, dt);
+}
+
 static int grid_for(int64_t n, int sms) {
     return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)sms * 16));
 }
@@ -830,6 +1094,7 @@ static void destroy_plan(rn_spectrum_plan* p) {
     cudaFree(p->d_ticket);
     cudaFree(p->d_cross);
     cudaFree(p->d_vdos);
+    cudaFree(p->d_proj);
     delete p;
 }
 
@@ -1285,6 +1550,96 @@ extern "C" int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_
                                 0, s>>>(plan->d_power, plan->d_epart + plan->pack_blocks, plan->pack_blocks + 1,
                                         d_group_slots, first, nb, g_lo, groups, M, scale, points, timestep_fs,
                                         first == 0 ? d_wavenumbers : nullptr, d_intensities);
+        RN_LAUNCHED();
+        RN_CUDA(cudaGetLastError());
+    }
+    return RN_OK;
+}
+
+// The modes, padded to windows of six, run in chunks of the plan's batch: per chunk one projection (the
+// trajectory streamed once per 64 modes of the chunk), the convolution of its 3 nb sequences with OUT_PLAIN and
+// one combine that separates the packed pairs into their rows.
+extern "C" int rn_projected_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms,
+                                 const double* h_lattice, const double* h_vectors, int64_t num_vectors,
+                                 double timestep_fs, double* d_wavenumbers, double* d_intensities, void* stream) {
+    RN_CHECK_ARG(plan != nullptr, "plan is null");
+    RN_CHECK_ARG(plan->world == 1, "rn_projected_vdos needs a single-GPU plan (rn_spectrum_plan_create_batched)");
+    RN_CHECK_ARG(d_positions && h_lattice && h_vectors, "null pointer");
+    RN_CHECK_ARG(num_atoms >= 1 && num_atoms <= INT32_MAX / 3, "invalid num_atoms %lld", (long long)num_atoms);
+    RN_CHECK_ARG(num_vectors >= 1 && num_vectors <= INT32_MAX / 3, "invalid num_vectors %lld",
+                 (long long)num_vectors);
+    RN_CHECK_ARG(timestep_fs > 0 && std::isfinite(timestep_fs), "timestep must be positive");
+    for (int i = 0; i < 9; i++) RN_CHECK_ARG(std::isfinite(h_lattice[i]), "lattice entry %d is not finite", i);
+    const int64_t cols = 3 * num_atoms;
+    for (int64_t e = 0; e < num_vectors * cols; e++)
+        RN_CHECK_ARG(std::isfinite(h_vectors[e]), "entry %lld of vectors is not finite", (long long)e);
+    const int64_t points = rn_spectrum_num_points(plan->S);
+    if (points == 0) return RN_OK;
+    RN_CHECK_ARG(d_wavenumbers && d_intensities, "null output pointer");
+    DeviceGuard guard(plan->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int64_t M = plan->M;
+    const int64_t rpad = (cols + kPvKC - 1) / kPvKC * kPvKC;
+    const int64_t windows = (num_vectors + 5) / 6;  // six modes per window of the plan
+    const int64_t rows = 6 * windows + kPvNT;       // a chunk's last mode tile reads up to 63 rows past its modes
+    const int64_t tiles = (M + kPvFT - 1) / kPvFT;
+    const int64_t mtiles_max = (6 * std::min(plan->batch, windows) + kPvNT - 1) / kPvNT;
+    const int64_t matrix = rows * rpad, parts = mtiles_max * kPvNT * tiles;
+    const int64_t need = (int64_t)sizeof(double) * (matrix + parts + mtiles_max * kPvNT);
+    if (need > plan->proj_bytes) {  // kept with the plan; calls on one plan are ordered on one stream
+        RN_CUDA(cudaStreamSynchronize(s));
+        cudaFree(plan->d_proj);
+        plan->d_proj = nullptr;
+        plan->proj_bytes = 0;
+        if (cudaMalloc((void**)&plan->d_proj, (size_t)need) != cudaSuccess) {
+            cudaGetLastError();
+            set_error("cudaMalloc of %lld bytes of projection matrix and energy partials failed", (long long)need);
+            return RN_ERR_OUT_OF_MEMORY;
+        }
+        plan->proj_bytes = need;
+    }
+    // B^T[k][3i + a] = sum_c lattice[a][c] vectors[k][i][c] / dt; padding rows (modes >= K) and columns are zero
+    std::vector<double> bt((size_t)matrix, 0.0);
+    for (int64_t k = 0; k < num_vectors; k++)
+        for (int64_t i = 0; i < num_atoms; i++) {
+            const double* v = h_vectors + (k * num_atoms + i) * 3;
+            for (int a = 0; a < 3; a++)
+                bt[(size_t)(k * rpad + 3 * i + a)] =
+                    (h_lattice[3 * a] * v[0] + h_lattice[3 * a + 1] * v[1] + h_lattice[3 * a + 2] * v[2]) / timestep_fs;
+        }
+    // pageable source: the copy returns once the data is staged, so the vector may go out of scope
+    RN_CUDA(cudaMemcpyAsync(plan->d_proj, bt.data(), sizeof(double) * (size_t)matrix, cudaMemcpyHostToDevice, s));
+
+    const bool align16 = reinterpret_cast<uintptr_t>(d_positions) % 16 == 0 && cols % 2 == 0;
+    const auto kernel = align16 ? project_velocity_kernel<true> : project_velocity_kernel<false>;
+    RN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPvSmemBytes));
+    ProjParams pp;
+    pp.pos = d_positions;
+    pp.cols = cols;
+    pp.M = M;
+    pp.Lh = plan->Lh;
+    pp.rpad = (int)rpad;
+    pp.tiles = tiles;
+    pp.dst = plan->d_work;
+    pp.epart = plan->d_proj + matrix;
+    pp.energy = pp.epart + parts;
+    pp.ticket = plan->d_ticket;
+    const double scale = 0.125 / ((double)plan->L * (double)plan->L);
+    for (int64_t first = 0; first < windows; first += plan->batch) {
+        const int64_t nb = std::min(plan->batch, windows - first);
+        const int64_t mtiles = (6 * nb + kPvNT - 1) / kPvNT;
+        pp.bt = plan->d_proj + 6 * first * rpad;
+        pp.nseq = (int)(3 * nb);
+        // mode tiles of one frame range run side by side, so the second reads the frames from L2
+        const int64_t ranges = std::max<int64_t>(1, std::min<int64_t>(tiles, plan->sm_count / mtiles));
+        kernel<<<dim3((unsigned)mtiles, (unsigned)ranges), kPvThreads, kPvSmemBytes, s>>>(pp);
+        RN_LAUNCHED();
+        int rc = run_convolution(plan, plan->d_work, (int)(3 * nb), M, plain_out(), nullptr, s);
+        if (rc != RN_OK) return rc;
+        combine_modes_kernel<<<dim3(grid_for(points, plan->sm_count), (unsigned)std::min<int64_t>(3 * nb, 65535)), 256,
+                               0, s>>>(plan->d_work, plan->Lh, (int)(3 * nb), pp.energy, 6 * first, num_vectors, M,
+                                       scale, points, timestep_fs, first == 0 ? d_wavenumbers : nullptr,
+                                       d_intensities);
         RN_LAUNCHED();
         RN_CUDA(cudaGetLastError());
     }

@@ -33,13 +33,19 @@ def _host_array(value):
     return value.detach().cpu().numpy() if _lib.is_torch_tensor(value) else np.asarray(value)
 
 
-def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_frames: int):
-    """Validate the arguments of ``get_vdos``; returns the lattice (3,3), the group offsets (G+1,) and atoms of the
-    groups as int64, and the weights (N,) or None, all contiguous host arrays."""
+def _check_lattice(lattice) -> np.ndarray:
+    """The (3,3) lattice as a contiguous float64 host array; raises for a wrong type, shape or a non-finite entry."""
     verify_ndarray_shape("lattice", lattice, (3, 3))
     lattice = np.ascontiguousarray(_host_array(lattice), dtype=np.float64)
     if not np.all(np.isfinite(lattice)):
         raise ValueError("lattice contains non-finite values")
+    return lattice
+
+
+def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_frames: int):
+    """Validate the arguments of ``get_vdos``; returns the lattice (3,3), the group offsets (G+1,) and atoms of the
+    groups as int64, and the weights (N,) or None, all contiguous host arrays."""
+    lattice = _check_lattice(lattice)
     if atom_groups is None:
         atom_groups = [range(num_atoms)]
     if isinstance(atom_groups, (str, bytes)) or not isinstance(atom_groups, (Sequence, np.ndarray)):
@@ -70,6 +76,23 @@ def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_fra
     if num_frames < 2:
         raise ValueError("positions_ts must contain at least 2 frames")
     return lattice, np.asarray(offsets, dtype=np.int64), np.asarray(atoms, dtype=np.int64), weights
+
+
+def _check_projection_args(lattice, vectors, num_atoms: int, num_frames: int):
+    """Validate the arguments of ``get_projected_vdos``; returns the lattice (3,3) and the vectors (K,N,3) as
+    contiguous float64 host arrays."""
+    lattice = _check_lattice(lattice)
+    verify_ndarray_shape("vectors", vectors, (None, None, 3))
+    if vectors.shape[1] != num_atoms:
+        raise ValueError(f"vectors has {vectors.shape[1]} atoms, the trajectory {num_atoms}")
+    if vectors.shape[0] == 0:
+        raise ValueError("vectors is empty")
+    vectors = np.ascontiguousarray(_host_array(vectors), dtype=np.float64)
+    if not np.all(np.isfinite(vectors)):
+        raise ValueError("vectors contains non-finite values")
+    if num_frames < 2:
+        raise ValueError("positions_ts must contain at least 2 frames")
+    return lattice, vectors
 
 
 class Trajectory(Dynamics, Sequence):
@@ -199,10 +222,7 @@ class Trajectory(Dynamics, Sequence):
         import torch  # pylint: disable=import-outside-toplevel
 
         points = int(_lib.lib().rn_spectrum_num_points(num_frames))
-        positions = self._positions_ts
-        if not _lib.is_torch_tensor(positions):  # host (pinned) trajectory: one copy to the device
-            positions = torch.from_numpy(np.ascontiguousarray(positions, dtype=np.float64)).to(
-                f"cuda:{_current_device()}")
+        positions = self._device_positions()
         device = int(positions.device.index or 0)
         num_groups = len(offsets) - 1
         with torch.cuda.device(device):
@@ -239,6 +259,65 @@ class Trajectory(Dynamics, Sequence):
         """
         wavenumbers, vdos = self.get_vdos_device(lattice, atom_groups, atom_weights)
         return wavenumbers.cpu().numpy(), vdos.cpu().numpy()
+
+    def _device_positions(self):
+        """The positions as a CUDA tensor: a device trajectory in place, a host (pinned) one copied once."""
+        if _lib.is_torch_tensor(self._positions_ts):
+            return self._positions_ts
+        import torch  # pylint: disable=import-outside-toplevel
+
+        return torch.from_numpy(np.ascontiguousarray(self._positions_ts, dtype=np.float64)).to(
+            f"cuda:{_current_device()}")
+
+    def get_projected_vdos_device(self, lattice, vectors):
+        """``get_projected_vdos`` with the result left on the GPU (two CUDA tensors)."""
+        num_frames, num_atoms = int(self._positions_ts.shape[0]), int(self._positions_ts.shape[1])
+        lattice, vectors = _check_projection_args(lattice, vectors, num_atoms, num_frames)
+        import torch  # pylint: disable=import-outside-toplevel
+
+        points = int(_lib.lib().rn_spectrum_num_points(num_frames))
+        positions = self._device_positions()
+        device = int(positions.device.index or 0)
+        num_vectors = int(vectors.shape[0])
+        with torch.cuda.device(device):
+            wavenumbers = torch.empty(points, dtype=torch.float64, device=positions.device)
+            intensities = torch.empty((num_vectors, points), dtype=torch.float64, device=positions.device)
+            if points > 0:
+                # a window's three sequences carry six modes
+                plan = _get_plan(num_frames, device, _window_batch(num_frames, -(-num_vectors // 6)))
+                status = _lib.lib().rn_projected_vdos(
+                    plan.handle, ctypes.c_void_p(positions.data_ptr()), num_atoms, ctypes.c_void_p(lattice.ctypes.data),
+                    ctypes.c_void_p(vectors.ctypes.data), num_vectors, self._timestep,
+                    ctypes.c_void_p(wavenumbers.data_ptr()), ctypes.c_void_p(intensities.data_ptr()),
+                    _lib.current_stream(device))
+                _lib.check(status, "rn_projected_vdos")
+        return wavenumbers, intensities
+
+    def get_projected_vdos(self, lattice, vectors):
+        """Power spectra of the velocities projected on K vectors -> (wavenumbers, rows), numpy arrays of shape
+        (P,) and (K, P), P = ceil((S-1)/2) - 1.
+
+        ``lattice`` is the (3,3) cell in Å with lattice vectors as rows.  ``vectors`` (K, N, 3), K >= 1, finite,
+        numpy, a CPU or a CUDA tensor (read on the host); ``vectors[k, i]`` is a Cartesian 3-vector of atom i.
+
+        Row k is by definition ``calc_signal_spectrum(q_k, timestep)[1][1:]`` of the projected velocity
+        ``q_k[n] = sum_{i,c} vectors[k, i, c] * v[n, i, c]``, with the velocities ``v = (d @ lattice) /
+        timestep`` (Å/fs) of the minimum-image steps ``d`` between consecutive frames, exactly as ``get_vdos``
+        forms them: 0 cm^-1 bin dropped, no corrections.  The rows are in (Å/fs)^2 times the units of
+        ``vectors`` squared; the wavenumbers are those of ``MDRamanSpectrum(series of S frames,
+        timestep).measure()`` and ``get_vdos`` bit for bit.  A zero vector gives an exactly zero row.
+
+        With ``Phonons.get_mode_vectors`` row k is the spectrum of the normal-mode velocity of mode k: its
+        anharmonic frequency and linewidth.  Sum rule: for any 3N orthonormal vectors e_k (over all 3N
+        coordinates) and ``vectors[k, i] = sqrt(m_i) e_{k,i}``, ``rows.sum(0)`` equals ``get_vdos(lattice,
+        atom_weights=m)[1][0]`` up to rounding, since an orthogonal change of basis commutes with the DFT.
+
+        The projection runs on the FP64 tensor pipe and the rows as one batched transform on the GPU.  A
+        device-resident trajectory is read in place; a host trajectory is copied to the device once (its S·N·24
+        bytes must fit there).  Argument errors are raised before any device work.
+        """
+        wavenumbers, rows = self.get_projected_vdos_device(lattice, vectors)
+        return wavenumbers.cpu().numpy(), rows.cpu().numpy()
 
     def __len__(self) -> int:
         return int(self._positions_ts.shape[0])
@@ -280,6 +359,32 @@ class Phonons(Dynamics):
     @property
     def displacements(self) -> np.ndarray:
         return self._displacements.copy()
+
+    def get_mode_vectors(self, lattice, atom_masses) -> np.ndarray:
+        """Projection vectors of the normal modes for ``Trajectory.get_projected_vdos`` -> (M, N, 3) numpy array.
+
+        ``lattice`` (3,3) in Å, lattice vectors as rows; ``atom_masses`` (N,) finite and > 0 (e.g. in amu).
+        The stored displacements are eigenvectors divided by sqrt(m) in fractional coordinates, so the
+        eigenvector of mode k is ``e_k = normalize(sqrt(m_i) * (displacements[k, i] @ lattice))`` over all 3N
+        coordinates; the result is ``sqrt(m_i) * e_{k,i}``.  With these vectors row k of ``get_projected_vdos``
+        is the power spectrum of the normal-mode velocity ``q_k = sum_i sqrt(m_i) e_{k,i} . v_i`` in
+        amu (Å/fs)^2 for masses in amu.  The eigenvectors are not orthogonalised (degenerate pairs would mix
+        arbitrarily); when they are orthonormal and complete, the rows add up to the mass-weighted
+        ``get_vdos(lattice, atom_weights=atom_masses)``.  Raises ValueError for a mode of zero norm.
+        """
+        lattice = _check_lattice(lattice)
+        num_atoms = self._ref_positions.shape[0]
+        verify_ndarray_shape("atom_masses", atom_masses, (num_atoms,))
+        masses = np.asarray(_host_array(atom_masses), dtype=np.float64)
+        if not np.all(np.isfinite(masses)) or np.any(masses <= 0):
+            raise ValueError("atom_masses must be finite and > 0")
+        sqrt_m = np.sqrt(masses)[None, :, None]
+        eigenvectors = sqrt_m * (np.asarray(self._displacements, dtype=np.float64) @ lattice)
+        norms = np.sqrt(np.sum(eigenvectors * eigenvectors, axis=(1, 2)))
+        zero = np.flatnonzero(norms == 0)
+        if zero.size:
+            raise ValueError(f"mode {zero[0]} has zero norm")
+        return sqrt_m * (eigenvectors / norms[:, None, None])
 
     def get_raman_spectrum(self, polarizability_model: PolarizabilityModel) -> PhononRamanSpectrum:
         epsilon = self._displacements * RAMAN_TENSOR_CENTRAL_DIFFERENCE
