@@ -251,6 +251,21 @@ int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms
 int rn_projected_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms, const double* h_lattice,
                       const double* h_vectors, int64_t num_vectors, double timestep_fs, double* d_wavenumbers,
                       double* d_intensities, void* stream);
+/* Mean squared displacement of G atom groups (no reference counterpart).  plan is a single-GPU plan created for
+ * S + 1 frames (rn_spectrum_plan_create or rn_spectrum_plan_create_batched), so that its M is S and its L >= 2S - 1,
+ * the length of a linear autocorrelation of S values; d_positions is a contiguous (S,N,3) array of fractional
+ * positions, S = M; h_lattice the (3,3) lattice in Angstrom, rows are lattice vectors; group g is the atoms
+ * h_atoms[h_group_offsets[g] .. h_group_offsets[g+1]-1] (CSR, non-empty, indices in [0, N)).  -> d_msd (G,S) in
+ * Angstrom^2: with the minimum-image steps d = wrap(x[n+1] - x[n]) of rn_vdos, their integer image shifts
+ * k = x[n+1] - x[n] - d and K(n) = sum_{j<n} k_j, the unwrapped path is r_i(n) = (x_i(n) - x_i(0) - K_i(n)) @ lattice
+ * and row g at lag m = 0 .. S-1 is (1/|g|) sum_{i in g} (1/(S-m)) sum_{n<S-m} |r_i(n+m) - r_i(n)|^2; lag 0 is
+ * exactly 0.  Two memberships of a group form a slot (the slots of rn_vdos); slots run in chunks of the plan's
+ * batch (a count pass, an unwrap + pack, the transform with |X|^2 in place of the filter and one combine per
+ * chunk, then one finishing launch) and every row is bit-identical for every batch, for repeated calls and
+ * whether its group is computed alone or with others.  The plan keeps the slot table (24 bytes per slot plus
+ * 16 (G+1)) and the image shifts of the frame blocks (48 ceil(S/256) bytes per slot of a chunk) between calls. */
+int rn_msd(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms, const double* h_lattice,
+           const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups, double* d_msd, void* stream);
 /* One transform shared by the ranks of a multi-GPU run (one process per GPU; no reference
  * counterpart — same result as rn_md_spectrum on the whole series).  The chirp-z transform of
  * length L is decimated in frequency over the G = 2, 4 or 8 ranks of the group (the largest power

@@ -75,6 +75,8 @@ PROTOTYPES = {
     "rn_projected_vdos": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
                                          ctypes.c_void_p, ctypes.c_int64, ctypes.c_double, ctypes.c_void_p,
                                          ctypes.c_void_p, ctypes.c_void_p]),
+    "rn_msd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                              ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p]),
     "rn_spectrum_plan_create_dist": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                     ctypes.POINTER(ctypes.c_void_p)]),
     "rn_spectrum_plan_info": (ctypes.c_int, [ctypes.c_void_p, c_int64_p]),

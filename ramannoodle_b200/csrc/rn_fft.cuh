@@ -273,7 +273,12 @@ struct TileParams {
     Twiddles tw;
 };
 
-template <bool FWD_ONLY, bool LEAN>
+// AUTOCORR: the filter multiply becomes x[q] -> (|x[q]|^2, 0) and H is not read, so the pass computes
+// L * IFFT(|FFT(z)|^2), the circular autocorrelation of z.  For z = a + i b with a, b real and Z = A + i B,
+// |Z|^2 = |A|^2 + |B|^2 - 2 Im(B conj A); A and B are Hermitian, so Im(B[k] conj A[k]) is odd in k and its
+// inverse transform is purely imaginary.  With plain output, Re(y[m]) / L is therefore the autocorrelation of
+// a plus that of b at lag m, linear for m < L - (length of z) when z is zero-padded.
+template <bool FWD_ONLY, bool LEAN, bool AUTOCORR = false>
 __global__ void __launch_bounds__(kNT, LEAN ? 3 : 2) tile_kernel(const __grid_constant__ TileParams P) {
     extern __shared__ __align__(16) unsigned char fft_smem[];
     double2* S = reinterpret_cast<double2*>(fft_smem);
@@ -303,7 +308,7 @@ __global__ void __launch_bounds__(kNT, LEAN ? 3 : 2) tile_kernel(const __grid_co
         // the filter spectrum of a tile is stored [q][u] (element pos0 + q of butterfly u at q * 512 + u):
         // consecutive threads read consecutive addresses
         const int hu = (int)threadIdx.x + m * kNT;
-        if (!FWD_ONLY) {
+        if (!FWD_ONLY && !AUTOCORR) {
 #pragma unroll
             for (int q = 0; q < 8; q++) h[q] = __ldg(P.H + tile_base + (q << 9) + hu);
         }
@@ -316,7 +321,8 @@ __global__ void __launch_bounds__(kNT, LEAN ? 3 : 2) tile_kernel(const __grid_co
             for (int q = 0; q < 8; q++) P.Hout[tile_base + (q << 9) + hu] = x[q];
         } else {
 #pragma unroll
-            for (int q = 0; q < 8; q++) x[q] = cmul(x[q], h[q]);
+            for (int q = 0; q < 8; q++)
+                x[q] = AUTOCORR ? make_double2(x[q].x * x[q].x + x[q].y * x[q].y, 0.0) : cmul(x[q], h[q]);
             Dft<8, +1>::run(x);
 #pragma unroll
             for (int q = 0; q < 8; q++) S[swz(pos0 + q)] = x[q];

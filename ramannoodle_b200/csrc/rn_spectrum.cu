@@ -977,6 +977,229 @@ __global__ void __launch_bounds__(256) combine_modes_kernel(const double2* __res
             wn_out[o] = wavenumber_of(o + 1, M, dt);
 }
 
+// ---- mean squared displacement (rn_msd) -------------------------------------------------------------
+// With the unwrapped path r(n) = (x(n) - x(0) - K(n)) @ lattice, K(n) = sum_{j<n} k_j the integer image shifts of
+// the minimum-image steps (k_j = ceil(x[j+1] - x[j] - 0.5), so that the step is wrap_disp(x[j+1], x[j])), and
+// D(n) = |r(n)|^2, expanding the square gives
+//   sum_{n<S-m} |r(n+m) - r(n)|^2 = sum_{n<S-m} D(n) + sum_{n>=m} D(n) - 2 C(m),
+// C the linear autocorrelation of r.  A slot (the VDOS slot layout, sqrt(w) = 1) carries the six coordinate paths
+// of its two atoms as z_c = r_a,c + i r_b,c, c = x, y, z: the autocorrelation tile pass turns them into
+// C_a(m) + C_b(m) = Re(y_0 + y_1 + y_2)[m] / L, and D_a + D_b is one row.  The frames of a slot run in blocks of
+// kPackThreads; K and the prefix sums of D combine per-block totals, scanned over the blocks by the block of the
+// slot that finishes last, with in-block scans of a fixed order: every value is bit-reproducible (the K are exact
+// integers in any order).
+
+struct MsdParams {
+    const double* pos;      // (S,N,3) fractional
+    int64_t num_atoms;
+    int64_t S, Lh;
+    int64_t nb;             // slots in the chunk: blockIdx.x = frame block * nb + slot
+    int64_t fblocks;        // frame blocks of a slot
+    const VdosSlot* slots;  // the chunk's slots
+    double lattice[9];      // rows are lattice vectors
+    double* counts;         // (nb, fblocks, 6) image shifts of each block's steps, then their inclusive scan
+    double2* dst;           // (3 nb, Lh) work buffer: r(n), n < S
+    double* dloc;           // (nb, 3 S) power rows: D summed over the frames of its block up to n (inclusive)
+    double* dsum;           // (nb, fblocks + 1) block sums of D, then their inclusive scan
+    unsigned int* ticket;   // nb tickets, zero between launches
+};
+
+// inclusive scan of NV values over the block in a fixed order (bit-reproducible); sm holds NV doubles per warp
+template <int NV>
+__device__ __forceinline__ void block_scan(double (&v)[NV], double* sm) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1)
+#pragma unroll
+        for (int c = 0; c < NV; c++) {
+            const double u = __shfl_up_sync(0xffffffffu, v[c], off);
+            if (lane >= off) v[c] += u;
+        }
+    if (lane == 31)
+#pragma unroll
+        for (int c = 0; c < NV; c++) sm[warp * NV + c] = v[c];
+    __syncthreads();
+    double before[NV];
+#pragma unroll
+    for (int c = 0; c < NV; c++) before[c] = 0.0;
+    for (int w = 0; w < warp; w++)
+#pragma unroll
+        for (int c = 0; c < NV; c++) before[c] += sm[w * NV + c];
+#pragma unroll
+    for (int c = 0; c < NV; c++) v[c] += before[c];
+    __syncthreads();  // sm is reused
+}
+
+// The last thread publishes its block's totals (NV values) at vals + NV * fb of the slot's row of `count` blocks;
+// the slot's block that finishes last replaces the row by its inclusive scan and re-arms the ticket.
+template <int NV>
+__device__ __forceinline__ void publish_and_scan(const double (&total)[NV], double* vals, int64_t fb, int64_t count,
+                                                 unsigned int* ticket, double* sm) {
+    __shared__ bool last;
+    if (threadIdx.x == blockDim.x - 1) {
+#pragma unroll
+        for (int c = 0; c < NV; c++) vals[fb * NV + c] = total[c];
+        __threadfence();
+        last = atomicAdd(ticket, 1u) == (unsigned int)(count - 1);
+    }
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    double carry[NV];
+#pragma unroll
+    for (int c = 0; c < NV; c++) carry[c] = 0.0;
+    for (int64_t base = 0; base < count; base += blockDim.x) {
+        const int64_t i = base + threadIdx.x;
+        double v[NV];
+#pragma unroll
+        for (int c = 0; c < NV; c++) v[c] = i < count ? __ldcg(vals + i * NV + c) : 0.0;
+        block_scan<NV>(v, sm);
+#pragma unroll
+        for (int c = 0; c < NV; c++) {
+            v[c] = carry[c] + v[c];
+            if (i < count) vals[i * NV + c] = v[c];
+        }
+        if (threadIdx.x == blockDim.x - 1)
+#pragma unroll
+            for (int c = 0; c < NV; c++) sm[c] = v[c];
+        __syncthreads();
+#pragma unroll
+        for (int c = 0; c < NV; c++) carry[c] = sm[c];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *ticket = 0;
+}
+
+// frames first .. first + avail - 1 of the slot's two atoms into rows (6 per frame); atom -1 reads as zero
+__device__ __forceinline__ void stage_slot_frames(const MsdParams& P, const VdosSlot& slot, int64_t first, int64_t avail,
+                                                  double* rows, int frames) {
+    const int64_t frame_stride = 3 * P.num_atoms;
+    for (int e = threadIdx.x; e < frames * 6; e += blockDim.x) {
+        const int f = e / 6, j = e - 6 * (e / 6);
+        const int atom = j < 3 ? slot.atom[0] : slot.atom[1];
+        rows[e] = (f < avail && atom >= 0) ? __ldg(P.pos + (first + f) * frame_stride + 3 * atom + (j < 3 ? j : j - 3))
+                                           : 0.0;
+    }
+}
+
+// Count pass: the image shifts of the steps n -> n + 1 of a frame block (its frames and the next block's first),
+// summed per block, then scanned over the slot's blocks.
+__global__ void __launch_bounds__(kPackThreads) msd_count_kernel(const __grid_constant__ MsdParams P) {
+    __shared__ double rows[(kPackThreads + 1) * 6];
+    __shared__ double sm[6 * (kPackThreads / 32)];
+    const int64_t j = blockIdx.x % P.nb, fb = blockIdx.x / P.nb;
+    const int64_t first = fb * kPackThreads;
+    const int64_t avail = min((int64_t)kPackThreads + 1, P.S - first);
+    stage_slot_frames(P, P.slots[j], first, avail, rows, kPackThreads + 1);
+    __syncthreads();
+    double k[6];
+#pragma unroll
+    for (int e = 0; e < 6; e++)
+        k[e] = threadIdx.x + 1 < avail ? ceil((rows[(threadIdx.x + 1) * 6 + e] - rows[threadIdx.x * 6 + e]) - 0.5) : 0.0;
+    block_scan<6>(k, sm);
+    publish_and_scan<6>(k, P.counts + j * P.fblocks * 6, fb, P.fblocks, P.ticket + j, sm);
+}
+
+// Unwrap + pack: r(n) of the slot's two atoms from the block's base shifts and an in-block scan of the step shifts,
+// stored as the three sequences z_c (no chirp: a plain zero-padded correlation), and the in-block prefix sums of D.
+__global__ void __launch_bounds__(kPackThreads) msd_pack_kernel(const __grid_constant__ MsdParams P) {
+    __shared__ double rows[kPackThreads * 6];
+    __shared__ double origin[6];
+    __shared__ double sm[6 * (kPackThreads / 32)];
+    const int64_t j = blockIdx.x % P.nb, fb = blockIdx.x / P.nb;
+    const VdosSlot slot = P.slots[j];
+    const int64_t first = fb * kPackThreads;
+    const int64_t avail = min((int64_t)kPackThreads, P.S - first);
+    stage_slot_frames(P, slot, first, avail, rows, kPackThreads);
+    if (threadIdx.x < 6) {
+        const int atom = slot.atom[threadIdx.x / 3];
+        origin[threadIdx.x] = atom >= 0 ? __ldg(P.pos + 3 * atom + threadIdx.x % 3) : 0.0;
+    }
+    __syncthreads();
+    const int t = threadIdx.x;
+    double k[6];
+#pragma unroll
+    for (int e = 0; e < 6; e++) k[e] = (t >= 1 && t < avail) ? ceil((rows[t * 6 + e] - rows[(t - 1) * 6 + e]) - 0.5) : 0.0;
+    block_scan<6>(k, sm);  // K(n) - K(first)
+    double d[1] = {0.0};
+    const int64_t n = first + t;
+    if (t < avail) {
+        const double* base = fb > 0 ? P.counts + (j * P.fblocks + fb - 1) * 6 : nullptr;  // K(first)
+        double2 z[3];
+#pragma unroll
+        for (int m = 0; m < 2; m++) {
+            double u[3];
+#pragma unroll
+            for (int e = 0; e < 3; e++) {
+                const double shift = base ? __ldcg(base + 3 * m + e) + k[3 * m + e] : k[3 * m + e];
+                u[e] = (rows[t * 6 + 3 * m + e] - origin[3 * m + e]) - shift;
+            }
+#pragma unroll
+            for (int c = 0; c < 3; c++) {
+                const double r = u[0] * P.lattice[c] + u[1] * P.lattice[3 + c] + u[2] * P.lattice[6 + c];
+                if (m == 0) z[c].x = r;
+                else z[c].y = r;
+            }
+        }
+        d[0] = (z[0].x * z[0].x + z[1].x * z[1].x + z[2].x * z[2].x) + (z[0].y * z[0].y + z[1].y * z[1].y + z[2].y * z[2].y);
+        double2* dst = P.dst + j * 3 * P.Lh;
+#pragma unroll
+        for (int c = 0; c < 3; c++) dst[(int64_t)c * P.Lh + n] = z[c];
+    }
+    block_scan<1>(d, sm);
+    if (t < avail) P.dloc[j * 3 * P.S + n] = d[0];
+    publish_and_scan<1>(d, P.dsum + j * (P.fblocks + 1), fb, P.fblocks, P.ticket + j, sm);
+}
+
+// sum_{n<k} D(n) of a slot: the scanned totals of the blocks before n's block plus the in-block prefix
+__device__ __forceinline__ double d_prefix(const double* dloc, const double* dsum, int64_t k) {
+    if (k == 0) return 0.0;
+    const int64_t n = k - 1, b = n / kPackThreads;
+    return b > 0 ? dsum[b - 1] + dloc[n] : dloc[n];
+}
+
+// Rows g_lo .. g_lo + num_groups - 1 of out (G, S), for the slots first .. first + nb - 1 of this chunk: row g at lag m
+// is the sum, over its slots in slot order, of A(m) - 2 C(m) with A(m) = sum_{n<S-m} D(n) + sum_{n>=m} D(n).  A
+// group's first slot writes the row and later slots add to it one at a time, as combine_groups_kernel does.
+__global__ void __launch_bounds__(256) msd_combine_kernel(const double2* __restrict__ y, int64_t Lh,
+                                                          const double* __restrict__ dloc,
+                                                          const double* __restrict__ dsum, int64_t dsum_stride,
+                                                          const int64_t* __restrict__ group_slots, int64_t first,
+                                                          int64_t nb, int64_t g_lo, int64_t num_groups, int64_t S,
+                                                          double inv_l, double* __restrict__ out) {
+    for (int64_t g = g_lo + blockIdx.y; g < g_lo + num_groups; g += gridDim.y) {
+        const int64_t begin = group_slots[g];
+        const int64_t s0 = max(begin, first), s1 = min(group_slots[g + 1], first + nb);
+        double* row = out + g * S;
+        for (int64_t m = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; m < S; m += (int64_t)gridDim.x * blockDim.x) {
+            double acc = begin < first ? row[m] : 0.0;
+#pragma unroll 1
+            for (int64_t slot = s0; slot < s1; slot++) {
+                const int64_t j = slot - first;
+                const double2* yj = y + j * 3 * Lh;
+                const double c = (yj[m].x + yj[Lh + m].x) + yj[2 * Lh + m].x;
+                const double* dl = dloc + j * 3 * S;
+                const double* ds = dsum + j * dsum_stride;
+                const double a = d_prefix(dl, ds, S - m) + (d_prefix(dl, ds, S) - d_prefix(dl, ds, m));
+                const double term = __fma_rn(-2.0 * inv_l, c, a);
+                acc = slot == begin ? term : __dadd_rn(acc, term);
+            }
+            row[m] = acc;
+        }
+    }
+}
+
+// MSD_g(m) = row_g(m) / ((S - m) |g|); lag 0 is exactly 0
+__global__ void __launch_bounds__(256) msd_finish_kernel(const int64_t* __restrict__ group_offsets, int64_t num_groups,
+                                                         int64_t S, double* __restrict__ out) {
+    for (int64_t g = blockIdx.y; g < num_groups; g += gridDim.y) {
+        const double size = (double)(group_offsets[g + 1] - group_offsets[g]);
+        double* row = out + g * S;
+        for (int64_t m = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; m < S; m += (int64_t)gridDim.x * blockDim.x)
+            row[m] = m == 0 ? 0.0 : row[m] / ((double)(S - m) * size);
+    }
+}
+
 static int grid_for(int64_t n, int sms) {
     return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)sms * 16));
 }
@@ -990,6 +1213,8 @@ static int ensure_smem_attr(int device) {
     RN_FFT_SMEM((fft::tile_kernel<false, false>));
     RN_FFT_SMEM((fft::tile_kernel<false, true>));
     RN_FFT_SMEM((fft::tile_kernel<true, false>));
+    RN_FFT_SMEM((fft::tile_kernel<false, false, true>));
+    RN_FFT_SMEM((fft::tile_kernel<false, true, true>));
     RN_FFT_SMEM((fft::level_kernel<-1, false>));
     RN_FFT_SMEM((fft::level_kernel<-1, true>));
     RN_FFT_SMEM((fft::level_kernel<+1, false>));
@@ -1049,8 +1274,9 @@ static int launch_level(const rn_spectrum_plan* p, double2* X, int nseq, int seq
 // forward levels, tile pass (with the filter), inverse levels: X (nseq, Lh) in place.  `limit`: input
 // elements at or beyond it are zero (never read); `out`: where the inverse transform's result goes.
 // hout != nullptr: forward transform only, written to hout (plan creation: the filter spectrum).
+// autocorr: |X|^2 in place of the filter multiply (tile_kernel's AUTOCORR), the circular autocorrelation of X.
 static int run_convolution(const rn_spectrum_plan* p, double2* X, int nseq, int64_t limit, const fft::OutSpec& out,
-                           double2* hout, cudaStream_t stream, int seq_base = 0) {
+                           double2* hout, cudaStream_t stream, int seq_base = 0, bool autocorr = false) {
     int rc = ensure_smem_attr(p->device);
     if (rc != RN_OK) return rc;
     const fft::OutSpec plain = plain_out();
@@ -1070,6 +1296,9 @@ static int run_convolution(const rn_spectrum_plan* p, double2* X, int nseq, int6
     T.tw = plan_twiddles(p);
     const unsigned grid = (unsigned)((int64_t)nseq * T.tiles_per_seq);
     if (hout) fft::tile_kernel<true, false><<<grid, kNT, fft::kTileSmemBytes, stream>>>(T);
+    else if (autocorr && (fft_lean() & 2))
+        fft::tile_kernel<false, true, true><<<grid, kNT, fft::kTileSmemBytes, stream>>>(T);
+    else if (autocorr) fft::tile_kernel<false, false, true><<<grid, kNT, fft::kTileSmemBytes, stream>>>(T);
     else if (fft_lean() & 2) fft::tile_kernel<false, true><<<grid, kNT, fft::kTileSmemBytes, stream>>>(T);
     else fft::tile_kernel<false, false><<<grid, kNT, fft::kTileSmemBytes, stream>>>(T);
     RN_LAUNCHED();
@@ -1449,6 +1678,68 @@ extern "C" int rn_md_cross_spectra(rn_spectrum_plan* plan, const double* d_alpha
     return RN_OK;
 }
 
+// The slots of G atom groups (CSR: group g is h_atoms[h_group_offsets[g] .. h_group_offsets[g+1]-1], checked here):
+// two memberships of a group per slot, in group order; a group of odd size pads its last slot with atom -1, the
+// zero signal.  group_slots (G+1) receives the slot offsets of the groups.
+static int make_slots(const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups, int64_t num_atoms,
+                      const double* h_weights, std::vector<int64_t>& group_slots, std::vector<VdosSlot>& slots) {
+    RN_CHECK_ARG(h_group_offsets[0] == 0, "group offsets must start at 0");
+    group_slots.assign((size_t)num_groups + 1, 0);
+    for (int64_t g = 0; g < num_groups; g++) {
+        const int64_t size = h_group_offsets[g + 1] - h_group_offsets[g];
+        RN_CHECK_ARG(size >= 1, "group %lld is empty", (long long)g);
+        group_slots[(size_t)g + 1] = group_slots[(size_t)g] + (size + 1) / 2;
+    }
+    slots.assign((size_t)group_slots[(size_t)num_groups], VdosSlot{});
+    for (int64_t g = 0; g < num_groups; g++) {
+        for (int64_t m = h_group_offsets[g]; m < h_group_offsets[g + 1]; m++) {
+            const int64_t atom = h_atoms[m];
+            RN_CHECK_ARG(atom >= 0 && atom < num_atoms, "atom index %lld of group %lld out of range [0, %lld)",
+                         (long long)atom, (long long)g, (long long)num_atoms);
+            const int64_t half = m - h_group_offsets[g];
+            VdosSlot& slot = slots[(size_t)(group_slots[(size_t)g] + half / 2)];
+            slot.atom[half & 1] = (int)atom;
+            slot.sqrtw[half & 1] = h_weights ? std::sqrt(h_weights[atom]) : 1.0;
+            if ((half & 1) == 0) {  // the partner, unless the group has another atom
+                slot.atom[1] = -1;
+                slot.sqrtw[1] = 0.0;
+            }
+        }
+    }
+    return RN_OK;
+}
+
+// Uploads the slot table, the groups' slot offsets and (h_group_offsets != nullptr) their atom offsets, in that
+// order, to the plan's slot-table buffer, which grows on demand and keeps scratch_bytes after them.
+static int upload_slots(rn_spectrum_plan* plan, const std::vector<VdosSlot>& slots,
+                        const std::vector<int64_t>& group_slots, const int64_t* h_group_offsets, int64_t scratch_bytes,
+                        cudaStream_t s, char** table_out) {
+    const int64_t table_bytes = (int64_t)sizeof(VdosSlot) * (int64_t)slots.size();
+    const int64_t group_bytes = (int64_t)sizeof(int64_t) * (int64_t)group_slots.size();
+    const int64_t need = table_bytes + group_bytes * (h_group_offsets ? 2 : 1) + scratch_bytes;
+    if (need > plan->vdos_bytes) {  // kept with the plan; calls on one plan are ordered on one stream
+        RN_CUDA(cudaStreamSynchronize(s));
+        cudaFree(plan->d_vdos);
+        plan->d_vdos = nullptr;
+        plan->vdos_bytes = 0;
+        if (cudaMalloc(&plan->d_vdos, (size_t)need) != cudaSuccess) {
+            cudaGetLastError();
+            set_error("cudaMalloc of %lld bytes of VDOS slot tables failed", (long long)need);
+            return RN_ERR_OUT_OF_MEMORY;
+        }
+        plan->vdos_bytes = need;
+    }
+    char* table = static_cast<char*>(plan->d_vdos);
+    // pageable sources: the copies return once the data is staged, so the vectors may go out of scope
+    RN_CUDA(cudaMemcpyAsync(table, slots.data(), (size_t)table_bytes, cudaMemcpyHostToDevice, s));
+    RN_CUDA(cudaMemcpyAsync(table + table_bytes, group_slots.data(), (size_t)group_bytes, cudaMemcpyHostToDevice, s));
+    if (h_group_offsets)
+        RN_CUDA(cudaMemcpyAsync(table + table_bytes + group_bytes, h_group_offsets, (size_t)group_bytes,
+                                cudaMemcpyHostToDevice, s));
+    *table_out = table;
+    return RN_OK;
+}
+
 // The slots of all groups, in group order, run in chunks of the plan's batch: per chunk one velocity pack, the
 // convolution of its 3 nb sequences with OUT_POWER and one combine that adds the chunk's slots to the rows of
 // the groups they belong to.
@@ -1467,56 +1758,21 @@ extern "C" int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_
         for (int64_t i = 0; i < num_atoms; i++)
             RN_CHECK_ARG(std::isfinite(h_weights[i]) && h_weights[i] >= 0, "invalid weight %g of atom %lld",
                          h_weights[i], (long long)i);
-    RN_CHECK_ARG(h_group_offsets[0] == 0, "group offsets must start at 0");
-    std::vector<int64_t> group_slots((size_t)num_groups + 1, 0);
-    for (int64_t g = 0; g < num_groups; g++) {
-        const int64_t size = h_group_offsets[g + 1] - h_group_offsets[g];
-        RN_CHECK_ARG(size >= 1, "group %lld is empty", (long long)g);
-        group_slots[(size_t)g + 1] = group_slots[(size_t)g] + (size + 1) / 2;
-    }
+    std::vector<int64_t> group_slots;
+    std::vector<VdosSlot> slots;
+    int rc = make_slots(h_group_offsets, h_atoms, num_groups, num_atoms, h_weights, group_slots, slots);
+    if (rc != RN_OK) return rc;
     const int64_t num_slots = group_slots[(size_t)num_groups];
-    std::vector<VdosSlot> slots((size_t)num_slots);
-    for (int64_t g = 0; g < num_groups; g++) {
-        for (int64_t m = h_group_offsets[g]; m < h_group_offsets[g + 1]; m++) {
-            const int64_t atom = h_atoms[m];
-            RN_CHECK_ARG(atom >= 0 && atom < num_atoms, "atom index %lld of group %lld out of range [0, %lld)",
-                         (long long)atom, (long long)g, (long long)num_atoms);
-            const int64_t half = m - h_group_offsets[g];
-            VdosSlot& slot = slots[(size_t)(group_slots[(size_t)g] + half / 2)];
-            slot.atom[half & 1] = (int)atom;
-            slot.sqrtw[half & 1] = h_weights ? std::sqrt(h_weights[atom]) : 1.0;
-            if ((half & 1) == 0) {  // the partner, unless the group has another atom
-                slot.atom[1] = -1;
-                slot.sqrtw[1] = 0.0;
-            }
-        }
-    }
     const int64_t points = rn_spectrum_num_points(plan->S);
     if (points == 0) return RN_OK;
     RN_CHECK_ARG(d_wavenumbers && d_intensities, "null output pointer");
     DeviceGuard guard(plan->device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    const int64_t table_bytes = (int64_t)sizeof(VdosSlot) * num_slots;
-    const int64_t need = table_bytes + (int64_t)sizeof(int64_t) * (num_groups + 1);
-    if (need > plan->vdos_bytes) {  // kept with the plan; calls on one plan are ordered on one stream
-        RN_CUDA(cudaStreamSynchronize(s));
-        cudaFree(plan->d_vdos);
-        plan->d_vdos = nullptr;
-        plan->vdos_bytes = 0;
-        if (cudaMalloc(&plan->d_vdos, (size_t)need) != cudaSuccess) {
-            cudaGetLastError();
-            set_error("cudaMalloc of %lld bytes of VDOS slot tables failed", (long long)need);
-            return RN_ERR_OUT_OF_MEMORY;
-        }
-        plan->vdos_bytes = need;
-    }
-    char* table = static_cast<char*>(plan->d_vdos);
-    // pageable sources: the copies return once the data is staged, so the vectors may go out of scope
-    RN_CUDA(cudaMemcpyAsync(table, slots.data(), (size_t)table_bytes, cudaMemcpyHostToDevice, s));
-    RN_CUDA(cudaMemcpyAsync(table + table_bytes, group_slots.data(), sizeof(int64_t) * (num_groups + 1),
-                            cudaMemcpyHostToDevice, s));
+    char* table = nullptr;
+    rc = upload_slots(plan, slots, group_slots, nullptr, 0, s, &table);
+    if (rc != RN_OK) return rc;
     const VdosSlot* d_slots = reinterpret_cast<const VdosSlot*>(table);
-    const int64_t* d_group_slots = reinterpret_cast<const int64_t*>(table + table_bytes);
+    const int64_t* d_group_slots = reinterpret_cast<const int64_t*>(table + sizeof(VdosSlot) * num_slots);
 
     const int64_t M = plan->M;
     const double scale = 0.25 / ((double)plan->L * (double)plan->L);
@@ -1543,7 +1799,7 @@ extern "C" int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_
         out.mode = fft::OUT_POWER;
         out.power = plan->d_power;
         out.M = M;
-        int rc = run_convolution(plan, plan->d_work, (int)(3 * nb), M, out, nullptr, s);
+        rc = run_convolution(plan, plan->d_work, (int)(3 * nb), M, out, nullptr, s);
         if (rc != RN_OK) return rc;
         const int64_t groups = g_hi - g_lo + 1;
         combine_groups_kernel<<<dim3(grid_for(points, plan->sm_count), (unsigned)std::min<int64_t>(groups, 65535)), 256,
@@ -1553,6 +1809,80 @@ extern "C" int rn_vdos(rn_spectrum_plan* plan, const double* d_positions, int64_
         RN_LAUNCHED();
         RN_CUDA(cudaGetLastError());
     }
+    return RN_OK;
+}
+
+// The MSD runs on the VDOS slots (two memberships of a group per slot, unit weights) in chunks of the plan's batch:
+// per chunk the count pass, the unwrap + pack, the autocorrelation of its 3 nb sequences (the transform passes of
+// one measure, the tile pass squaring instead of filtering) and one combine that adds the chunk's slots to their
+// group rows; one finishing launch divides the rows.
+extern "C" int rn_msd(rn_spectrum_plan* plan, const double* d_positions, int64_t num_atoms, const double* h_lattice,
+                      const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups, double* d_msd,
+                      void* stream) {
+    RN_CHECK_ARG(plan != nullptr, "plan is null");
+    RN_CHECK_ARG(plan->world == 1, "rn_msd needs a single-GPU plan (rn_spectrum_plan_create_batched)");
+    RN_CHECK_ARG(d_positions && h_lattice && h_group_offsets && h_atoms && d_msd, "null pointer");
+    RN_CHECK_ARG(num_atoms >= 1 && num_atoms <= INT32_MAX, "invalid num_atoms %lld", (long long)num_atoms);
+    RN_CHECK_ARG(num_groups >= 1, "num_groups must be at least 1 (got %lld)", (long long)num_groups);
+    for (int i = 0; i < 9; i++) RN_CHECK_ARG(std::isfinite(h_lattice[i]), "lattice entry %d is not finite", i);
+    std::vector<int64_t> group_slots;
+    std::vector<VdosSlot> slots;
+    int rc = make_slots(h_group_offsets, h_atoms, num_groups, num_atoms, nullptr, group_slots, slots);
+    if (rc != RN_OK) return rc;
+    const int64_t num_slots = group_slots[(size_t)num_groups];
+    DeviceGuard guard(plan->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int64_t S = plan->M, fblocks = plan->pack_blocks;
+    const int64_t chunk = std::min(plan->batch, (int64_t)INT32_MAX / fblocks);  // the passes' blocks on gridDim.x
+    char* table = nullptr;
+    rc = upload_slots(plan, slots, group_slots, h_group_offsets, (int64_t)sizeof(double) * 6 * fblocks * chunk, s,
+                      &table);
+    if (rc != RN_OK) return rc;
+    const int64_t group_bytes = (int64_t)sizeof(int64_t) * (num_groups + 1);
+    const VdosSlot* d_slots = reinterpret_cast<const VdosSlot*>(table);
+    const int64_t* d_group_slots = reinterpret_cast<const int64_t*>(table + sizeof(VdosSlot) * num_slots);
+    const int64_t* d_group_offsets = reinterpret_cast<const int64_t*>(table + sizeof(VdosSlot) * num_slots + group_bytes);
+
+    MsdParams pp;
+    pp.pos = d_positions;
+    pp.num_atoms = num_atoms;
+    pp.S = S;
+    pp.Lh = plan->Lh;
+    pp.fblocks = fblocks;
+    for (int i = 0; i < 9; i++) pp.lattice[i] = h_lattice[i];
+    pp.counts = reinterpret_cast<double*>(table + sizeof(VdosSlot) * num_slots + 2 * group_bytes);
+    pp.dst = plan->d_work;
+    pp.dloc = plan->d_power;
+    pp.dsum = plan->d_epart;
+    pp.ticket = plan->d_ticket;
+    const double inv_l = 1.0 / (double)plan->L;
+    int64_t g_lo = 0;  // first group with a slot in the chunk
+    for (int64_t first = 0; first < num_slots; first += chunk) {
+        const int64_t nb = std::min(chunk, num_slots - first);
+        while (group_slots[(size_t)g_lo + 1] <= first) g_lo++;
+        int64_t g_hi = g_lo;  // last group with a slot in the chunk
+        while (group_slots[(size_t)g_hi + 1] < first + nb) g_hi++;
+        pp.slots = d_slots + first;
+        pp.nb = nb;
+        // slot fastest: the blocks of neighbouring slots read the same frames side by side
+        const unsigned blocks = (unsigned)(nb * fblocks);
+        msd_count_kernel<<<blocks, kPackThreads, 0, s>>>(pp);
+        RN_LAUNCHED();
+        msd_pack_kernel<<<blocks, kPackThreads, 0, s>>>(pp);
+        RN_LAUNCHED();
+        rc = run_convolution(plan, plan->d_work, (int)(3 * nb), S, plain_out(), nullptr, s, 0, true);
+        if (rc != RN_OK) return rc;
+        const int64_t groups = g_hi - g_lo + 1;
+        msd_combine_kernel<<<dim3(grid_for(S, plan->sm_count), (unsigned)std::min<int64_t>(groups, 65535)), 256, 0,
+                             s>>>(plan->d_work, plan->Lh, plan->d_power, plan->d_epart, plan->pack_blocks + 1,
+                                  d_group_slots, first, nb, g_lo, groups, S, inv_l, d_msd);
+        RN_LAUNCHED();
+        RN_CUDA(cudaGetLastError());
+    }
+    msd_finish_kernel<<<dim3(grid_for(S, plan->sm_count), (unsigned)std::min<int64_t>(num_groups, 65535)), 256, 0, s>>>(
+        d_group_offsets, num_groups, S, d_msd);
+    RN_LAUNCHED();
+    RN_CUDA(cudaGetLastError());
     return RN_OK;
 }
 

@@ -319,6 +319,51 @@ class Trajectory(Dynamics, Sequence):
         wavenumbers, rows = self.get_projected_vdos_device(lattice, vectors)
         return wavenumbers.cpu().numpy(), rows.cpu().numpy()
 
+    def get_msd_device(self, lattice, atom_groups=None):
+        """``get_msd`` with the result left on the GPU (two CUDA tensors)."""
+        num_frames, num_atoms = int(self._positions_ts.shape[0]), int(self._positions_ts.shape[1])
+        lattice, offsets, atoms, _ = _check_vdos_args(lattice, atom_groups, None, num_atoms, num_frames)
+        import torch  # pylint: disable=import-outside-toplevel
+
+        lib = _lib.lib()
+        positions = self._device_positions()
+        device = int(positions.device.index or 0)
+        num_groups = len(offsets) - 1
+        with torch.cuda.device(device):
+            lag_times = torch.arange(num_frames, dtype=torch.float64, device=positions.device) * self._timestep
+            msd = torch.empty((num_groups, num_frames), dtype=torch.float64, device=positions.device)
+            slots = int(np.sum((np.diff(offsets) + 1) // 2))
+            # a plan of S + 1 frames has M = S and L >= 2S - 1: a linear autocorrelation of S values
+            plan = _get_plan(num_frames + 1, device, _window_batch(num_frames + 1, slots))
+            status = lib.rn_msd(plan.handle, ctypes.c_void_p(positions.data_ptr()), num_atoms,
+                                ctypes.c_void_p(lattice.ctypes.data), ctypes.c_void_p(offsets.ctypes.data),
+                                ctypes.c_void_p(atoms.ctypes.data), num_groups, ctypes.c_void_p(msd.data_ptr()),
+                                _lib.current_stream(device))
+            _lib.check(status, "rn_msd")
+        return lag_times, msd
+
+    def get_msd(self, lattice, atom_groups=None):
+        """Mean squared displacement -> (lag_times, msd), numpy arrays of shape (S,) and (G, S) in fs and Å².
+
+        ``lattice`` and ``atom_groups`` are those of ``get_vdos``: the (3,3) cell in Å with lattice vectors as rows,
+        and G non-empty sequences of atom indices in [0, N) without repeats inside a group (groups may overlap); the
+        default is one group of all atoms.  ``lag_times`` is ``np.arange(S) * timestep``.
+
+        The path of atom i is unwrapped with the minimum-image steps of ``get_vdos``: with the steps ``d`` between
+        consecutive frames, their integer image shifts ``k = x[n+1] - x[n] - d`` and ``K(n) = sum_{j<n} k_j``,
+        ``r_i(n) = (x_i(n) - x_i(0) - K_i(n)) @ lattice``.  Row g at lag m is by definition
+        ``mean_{i in g} mean_{n < S-m} |r_i(n+m) - r_i(n)|^2``; ``msd[:, 0]`` is exactly 0.  Every lag comes from
+        one FFT autocorrelation per pair of atoms on the GPU, so the rounding error at lag m is of the order of
+        ``1e-16 * log2(S) * mean_i sum_n |r_i(n)|^2 / (S - m)``, largest at long lags, where few pairs are averaged.
+        A device-resident trajectory is read in place; a host trajectory is copied to the device once (its S·N·24
+        bytes must fit there).  Argument errors are raised before any device work.
+
+        A diffusion coefficient in Å²/fs is the slope of a linear range of lags over 6, for example
+        ``np.polyfit(lag_times[a:b], msd[g, a:b], 1)[0] / 6``.
+        """
+        lag_times, msd = self.get_msd_device(lattice, atom_groups)
+        return lag_times.cpu().numpy(), msd.cpu().numpy()
+
     def __len__(self) -> int:
         return int(self._positions_ts.shape[0])
 
