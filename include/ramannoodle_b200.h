@@ -338,6 +338,22 @@ int rn_convolve_spectra(const double* d_wavenumbers, const double* d_intensities
                         int kind, double width, const double* d_out_wavenumbers, int64_t num_out,
                         double* d_out_intensities, void* d_workspace, void* stream);
 
+/* Radial distribution functions of atom groups (no reference counterpart; Trajectory.get_rdf):
+ * d_positions (S,N,3) fractional, h_lattice (3,3) in Å with lattice vectors as rows, CSR groups (group g is
+ * h_atoms[h_group_offsets[g] .. h_group_offsets[g+1]-1], non-empty, no repeats, groups may overlap) ->
+ * d_rdf (G,G,B) float64.  For a <= b every pair (i in a, j in b, i != j; for a == b the list positions p < q,
+ * counted twice) of every frame adds to bin k = floor(|wrap(x_j - x_i) @ lattice| * B / r_max) when k < B, with the
+ * component-wise minimum image d - ceil(d - 0.5) and every product and sum rounded on its own (no fused multiply-add),
+ * so the integer counts are exact and independent of the launch configuration.  g[a,b,k] = count * V /
+ * (S n_ab shell_k), n_ab = |a||b| - |a n b|, shell_k = (4 pi/3)(e_{k+1}^3 - e_k^3), e_k = k r_max / B, V = |det L|;
+ * a pair with n_ab = 0 gets a zero row and g[b,a] = g[a,b].  Needs 0 < r_max <= w_min/2 (w_c the perpendicular
+ * widths of the cell), where at most one image of a pair lies within r_max.  num_bins in 1..4096.
+ * d_workspace must hold rn_rdf_workspace_size(G, h_group_offsets[G], B) bytes.  Two launches whatever S, N, G, B. */
+size_t rn_rdf_workspace_size(int64_t num_groups, int64_t num_listed_atoms, int64_t num_bins);
+int rn_rdf(const double* d_positions, int64_t num_frames, int64_t num_atoms, const double* h_lattice, double r_max,
+           int64_t num_bins, const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups, double* d_rdf,
+           void* d_workspace, void* stream);
+
 /* Trajectory ingest — replaces the Python text parsing of io.vasp.xdatcar.read_positions_ts
  * (ramannoodle/io/vasp/xdatcar.py:21-56; header/frames as io/vasp/poscar.py:_read_lattice,
  * _read_atomic_symbols, _read_positions).  Host-only (no GPU needed): mmap + a thread pool

@@ -102,6 +102,10 @@ PROTOTYPES = {
     "rn_convolve_spectra": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64,
                                            ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_int64,
                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "rn_rdf_workspace_size": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int64]),
+    "rn_rdf": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_double,
+                              ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                              ctypes.c_void_p, ctypes.c_void_p]),
     "rn_calc_polarizabilities_sweep":(ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64,
                                                       ctypes.c_void_p, ctypes.c_void_p]),
     "rn_calc_polarizabilities_host_sweep": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,

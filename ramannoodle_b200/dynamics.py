@@ -42,10 +42,9 @@ def _check_lattice(lattice) -> np.ndarray:
     return lattice
 
 
-def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_frames: int):
-    """Validate the arguments of ``get_vdos``; returns the lattice (3,3), the group offsets (G+1,) and atoms of the
-    groups as int64, and the weights (N,) or None, all contiguous host arrays."""
-    lattice = _check_lattice(lattice)
+def _check_atom_groups(atom_groups, num_atoms: int):
+    """Validate G atom groups (default: one group of all atoms); returns the group offsets (G+1,) and the atoms of the
+    groups (CSR) as contiguous int64 host arrays."""
     if atom_groups is None:
         atom_groups = [range(num_atoms)]
     if isinstance(atom_groups, (str, bytes)) or not isinstance(atom_groups, (Sequence, np.ndarray)):
@@ -67,6 +66,14 @@ def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_fra
             raise ValueError(f"atom_groups[{g}] repeats an atom")
         atoms.extend(int(atom) for atom in group)
         offsets.append(len(atoms))
+    return np.asarray(offsets, dtype=np.int64), np.asarray(atoms, dtype=np.int64)
+
+
+def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_frames: int):
+    """Validate the arguments of ``get_vdos``; returns the lattice (3,3), the group offsets (G+1,) and atoms of the
+    groups as int64, and the weights (N,) or None, all contiguous host arrays."""
+    lattice = _check_lattice(lattice)
+    offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
     weights = None
     if atom_weights is not None:
         verify_ndarray_shape("atom_weights", atom_weights, (num_atoms,))
@@ -75,7 +82,42 @@ def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_fra
             raise ValueError("atom_weights must be finite and >= 0")
     if num_frames < 2:
         raise ValueError("positions_ts must contain at least 2 frames")
-    return lattice, np.asarray(offsets, dtype=np.int64), np.asarray(atoms, dtype=np.int64), weights
+    return lattice, offsets, atoms, weights
+
+
+RDF_MAX_BINS = 4096  # one shared-memory histogram of the kernel
+
+
+def _cell_widths(lattice: np.ndarray):
+    """(V, w) of a (3,3) lattice: the volume V = |L_0 . (L_1 x L_2)| (exact for an orthorhombic cell, like the C entry's)
+    and the perpendicular widths w_c = V / |L_{c+1} x L_{c+2}|, or None if V is 0."""
+    cross = np.cross(lattice[[1, 2, 0]], lattice[[2, 0, 1]])
+    volume = abs(float(np.dot(lattice[0], cross[0])))
+    return volume, (volume / np.sqrt(np.sum(cross * cross, axis=1)) if volume > 0 else None)
+
+
+def _check_rdf_args(lattice, r_max, num_bins, atom_groups, num_atoms: int, num_frames: int):
+    """Validate the arguments of ``get_rdf`` in the order lattice, r_max, num_bins, atom_groups, frames; returns the
+    lattice (3,3), r_max as a float, and the group offsets and atoms (CSR, int64)."""
+    lattice = _check_lattice(lattice)
+    volume, widths = _cell_widths(lattice)
+    if not volume > 0:
+        raise ValueError("lattice has zero cell volume")
+    if isinstance(r_max, (bool, np.bool_)) or not isinstance(r_max, (int, float, np.integer, np.floating)):
+        raise get_type_error("r_max", r_max, "float")
+    r_max = float(r_max)
+    bound = 0.5 * float(np.min(widths))
+    if not (np.isfinite(r_max) and 0 < r_max <= bound):
+        raise ValueError(f"r_max must be finite and in (0, {bound:.6g}] Å, half the smallest perpendicular width "
+                         f"of the cell (got {r_max})")
+    if not _is_integer(num_bins):
+        raise get_type_error("num_bins", num_bins, "int")
+    if not 1 <= num_bins <= RDF_MAX_BINS:
+        raise ValueError(f"num_bins must be in 1..{RDF_MAX_BINS} (got {num_bins})")
+    offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
+    if num_frames < 1:
+        raise ValueError("positions_ts must contain at least 1 frame")
+    return lattice, r_max, offsets, atoms
 
 
 def _check_projection_args(lattice, vectors, num_atoms: int, num_frames: int):
@@ -363,6 +405,58 @@ class Trajectory(Dynamics, Sequence):
         """
         lag_times, msd = self.get_msd_device(lattice, atom_groups)
         return lag_times.cpu().numpy(), msd.cpu().numpy()
+
+    def get_rdf_device(self, lattice, r_max, num_bins, atom_groups=None):
+        """``get_rdf`` with the result left on the GPU (two CUDA tensors)."""
+        num_frames, num_atoms = int(self._positions_ts.shape[0]), int(self._positions_ts.shape[1])
+        lattice, r_max, offsets, atoms = _check_rdf_args(lattice, r_max, num_bins, atom_groups, num_atoms,
+                                                         num_frames)
+        import torch  # pylint: disable=import-outside-toplevel
+
+        lib = _lib.lib()
+        positions = self._device_positions()
+        device = int(positions.device.index or 0)
+        num_groups = len(offsets) - 1
+        num_bins = int(num_bins)
+        radii = (np.arange(num_bins) + 0.5) * (r_max / num_bins)
+        with torch.cuda.device(device):
+            rdf = torch.empty((num_groups, num_groups, num_bins), dtype=torch.float64, device=positions.device)
+            ws_bytes = int(lib.rn_rdf_workspace_size(num_groups, len(atoms), num_bins))
+            workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=positions.device)
+            status = lib.rn_rdf(ctypes.c_void_p(positions.data_ptr()), num_frames, num_atoms,
+                                ctypes.c_void_p(lattice.ctypes.data), r_max, num_bins,
+                                ctypes.c_void_p(offsets.ctypes.data), ctypes.c_void_p(atoms.ctypes.data), num_groups,
+                                ctypes.c_void_p(rdf.data_ptr()), ctypes.c_void_p(workspace.data_ptr()),
+                                _lib.current_stream(device))
+            _lib.check(status, "rn_rdf")
+            return torch.from_numpy(radii).to(positions.device), rdf
+
+    def get_rdf(self, lattice, r_max, num_bins, atom_groups=None):
+        """Radial distribution functions of atom groups -> (r, g), numpy arrays of shape (B,) and (G, G, B).
+
+        ``lattice`` is the (3,3) cell in Å with lattice vectors as rows; ``atom_groups`` are those of ``get_vdos``: G
+        non-empty sequences of atom indices in [0, N) without repeats inside a group (groups may overlap), by default
+        one group of all atoms.  ``num_bins`` B is an integer in 1..4096, ``r_max`` a float in Å with
+        ``0 < r_max <= w_min / 2``, w_c = V / |L_{c+1} x L_{c+2}| the perpendicular widths of the cell: below that
+        bound at most one image of a pair lies within r_max and the component-wise minimum image finds it, so no sum
+        over images is needed.  A single frame is a valid input.
+
+        With width = r_max / B, ``r = (np.arange(B) + 0.5) * width`` are the bin centres and e_k = k * width the edges.
+        For every group pair a <= b and every frame, each pair (i, j) counts into bin k = floor(|v| / width) when
+        k < B, with ``v = (d - ceil(d - 0.5)) @ lattice`` and d = x_j - x_i: for a == b the pairs of list positions
+        p < q count twice (ordered pairs), for a < b every i in a and j in b with i != j counts once.  Then
+        ``g[a, b, k] = count[a, b, k] * V / (S * n_ab * shell_k)`` with V = |det lattice|, n_ab = |a| |b| - |a n b|
+        the number of ordered pairs and shell_k = (4 pi / 3)(e_{k+1}^3 - e_k^3); a pair of groups with n_ab = 0 (a
+        one-atom group with itself) gets a zero row, and ``g[b, a] == g[a, b]``.  The distances are evaluated in FP64
+        with every product and sum rounded on its own, so the counts are exact integers, the same for every launch
+        configuration and for host and device trajectories.
+
+        The running coordination number of b around a is ``np.cumsum(g[a, b] * shell) * n_ab / (|a| * V)``, with
+        shell the shell volumes above.  A device-resident trajectory is read in place; a host trajectory is copied to
+        the device once (its S·N·24 bytes must fit there).  Argument errors are raised before any device work.
+        """
+        radii, rdf = self.get_rdf_device(lattice, r_max, num_bins, atom_groups)
+        return radii.cpu().numpy(), rdf.cpu().numpy()
 
     def __len__(self) -> int:
         return int(self._positions_ts.shape[0])
