@@ -69,6 +69,11 @@ def _check_atom_groups(atom_groups, num_atoms: int):
     return np.asarray(offsets, dtype=np.int64), np.asarray(atoms, dtype=np.int64)
 
 
+def _num_slots(offsets) -> int:
+    """The slots of the groups with these offsets: the GPU pairs two memberships of a group per slot."""
+    return int(np.sum((np.diff(offsets) + 1) // 2))
+
+
 def _check_vdos_args(lattice, atom_groups, atom_weights, num_atoms: int, num_frames: int):
     """Validate the arguments of ``get_vdos``; returns the lattice (3,3), the group offsets (G+1,) and atoms of the
     groups as int64, and the weights (N,) or None, all contiguous host arrays."""
@@ -264,15 +269,13 @@ class Trajectory(Dynamics, Sequence):
         import torch  # pylint: disable=import-outside-toplevel
 
         points = int(_lib.lib().rn_spectrum_num_points(num_frames))
-        positions = self._device_positions()
-        device = int(positions.device.index or 0)
+        positions, device = self._device_positions()
         num_groups = len(offsets) - 1
         with torch.cuda.device(device):
             wavenumbers = torch.empty(points, dtype=torch.float64, device=positions.device)
             intensities = torch.empty((num_groups, points), dtype=torch.float64, device=positions.device)
             if points > 0:
-                slots = int(np.sum((np.diff(offsets) + 1) // 2))
-                plan = _get_plan(num_frames, device, _window_batch(num_frames, slots))
+                plan = _get_plan(num_frames, device, _window_batch(num_frames, _num_slots(offsets)))
                 status = _lib.lib().rn_vdos(
                     plan.handle, ctypes.c_void_p(positions.data_ptr()), num_atoms, ctypes.c_void_p(lattice.ctypes.data),
                     None if weights is None else ctypes.c_void_p(weights.ctypes.data),
@@ -303,13 +306,15 @@ class Trajectory(Dynamics, Sequence):
         return wavenumbers.cpu().numpy(), vdos.cpu().numpy()
 
     def _device_positions(self):
-        """The positions as a CUDA tensor: a device trajectory in place, a host (pinned) one copied once."""
-        if _lib.is_torch_tensor(self._positions_ts):
-            return self._positions_ts
-        import torch  # pylint: disable=import-outside-toplevel
+        """The positions as a CUDA tensor and its device index: a device trajectory in place, a host (pinned) one
+        copied once."""
+        positions = self._positions_ts
+        if not _lib.is_torch_tensor(positions):
+            import torch  # pylint: disable=import-outside-toplevel
 
-        return torch.from_numpy(np.ascontiguousarray(self._positions_ts, dtype=np.float64)).to(
-            f"cuda:{_current_device()}")
+            positions = torch.from_numpy(np.ascontiguousarray(positions, dtype=np.float64)).to(
+                f"cuda:{_current_device()}")
+        return positions, int(positions.device.index or 0)
 
     def get_projected_vdos_device(self, lattice, vectors):
         """``get_projected_vdos`` with the result left on the GPU (two CUDA tensors)."""
@@ -318,8 +323,7 @@ class Trajectory(Dynamics, Sequence):
         import torch  # pylint: disable=import-outside-toplevel
 
         points = int(_lib.lib().rn_spectrum_num_points(num_frames))
-        positions = self._device_positions()
-        device = int(positions.device.index or 0)
+        positions, device = self._device_positions()
         num_vectors = int(vectors.shape[0])
         with torch.cuda.device(device):
             wavenumbers = torch.empty(points, dtype=torch.float64, device=positions.device)
@@ -364,19 +368,20 @@ class Trajectory(Dynamics, Sequence):
     def get_msd_device(self, lattice, atom_groups=None):
         """``get_msd`` with the result left on the GPU (two CUDA tensors)."""
         num_frames, num_atoms = int(self._positions_ts.shape[0]), int(self._positions_ts.shape[1])
-        lattice, offsets, atoms, _ = _check_vdos_args(lattice, atom_groups, None, num_atoms, num_frames)
+        lattice = _check_lattice(lattice)
+        offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
+        if num_frames < 2:
+            raise ValueError("positions_ts must contain at least 2 frames")
         import torch  # pylint: disable=import-outside-toplevel
 
         lib = _lib.lib()
-        positions = self._device_positions()
-        device = int(positions.device.index or 0)
+        positions, device = self._device_positions()
         num_groups = len(offsets) - 1
         with torch.cuda.device(device):
             lag_times = torch.arange(num_frames, dtype=torch.float64, device=positions.device) * self._timestep
             msd = torch.empty((num_groups, num_frames), dtype=torch.float64, device=positions.device)
-            slots = int(np.sum((np.diff(offsets) + 1) // 2))
             # a plan of S + 1 frames has M = S and L >= 2S - 1: a linear autocorrelation of S values
-            plan = _get_plan(num_frames + 1, device, _window_batch(num_frames + 1, slots))
+            plan = _get_plan(num_frames + 1, device, _window_batch(num_frames + 1, _num_slots(offsets)))
             status = lib.rn_msd(plan.handle, ctypes.c_void_p(positions.data_ptr()), num_atoms,
                                 ctypes.c_void_p(lattice.ctypes.data), ctypes.c_void_p(offsets.ctypes.data),
                                 ctypes.c_void_p(atoms.ctypes.data), num_groups, ctypes.c_void_p(msd.data_ptr()),
@@ -414,8 +419,7 @@ class Trajectory(Dynamics, Sequence):
         import torch  # pylint: disable=import-outside-toplevel
 
         lib = _lib.lib()
-        positions = self._device_positions()
-        device = int(positions.device.index or 0)
+        positions, device = self._device_positions()
         num_groups = len(offsets) - 1
         num_bins = int(num_bins)
         radii = (np.arange(num_bins) + 0.5) * (r_max / num_bins)
