@@ -354,6 +354,24 @@ int rn_rdf(const double* d_positions, int64_t num_frames, int64_t num_atoms, con
            int64_t num_bins, const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups, double* d_rdf,
            void* d_workspace, void* stream);
 
+/* Self part of the Van Hove correlation of atom groups (no reference counterpart; Trajectory.get_van_hove):
+ * d_positions (S,N,3) fractional, S >= 2, h_lattice (3,3) in Å with lattice vectors as rows (non-zero volume),
+ * h_lags (T,) strictly increasing in [0, S), CSR groups as rn_rdf -> d_van_hove (G,T,B) and d_moments (G,T,2)
+ * float64.  Every membership's path is unwrapped with the minimum-image steps of rn_vdos and their exact integer
+ * image shifts, r(n) = (x(n) - x(0) - K(n)) @ lattice; each displacement |r(n+t) - r(n)|, n < S - t, adds to bin
+ * k = floor(|.| * B / r_max) when k < B, every product and sum rounded on its own, so the counts are exact.
+ * van_hove[g,t,k] = count / ((S - t) |g| shell_k) in Å^-3 (shell_k as rn_rdf), moments[g,t] = (sum rr, sum rr^2) /
+ * ((S - t) |g|) over all displacements, summed in an order fixed by S, the lags and the group sizes (bit-identical
+ * across calls, chunkings and group sets).  r_max finite and > 0, num_bins in 1..4096.  d_workspace must hold
+ * rn_van_hove_workspace_size(S, h_group_offsets[G], G, T, B) bytes (paths of at most 1 GiB per membership chunk).
+ * Launches: 4 per membership chunk + 1. */
+size_t rn_van_hove_workspace_size(int64_t num_frames, int64_t num_listed_atoms, int64_t num_groups, int64_t num_lags,
+                                  int64_t num_bins);
+int rn_van_hove(const double* d_positions, int64_t num_frames, int64_t num_atoms, const double* h_lattice,
+                const int64_t* h_lags, int64_t num_lags, double r_max, int64_t num_bins, const int64_t* h_group_offsets,
+                const int64_t* h_atoms, int64_t num_groups, double* d_van_hove, double* d_moments, void* d_workspace,
+                void* stream);
+
 /* Trajectory ingest — replaces the Python text parsing of io.vasp.xdatcar.read_positions_ts
  * (ramannoodle/io/vasp/xdatcar.py:21-56; header/frames as io/vasp/poscar.py:_read_lattice,
  * _read_atomic_symbols, _read_positions).  Host-only (no GPU needed): mmap + a thread pool

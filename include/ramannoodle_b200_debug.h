@@ -29,6 +29,8 @@ void rn_debug_set_dense_split(int mode);
 /* mask sweeps: fused sweep kernels on/off; shortest run of linear models worth fusing (2..4) */
 void rn_debug_set_sweep_fused(int on);
 void rn_debug_set_sweep_min_run(int run);
+/* memberships per chunk of rn_van_hove (whole member tiles, at least one; 0 = automatic) */
+void rn_debug_set_van_hove_chunk(int memberships);
 /* FFT core of the spectrum path (csrc/rn_fft.cuh), single-GPU plans: forward transform of 2^info[2]
  * complex values left in the transform's own digit-reversed order, and IFFT(FFT(in) * H) (unnormalised,
  * natural order) with H the plan's chirp filter spectrum.  d_out must not alias d_in. */

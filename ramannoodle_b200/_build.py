@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "libramannoodle_b200.so")
-SOURCES = ["rn_model.cu", "rn_polarizability.cu", "rn_dense.cu", "rn_spectrum.cu", "rn_trajectory.cu", "rn_smear.cu", "rn_rdf.cu", "rn_host.cu", "rn_ingest.cu", "rn_vasprun.cu", "rn_sweep.cu", "rn_dense_sweep.cu"]
+SOURCES = ["rn_model.cu", "rn_polarizability.cu", "rn_dense.cu", "rn_spectrum.cu", "rn_trajectory.cu", "rn_smear.cu", "rn_rdf.cu", "rn_van_hove.cu", "rn_host.cu", "rn_ingest.cu", "rn_vasprun.cu", "rn_sweep.cu", "rn_dense_sweep.cu"]
 HEADERS = [os.path.join(CSRC, "rn_common.cuh"), os.path.join(CSRC, "rn_device.cuh"), os.path.join(CSRC, "rn_dense_tp.cuh"),
            os.path.join(CSRC, "rn_fft.cuh"), os.path.join(CSRC, "rn_spectrum_plan.cuh"), os.path.join(CSRC, "rn_textparse.hpp"),
            os.path.join(os.path.dirname(HERE), "include", "ramannoodle_b200.h")]

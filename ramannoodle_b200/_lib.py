@@ -106,6 +106,11 @@ PROTOTYPES = {
     "rn_rdf": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_double,
                               ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
                               ctypes.c_void_p, ctypes.c_void_p]),
+    "rn_van_hove_workspace_size": (ctypes.c_size_t, [ctypes.c_int64] * 5),
+    "rn_van_hove": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                                   ctypes.c_int64, ctypes.c_double, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                                   ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                   ctypes.c_void_p]),
     "rn_calc_polarizabilities_sweep":(ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64,
                                                       ctypes.c_void_p, ctypes.c_void_p]),
     "rn_calc_polarizabilities_host_sweep": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
@@ -145,6 +150,7 @@ DEBUG_PROTOTYPES = {
     "rn_debug_set_dense_split": (None, [ctypes.c_int]),
     "rn_debug_set_sweep_fused": (None, [ctypes.c_int]),
     "rn_debug_set_sweep_min_run": (None, [ctypes.c_int]),
+    "rn_debug_set_van_hove_chunk": (None, [ctypes.c_int]),
     "rn_debug_fft_forward": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "rn_debug_fft_convolve": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
 }

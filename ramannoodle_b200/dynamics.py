@@ -115,14 +115,52 @@ def _check_rdf_args(lattice, r_max, num_bins, atom_groups, num_atoms: int, num_f
     if not (np.isfinite(r_max) and 0 < r_max <= bound):
         raise ValueError(f"r_max must be finite and in (0, {bound:.6g}] Å, half the smallest perpendicular width "
                          f"of the cell (got {r_max})")
-    if not _is_integer(num_bins):
-        raise get_type_error("num_bins", num_bins, "int")
-    if not 1 <= num_bins <= RDF_MAX_BINS:
-        raise ValueError(f"num_bins must be in 1..{RDF_MAX_BINS} (got {num_bins})")
+    _check_num_bins(num_bins)
     offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
     if num_frames < 1:
         raise ValueError("positions_ts must contain at least 1 frame")
     return lattice, r_max, offsets, atoms
+
+
+def _check_num_bins(num_bins):
+    """The histogram bin count of ``get_rdf`` and ``get_van_hove``: an integer in 1..RDF_MAX_BINS."""
+    if not _is_integer(num_bins):
+        raise get_type_error("num_bins", num_bins, "int")
+    if not 1 <= num_bins <= RDF_MAX_BINS:
+        raise ValueError(f"num_bins must be in 1..{RDF_MAX_BINS} (got {num_bins})")
+
+
+def _check_van_hove_args(lattice, lags, r_max, num_bins, atom_groups, num_atoms: int, num_frames: int):
+    """Validate the arguments of ``get_van_hove`` in the order lattice, lags, r_max, num_bins, atom_groups, frames;
+    returns the lattice (3,3), the lags (T,) as int64, r_max as a float, and the group offsets and atoms (CSR, int64)."""
+    lattice = _check_lattice(lattice)
+    volume, _ = _cell_widths(lattice)
+    if not volume > 0:
+        raise ValueError("lattice has zero cell volume")
+    if isinstance(lags, (str, bytes)):
+        raise get_type_error("lags", lags, "list")
+    lags = np.asarray(_host_array(lags))
+    if lags.ndim != 1:
+        raise ValueError(f"lags must be 1-D (got shape {lags.shape})")
+    if lags.size == 0:
+        raise ValueError("lags is empty")
+    if lags.dtype.kind not in "iu":
+        raise get_type_error("lags", lags, "int")
+    lags = lags.astype(np.int64)
+    if np.any(np.diff(lags) <= 0):
+        raise ValueError("lags must be strictly increasing")
+    if lags[0] < 0 or lags[-1] >= num_frames:
+        raise ValueError(f"lags must be in [0, {num_frames}) (got {int(lags[0])}..{int(lags[-1])})")
+    if isinstance(r_max, (bool, np.bool_)) or not isinstance(r_max, (int, float, np.integer, np.floating)):
+        raise get_type_error("r_max", r_max, "float")
+    r_max = float(r_max)
+    if not (np.isfinite(r_max) and r_max > 0):
+        raise ValueError(f"r_max must be finite and > 0 (got {r_max})")
+    _check_num_bins(num_bins)
+    offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
+    if num_frames < 2:
+        raise ValueError("positions_ts must contain at least 2 frames")
+    return lattice, np.ascontiguousarray(lags), r_max, offsets, atoms
 
 
 def _check_projection_args(lattice, vectors, num_atoms: int, num_frames: int):
@@ -461,6 +499,63 @@ class Trajectory(Dynamics, Sequence):
         """
         radii, rdf = self.get_rdf_device(lattice, r_max, num_bins, atom_groups)
         return radii.cpu().numpy(), rdf.cpu().numpy()
+
+    def get_van_hove_device(self, lattice, lags, r_max, num_bins, atom_groups=None):
+        """``get_van_hove`` with the result left on the GPU (four CUDA tensors)."""
+        num_frames, num_atoms = int(self._positions_ts.shape[0]), int(self._positions_ts.shape[1])
+        lattice, lags, r_max, offsets, atoms = _check_van_hove_args(lattice, lags, r_max, num_bins, atom_groups,
+                                                                    num_atoms, num_frames)
+        import torch  # pylint: disable=import-outside-toplevel
+
+        lib = _lib.lib()
+        positions, device = self._device_positions()
+        num_groups, num_lags, num_bins = len(offsets) - 1, len(lags), int(num_bins)
+        lag_times = np.asarray(lags, dtype=np.float64) * self._timestep
+        radii = (np.arange(num_bins) + 0.5) * (r_max / num_bins)
+        with torch.cuda.device(device):
+            van_hove = torch.empty((num_groups, num_lags, num_bins), dtype=torch.float64, device=positions.device)
+            moments = torch.empty((num_groups, num_lags, 2), dtype=torch.float64, device=positions.device)
+            ws_bytes = int(lib.rn_van_hove_workspace_size(num_frames, len(atoms), num_groups, num_lags, num_bins))
+            workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=positions.device)
+            status = lib.rn_van_hove(ctypes.c_void_p(positions.data_ptr()), num_frames, num_atoms,
+                                     ctypes.c_void_p(lattice.ctypes.data), ctypes.c_void_p(lags.ctypes.data), num_lags,
+                                     r_max, num_bins, ctypes.c_void_p(offsets.ctypes.data),
+                                     ctypes.c_void_p(atoms.ctypes.data), num_groups,
+                                     ctypes.c_void_p(van_hove.data_ptr()), ctypes.c_void_p(moments.data_ptr()),
+                                     ctypes.c_void_p(workspace.data_ptr()), _lib.current_stream(device))
+            _lib.check(status, "rn_van_hove")
+            return (torch.from_numpy(lag_times).to(positions.device), torch.from_numpy(radii).to(positions.device),
+                    van_hove, moments)
+
+    def get_van_hove(self, lattice, lags, r_max, num_bins, atom_groups=None):
+        """Self part of the Van Hove correlation of atom groups -> (lag_times, r, g_s, moments), numpy arrays of shape
+        (T,), (B,), (G, T, B) and (G, T, 2).
+
+        ``lattice`` is the (3,3) cell in Å with lattice vectors as rows; ``atom_groups`` are those of ``get_vdos``: G
+        non-empty sequences of atom indices in [0, N) without repeats inside a group (groups may overlap), by default
+        one group of all atoms.  ``lags`` are T >= 1 strictly increasing integer frame lags in [0, S);
+        ``lag_times = lags * timestep`` in fs.  ``r_max`` in Å is finite and > 0 (the paths are unwrapped, so it is not
+        bounded by the cell) and ``num_bins`` B an integer in 1..4096; ``r`` are the bin centres of ``get_rdf``.
+
+        The path of atom i is unwrapped as in ``get_msd``: with the minimum-image steps of ``get_vdos``, their integer
+        image shifts and ``K(n)`` their running sum, ``r_i(n) = (x_i(n) - x_i(0) - K_i(n)) @ lattice``.  For lag t,
+        every membership i of group g and every origin n < S - t, the displacement ``|r_i(n+t) - r_i(n)|`` counts into
+        bin k = floor(|.| * B / r_max) when k < B, and ``g_s[g, t, k] = count / ((S - t) |g| shell_k)`` in Å^-3 with the
+        shell volumes of ``get_rdf``: ``sum_k g_s * shell`` is the fraction of displacements shorter than r_max and
+        ``4 pi r^2 g_s`` the radial density.  Lag 0 puts every count in bin 0.  The moments run over all displacements:
+        ``moments[g, t] = (<rr>, <rr^2>)``, the means of ``|.|^2`` and ``|.|^4`` over the (S - t) |g| displacements;
+        ``moments[..., 0]`` is the MSD of ``get_msd`` at those lags up to rounding.  The non-Gaussian parameter is
+        ``alpha2 = 3 * moments[..., 1] / (5 * moments[..., 0] ** 2) - 1``: 0 for Gaussian diffusion and harmonic
+        rattling, positive for hopping.
+
+        The displacements are evaluated in FP64 with every product and sum rounded on its own, so the counts are exact
+        integers; the moments are summed in an order fixed by S, the lags and the group sizes, so every result is the
+        same bit for bit for host and device trajectories, repeated calls and a group computed alone or with others.
+        A device-resident trajectory is read in place; a host trajectory is copied to the device once (its S·N·24
+        bytes must fit there).  Argument errors are raised before any device work.
+        """
+        lag_times, radii, van_hove, moments = self.get_van_hove_device(lattice, lags, r_max, num_bins, atom_groups)
+        return lag_times.cpu().numpy(), radii.cpu().numpy(), van_hove.cpu().numpy(), moments.cpu().numpy()
 
     def __len__(self) -> int:
         return int(self._positions_ts.shape[0])
