@@ -372,6 +372,22 @@ int rn_van_hove(const double* d_positions, int64_t num_frames, int64_t num_atoms
                 const int64_t* h_atoms, int64_t num_groups, double* d_van_hove, double* d_moments, void* d_workspace,
                 void* stream);
 
+/* Distinct part of the Van Hove correlation of atom groups (no reference counterpart;
+ * Trajectory.get_distinct_van_hove): d_positions (S,N,3) fractional, h_lattice (3,3) in Å with lattice vectors as rows,
+ * h_lags (T,) strictly increasing in [0, S), CSR groups as rn_rdf -> d_out (G,G,T,B) float64.  For every ordered group
+ * pair (a, b), lag t, origin n < S - t and pair i in a, j in b, i != j, d = x_j(n+t) - x_i(n) adds to bin
+ * k = floor(|wrap(d) @ lattice| * B / r_max) when k < B, with the wrap, operation order and exact integer counts of
+ * rn_rdf.  g_d[a,b,t,k] = count * V / ((S - t) n_ab shell_k), n_ab and shell_k as rn_rdf, a zero row where n_ab = 0;
+ * not mirrored ([b,a,t] and [a,b,t] differ for t > 0).  Lag-0 rows are bit-identical to rn_rdf's on inputs without
+ * a component at an exact +-1/2 wrap tie.  r_max and num_bins as rn_rdf.  d_workspace must hold
+ * rn_distinct_van_hove_workspace_size(h_group_offsets[G], G, T, B) bytes.  Two launches whatever S, N, T, G, B. */
+size_t rn_distinct_van_hove_workspace_size(int64_t num_listed_atoms, int64_t num_groups, int64_t num_lags,
+                                           int64_t num_bins);
+int rn_distinct_van_hove(const double* d_positions, int64_t num_frames, int64_t num_atoms, const double* h_lattice,
+                         const int64_t* h_lags, int64_t num_lags, double r_max, int64_t num_bins,
+                         const int64_t* h_group_offsets, const int64_t* h_atoms, int64_t num_groups, double* d_out,
+                         void* d_workspace, void* stream);
+
 /* Trajectory ingest — replaces the Python text parsing of io.vasp.xdatcar.read_positions_ts
  * (ramannoodle/io/vasp/xdatcar.py:21-56; header/frames as io/vasp/poscar.py:_read_lattice,
  * _read_atomic_symbols, _read_positions).  Host-only (no GPU needed): mmap + a thread pool

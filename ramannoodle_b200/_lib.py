@@ -111,6 +111,11 @@ PROTOTYPES = {
                                    ctypes.c_int64, ctypes.c_double, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
                                    ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                    ctypes.c_void_p]),
+    "rn_distinct_van_hove_workspace_size": (ctypes.c_size_t, [ctypes.c_int64] * 4),
+    "rn_distinct_van_hove": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p,
+                                            ctypes.c_void_p, ctypes.c_int64, ctypes.c_double, ctypes.c_int64,
+                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                            ctypes.c_void_p, ctypes.c_void_p]),
     "rn_calc_polarizabilities_sweep":(ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64,
                                                       ctypes.c_void_p, ctypes.c_void_p]),
     "rn_calc_polarizabilities_host_sweep": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,

@@ -108,18 +108,30 @@ def _check_rdf_args(lattice, r_max, num_bins, atom_groups, num_atoms: int, num_f
     volume, widths = _cell_widths(lattice)
     if not volume > 0:
         raise ValueError("lattice has zero cell volume")
-    if isinstance(r_max, (bool, np.bool_)) or not isinstance(r_max, (int, float, np.integer, np.floating)):
-        raise get_type_error("r_max", r_max, "float")
-    r_max = float(r_max)
-    bound = 0.5 * float(np.min(widths))
-    if not (np.isfinite(r_max) and 0 < r_max <= bound):
-        raise ValueError(f"r_max must be finite and in (0, {bound:.6g}] Å, half the smallest perpendicular width "
-                         f"of the cell (got {r_max})")
+    r_max = _check_cell_r_max(r_max, widths)
     _check_num_bins(num_bins)
     offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
     if num_frames < 1:
         raise ValueError("positions_ts must contain at least 1 frame")
     return lattice, r_max, offsets, atoms
+
+
+def _check_r_max_type(r_max) -> float:
+    """r_max as a float; raises TypeError for a bool or a non-number."""
+    if isinstance(r_max, (bool, np.bool_)) or not isinstance(r_max, (int, float, np.integer, np.floating)):
+        raise get_type_error("r_max", r_max, "float")
+    return float(r_max)
+
+
+def _check_cell_r_max(r_max, widths) -> float:
+    """The r_max of ``get_rdf`` and ``get_distinct_van_hove``: a float with 0 < r_max <= w_min / 2 for the
+    perpendicular widths w of the cell."""
+    r_max = _check_r_max_type(r_max)
+    bound = 0.5 * float(np.min(widths))
+    if not (np.isfinite(r_max) and 0 < r_max <= bound):
+        raise ValueError(f"r_max must be finite and in (0, {bound:.6g}] Å, half the smallest perpendicular width "
+                         f"of the cell (got {r_max})")
+    return r_max
 
 
 def _check_num_bins(num_bins):
@@ -137,6 +149,20 @@ def _check_van_hove_args(lattice, lags, r_max, num_bins, atom_groups, num_atoms:
     volume, _ = _cell_widths(lattice)
     if not volume > 0:
         raise ValueError("lattice has zero cell volume")
+    lags = _check_lags(lags, num_frames)
+    r_max = _check_r_max_type(r_max)
+    if not (np.isfinite(r_max) and r_max > 0):
+        raise ValueError(f"r_max must be finite and > 0 (got {r_max})")
+    _check_num_bins(num_bins)
+    offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
+    if num_frames < 2:
+        raise ValueError("positions_ts must contain at least 2 frames")
+    return lattice, lags, r_max, offsets, atoms
+
+
+def _check_lags(lags, num_frames: int) -> np.ndarray:
+    """The lags of ``get_van_hove`` and ``get_distinct_van_hove``: T >= 1 strictly increasing integers in [0, S), as
+    a contiguous int64 host array."""
     if isinstance(lags, (str, bytes)):
         raise get_type_error("lags", lags, "list")
     lags = np.asarray(_host_array(lags))
@@ -151,16 +177,22 @@ def _check_van_hove_args(lattice, lags, r_max, num_bins, atom_groups, num_atoms:
         raise ValueError("lags must be strictly increasing")
     if lags[0] < 0 or lags[-1] >= num_frames:
         raise ValueError(f"lags must be in [0, {num_frames}) (got {int(lags[0])}..{int(lags[-1])})")
-    if isinstance(r_max, (bool, np.bool_)) or not isinstance(r_max, (int, float, np.integer, np.floating)):
-        raise get_type_error("r_max", r_max, "float")
-    r_max = float(r_max)
-    if not (np.isfinite(r_max) and r_max > 0):
-        raise ValueError(f"r_max must be finite and > 0 (got {r_max})")
+    return np.ascontiguousarray(lags)
+
+
+def _check_distinct_van_hove_args(lattice, lags, r_max, num_bins, atom_groups, num_atoms: int, num_frames: int):
+    """Validate the arguments of ``get_distinct_van_hove`` in the order lattice, lags, r_max, num_bins, atom_groups
+    (valid lags imply a frame); returns the lattice (3,3), the lags (T,) as int64, r_max as a float, and the group
+    offsets and atoms (CSR, int64)."""
+    lattice = _check_lattice(lattice)
+    volume, widths = _cell_widths(lattice)
+    if not volume > 0:
+        raise ValueError("lattice has zero cell volume")
+    lags = _check_lags(lags, num_frames)
+    r_max = _check_cell_r_max(r_max, widths)
     _check_num_bins(num_bins)
     offsets, atoms = _check_atom_groups(atom_groups, num_atoms)
-    if num_frames < 2:
-        raise ValueError("positions_ts must contain at least 2 frames")
-    return lattice, np.ascontiguousarray(lags), r_max, offsets, atoms
+    return lattice, lags, r_max, offsets, atoms
 
 
 def _check_projection_args(lattice, vectors, num_atoms: int, num_frames: int):
@@ -556,6 +588,66 @@ class Trajectory(Dynamics, Sequence):
         """
         lag_times, radii, van_hove, moments = self.get_van_hove_device(lattice, lags, r_max, num_bins, atom_groups)
         return lag_times.cpu().numpy(), radii.cpu().numpy(), van_hove.cpu().numpy(), moments.cpu().numpy()
+
+    def get_distinct_van_hove_device(self, lattice, lags, r_max, num_bins, atom_groups=None):
+        """``get_distinct_van_hove`` with the result left on the GPU (three CUDA tensors)."""
+        num_frames, num_atoms = int(self._positions_ts.shape[0]), int(self._positions_ts.shape[1])
+        lattice, lags, r_max, offsets, atoms = _check_distinct_van_hove_args(lattice, lags, r_max, num_bins,
+                                                                             atom_groups, num_atoms, num_frames)
+        import torch  # pylint: disable=import-outside-toplevel
+
+        lib = _lib.lib()
+        positions, device = self._device_positions()
+        num_groups, num_lags, num_bins = len(offsets) - 1, len(lags), int(num_bins)
+        lag_times = np.asarray(lags, dtype=np.float64) * self._timestep
+        radii = (np.arange(num_bins) + 0.5) * (r_max / num_bins)
+        with torch.cuda.device(device):
+            g_d = torch.empty((num_groups, num_groups, num_lags, num_bins), dtype=torch.float64,
+                              device=positions.device)
+            ws_bytes = int(lib.rn_distinct_van_hove_workspace_size(len(atoms), num_groups, num_lags, num_bins))
+            workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=positions.device)
+            status = lib.rn_distinct_van_hove(ctypes.c_void_p(positions.data_ptr()), num_frames, num_atoms,
+                                              ctypes.c_void_p(lattice.ctypes.data), ctypes.c_void_p(lags.ctypes.data),
+                                              num_lags, r_max, num_bins, ctypes.c_void_p(offsets.ctypes.data),
+                                              ctypes.c_void_p(atoms.ctypes.data), num_groups,
+                                              ctypes.c_void_p(g_d.data_ptr()), ctypes.c_void_p(workspace.data_ptr()),
+                                              _lib.current_stream(device))
+            _lib.check(status, "rn_distinct_van_hove")
+            return torch.from_numpy(lag_times).to(positions.device), torch.from_numpy(radii).to(positions.device), g_d
+
+    def get_distinct_van_hove(self, lattice, lags, r_max, num_bins, atom_groups=None):
+        """Distinct part of the Van Hove correlation of atom groups -> (lag_times, r, g_d), numpy arrays of shape (T,),
+        (B,) and (G, G, T, B).
+
+        ``lattice``, ``r_max``, ``num_bins`` and ``atom_groups`` are those of ``get_rdf`` (``0 < r_max <= w_min / 2``,
+        B in 1..4096, groups may overlap); ``r`` are its bin centres.  ``lags`` are T >= 1 strictly increasing integer
+        frame lags in [0, S) and ``lag_times = lags * timestep`` in fs, as in ``get_van_hove``.
+
+        For every ordered group pair (a, b), lag t, origin n < S - t and pair i in a, j in b with i != j, the
+        minimum-image vector ``v = (d - ceil(d - 0.5)) @ lattice`` of ``d = x_j(n + t) - x_i(n)`` counts into bin
+        k = floor(|v| * B / r_max) when k < B, and ``g_d[a, b, t, k] = count * V / ((S - t) * n_ab * shell_k)`` with the
+        V, n_ab and shell_k of ``get_rdf``; a pair of groups with n_ab = 0 gets a zero row.  It is the probability of
+        finding a b atom at distance r at time n + t from where an a atom was at time n, relative to an ideal gas.  The
+        result is not mirrored: ``g_d[a, b, t]`` and ``g_d[b, a, t]`` are different sums for t > 0 (the first is the
+        second of the time-reversed trajectory).
+
+        At lag 0 it is the RDF: ``g_d[:, :, lags == 0]`` equals ``get_rdf(lattice, r_max, num_bins, atom_groups)[1]``
+        bit for bit (unless a coordinate difference sits exactly on a ±1/2 wrap tie with r_max exactly at w_min / 2).
+        At long lags it tends to 1 for an uncorrelated or diffusing species, and to the time-averaged site structure
+        (the RDF of the average positions, broadened by the vibrations) for a crystal.  A peak of ``g_d[a, a, t]`` at
+        r -> 0 that grows with t means that other atoms of a move into the sites a atoms left: site refilling and
+        concerted hopping, as of Li in a superionic conductor; the decay of the shells towards 1 shows the cage
+        relaxing.  For one species a, the total Van Hove function in Å^-3 is
+        ``G(r, t) = g_s[a, t] + (|a| - 1) / V * g_d[a, a, t]`` with the ``g_s`` of ``get_van_hove`` on the same lags,
+        r_max and bins.
+
+        The distances are evaluated in FP64 with every product and sum rounded on its own, so the counts are exact
+        integers, the same for every launch configuration, host and device trajectories, repeated calls and a group
+        pair computed alone or with others.  A device-resident trajectory is read in place; a host trajectory is copied
+        to the device once (its S·N·24 bytes must fit there).  Argument errors are raised before any device work.
+        """
+        lag_times, radii, g_d = self.get_distinct_van_hove_device(lattice, lags, r_max, num_bins, atom_groups)
+        return lag_times.cpu().numpy(), radii.cpu().numpy(), g_d.cpu().numpy()
 
     def __len__(self) -> int:
         return int(self._positions_ts.shape[0])
